@@ -688,8 +688,10 @@ def run_ours(args):
     sampler.rows.clear()                       # keep only the samples taken during the timed region
     torch.cuda.nvtx.range_push("timed")
     g0 = trainer.global_step
-    ms_total, (_, out) = timed(step_resident, args.steps)
+    ms_total, (loss, out) = timed(step_resident, args.steps)
     torch.cuda.nvtx.range_pop()
+    if args.dump_outputs and rank == 0:        # before any later step can touch the last timed step's results
+        dump_outputs(args.dump_outputs, {"loss": loss, **out})
     clocks = sampler.stop() if rank == 0 else None
     launches = L.STATS["launches"]
     L.stats_reset(False)
@@ -816,6 +818,30 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+DUMP_ROWS = 1 << 19        # per-sample outputs (~3.4 M samples a step) are cut to this many rows: 18 MB written in all
+
+
+def dump_outputs(out_dir, named):
+    """Write every tensor of `named` as out_dir/<name>.npy: float32, or float64 for float64, integer and bool data
+    (which float64 holds exactly).  An output with more than DUMP_ROWS rows keeps the rows of one fixed seeded sample,
+    the same rows for every output of that length, so that two builds can be compared output for output."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in named.items():
+        if not isinstance(t, torch.Tensor):
+            continue
+        t = t.detach()
+        if t.dim() and t.shape[0] > DUMP_ROWS:
+            rows = np.sort(np.random.default_rng(0).choice(t.shape[0], DUMP_ROWS, replace=False))
+            t = t[torch.from_numpy(rows).to(t.device)]
+        a = (t.float() if t.is_floating_point() and t.dtype != torch.float64 else t.double()).cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        total += a.nbytes
+    assert total <= 64 << 20, f"--dump-outputs wrote {total} bytes"
+
+
 _REAL_STDOUT = None
 
 
@@ -839,6 +865,8 @@ def main():
                     help="skip the reference-GPU-kernel comparison and the PyTorch-CUDA stand-in step (1-GPU runs only)")
     ap.add_argument("--no-relight", action="store_true",
                     help="skip the split-train rays/s and relit-frames/s sections (configs[2], configs[3])")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and render outputs of the last timed training step as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     # stdout carries exactly ONE JSON line: anything a library prints on fd 1 meanwhile (NCCL's version banner under

@@ -14,6 +14,26 @@ from oracle import ref as oref  # noqa: E402
 from rise_sdf_b200 import synthetic as syn  # noqa: E402
 
 ROI = [-1.5] * 3 + [1.5] * 3
+# rays stored per file: the five special rays and every k-th ray after them, so that each file stays under 1 MB
+KEEP_EVERY = {"ball": 5, "random": 3}
+PER_RAY = ("rays_o", "rays_d", "t_min", "t_max")
+PER_SAMPLE = ("t_starts", "t_ends", "alphas", "weights", "trans", "grad_weights", "grad_alphas")
+
+
+def keep_rays(rec, every):
+    """`rec` restricted to rays 0-4 and every `every`-th ray.  A ray's samples are one contiguous run of the packed
+    arrays and every kernel here works ray by ray, so the kept runs are exactly what the kernels give for the kept rays;
+    only packed_info and ray_indices are renumbered."""
+    pk = rec["packed_info"]
+    keep = np.array([r for r in range(len(pk)) if r < 5 or r % every == 0])
+    sel = np.concatenate([np.arange(pk[r, 0], pk[r, 0] + pk[r, 1]) for r in keep]).astype(np.int64)
+    n = pk[keep, 1]
+    out = dict(rec)
+    out.update({k: rec[k][keep] for k in PER_RAY})
+    out.update({k: rec[k][sel] for k in PER_SAMPLE})
+    out["packed_info"] = np.stack([np.cumsum(n) - n, n], 1).astype(pk.dtype)
+    out["ray_indices"] = np.repeat(np.arange(len(keep)), n).astype(rec["ray_indices"].dtype)
+    return out
 
 
 def main(out_dir):
@@ -41,13 +61,16 @@ def main(out_dir):
         T = C.transmittance_from_alpha_forward_naive(pk, a)
         gw = torch.randn_like(w)
         ga = C.weight_from_alpha_backward_naive(w, gw, pk, a)
-        np.savez_compressed(
-            os.path.join(out_dir, f"march_{tag}.npz"), cone=np.float32(cone), rays_o=o.cpu().numpy(), rays_d=d.cpu().numpy(),
+        rec = dict(
+            cone=np.float32(cone), rays_o=o.cpu().numpy(), rays_d=d.cpu().numpy(),
             roi=np.array(ROI, np.float32), grid=grid.numpy(), step=np.float32(step), t_min=tmin.cpu().numpy(),
             t_max=tmax.cpu().numpy(), packed_info=pk.cpu().numpy(), ray_indices=ri.cpu().numpy(),
             t_starts=ts[:, 0].cpu().numpy(), t_ends=te[:, 0].cpu().numpy(), alphas=a[:, 0].cpu().numpy(),
             weights=w[:, 0].cpu().numpy(), trans=T[:, 0].cpu().numpy(), grad_weights=gw[:, 0].cpu().numpy(),
             grad_alphas=ga[:, 0].cpu().numpy())
+        if tag in KEEP_EVERY:
+            rec = keep_rays(rec, KEEP_EVERY[tag])
+        np.savez_compressed(os.path.join(out_dir, f"march_{tag}.npz"), **rec)
         print(tag, "rays", R, "samples", ri.shape[0])
 
 

@@ -1,5 +1,8 @@
 """K4 parity: scan / accumulate / fused NeuS render vs the C oracle (serial order), the torch
-oracle (autograd) and the reference's compiled kernels when oracle/_ref is present."""
+oracle (autograd) and the reference's compiled kernels (through the golden vectors they produced)."""
+import glob
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -7,11 +10,11 @@ import torch.nn.functional as F
 
 from oracle import fields as of
 from oracle import march as omarch
-from oracle import ref as oref
 from rise_sdf_b200 import nerfacc as rn
 from rise_sdf_b200.neus import _NeusRender
 
 pytestmark = pytest.mark.gpu
+GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def ragged(n_rays=300, max_len=1024, seed=0, special=True):
@@ -80,18 +83,20 @@ def test_scan_backward_vs_oracles():
     assert np.abs(g_w_only - ga0).max() <= 2e-4 * max(np.abs(ga0).max(), 1)
 
 
-def test_scan_vs_reference_kernels():
-    C = oref.nerfacc_cuda()
-    if C is None:
-        pytest.skip("oracle/_ref/nerfacc_cuda.so not built")
-    ri, a, n = ragged()
-    pk = torch.tensor(omarch.pack_info(ri, n)).cuda()
-    at = torch.tensor(a).cuda()
-    w_ref = C.weight_from_alpha_forward_naive(pk, at[:, None].contiguous())[:, 0]
-    T_ref = C.transmittance_from_alpha_forward_naive(pk, at[:, None].contiguous())[:, 0]
+@pytest.mark.parametrize("gold", sorted(glob.glob(os.path.join(GOLD, "march_*.npz"))), ids=os.path.basename)
+def test_scan_vs_reference_kernels(gold):
+    """Against the reference's compiled weight_from_alpha_{forward,backward}_naive and
+    transmittance_from_alpha_forward_naive (render_weight.cu:86-154), whose outputs on the marched samples
+    are stored in tests/golden/march_*.npz (tests/golden/make_golden.py)."""
+    z = np.load(gold)
+    pk = torch.from_numpy(z["packed_info"]).cuda()
+    at = torch.from_numpy(z["alphas"]).cuda().requires_grad_(True)
     w, T = rn.render_weight_from_alpha(at, packed_info=pk)
-    np.testing.assert_allclose(w.cpu().numpy(), w_ref.cpu().numpy(), rtol=1e-5, atol=1e-30)
-    np.testing.assert_allclose(T.cpu().numpy(), T_ref.cpu().numpy(), rtol=1e-5, atol=1e-30)
+    np.testing.assert_allclose(w.detach().cpu().numpy(), z["weights"], rtol=1e-5, atol=1e-30)
+    np.testing.assert_allclose(T.detach().cpu().numpy(), z["trans"], rtol=1e-5, atol=1e-30)
+    (w * torch.from_numpy(z["grad_weights"]).cuda()).sum().backward()
+    ga = z["grad_alphas"]
+    assert np.abs(at.grad.cpu().numpy() - ga).max() <= 2e-4 * max(np.abs(ga).max(), 1)
 
 
 @pytest.mark.parametrize("D", [1, 3, 8, 24])
