@@ -343,11 +343,12 @@ int rsdf_sdf_mlp_bwd(const rsdf_sdf_mlp *net, const float *in0, int w0, float sc
                      const float *in1, int w1, int n_samples, const float *g_out, const float *g_sdf,
                      const float *g_g0a, const float *g_g0b, const uint32_t *amax_bits, float *g_in0, float *g_in1,
                      float *gW1, float *gb1, float *gW2, float *gb2, float *gW3, float *gb3, void *stream);
-/* Inference forward of the same network with the activations as the A operand in TENSOR MEMORY (tcgen05.mma TS
- * form, csrc/sdf_eval_ts.cu): 128-sample tiles, full 128x128x16 instructions, two independent half-CTAs.
- * out[S,n_out] and/or sdf[S] = out[:,0]; with out == NULL the output layer is replaced by an fp32 dot product. */
+/* sdf-only inference forward of the same network, sdf[S] = out[:,0], with the activations as the A operand in
+ * TENSOR MEMORY (tcgen05.mma TS form, csrc/sdf_eval_ts.cu): 128-sample tiles, full 128x128x16 instructions, two
+ * independent half-CTAs; the output layer is replaced by an fp32 dot product with w3_row0.  fp32-class only
+ * (precision is not read).  The full output is rsdf_sdf_mlp_fwd's. */
 int rsdf_sdf_mlp_eval(const rsdf_sdf_mlp *net, const float *in0, int w0, float scale0, float shift0,
-                      const float *in1, int w1, int n_samples, float *out, float *sdf, void *stream);
+                      const float *in1, int w1, int n_samples, float *sdf, void *stream);
 /* *out_bits = float bits of max(|a|, |b|) (device scalar; either array may be empty; 16-byte aligned);
  * accumulate != 0 keeps the value already in *out_bits as a third candidate.  The fp16-split kernels derive
  * their power-of-two cotangent scaling from it. */

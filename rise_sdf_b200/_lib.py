@@ -116,7 +116,7 @@ _SIGS = {
     "rsdf_sdf_mlp_fwd": [c_p, c_p, c_i, c_f, c_f, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_p],
     "rsdf_sdf_mlp_bwd": [c_p, c_p, c_i, c_f, c_f, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p,
                          c_p, c_p, c_p, c_p, c_p],
-    "rsdf_sdf_mlp_eval": [c_p, c_p, c_i, c_f, c_f, c_p, c_i, c_i, c_p, c_p, c_p],
+    "rsdf_sdf_mlp_eval": [c_p, c_p, c_i, c_f, c_f, c_p, c_i, c_i, c_p, c_p],
     "rsdf_absmax2": [c_p, ctypes.c_longlong, c_p, ctypes.c_longlong, c_p, c_i, c_p],
     "rsdf_relu_layer_fwd": [c_p, c_p],
     "rsdf_relu_layer_bwd": [c_p, c_p],

@@ -1,9 +1,10 @@
-// K3e -- inference forward of the SDF field MLP (35 -> 128 -> 128 -> 48, Softplus(100); models/geometry.py:206-244,
-// models/network_utils.py:109-157) with the ACTIVATIONS AS THE A OPERAND IN TENSOR MEMORY (tcgen05.mma "TS" form).
+// K3e -- sdf-only inference forward of the SDF field MLP (35 -> 128 -> 128 -> 48, Softplus(100), sdf = out[:, 0];
+// models/geometry.py:206-244, models/network_utils.py:109-157) with the ACTIVATIONS AS THE A OPERAND IN TENSOR MEMORY
+// (tcgen05.mma "TS" form).
 //
-// Used by everything that evaluates the field without a graph: eval / relighting render, occupancy update, and
-// the 7 evaluations per sample behind the finite-difference normals of the split-sum config (the most-called
-// kernel of a relit frame).  Compared with the shared-memory-operand kernels of csrc/sdf_train.cu:
+// Used where only the sdf is wanted: the 6 finite-difference neighbours per sample of the split-sum config (the
+// most-called kernel of a relit frame; in training too, as the forward of the sdf-only node) and isosurface
+// levels.  Compared with the shared-memory-operand kernels of csrc/sdf_train.cu:
 //   * samples sit on the 128 TMEM lanes (M = 128 samples per tile), features on the N axis: D[sample, feature] =
 //     A[sample, :] . W[feature, :], B = the weight blob straight from shared memory (K-major, N = 128);
 //   * the A operand is never in shared memory: an epilogue thread reads its sample row of the accumulator with
@@ -12,8 +13,8 @@
 //     where the next layer's MMAs read them.  The shared-memory form at N <= 64 is bound by the 4 KB A fetch per
 //     instruction (~55 cycles per K-step measured); here every instruction is a full 128 x 128 x 16 (64 cycles of
 //     math for twice the samples) and shared memory holds nothing but the 112 KB of weights;
-//   * sdf-only calls (6 of 7 evaluations) skip the output layer: each thread dots its half row of a2 with
-//     W3[0, :] in fp32 and the two halves meet in shared memory;
+//   * no output layer GEMM: each thread dots its half row of a2 with W3[0, :] in fp32 and the two halves meet in
+//     shared memory;
 //   * two independent half-CTAs as in sdf_eval_kernel: epilogue group g (8 warps: 4 lane quadrants x 2 feature
 //     halves, named barrier 1 + g) with its own tile stream and 256 TMEM columns (A hi 64 | A lo 64 | D 128),
 //     served by MMA-issuer warp 16 + g through mbarriers ready[g] / done[g].
@@ -111,9 +112,8 @@ __device__ __forceinline__ float sp_act(float z) {            // torch Softplus(
 #define EPI_DONE() { tmem_st_wait(); tc::tc_fence_before(); grp_sync(g); if (tg == 0) mbar_arrive(&ct->ready[g]); }
 #define EPI_WAIT() { tc::mbar_wait(&ct->done[g], dpar); dpar ^= 1u; tc::tc_fence_after(); }
 
-template <bool SDF_ONLY>
 __global__ void __launch_bounds__(THREADS, 1)
-sdf_eval_ts_kernel(const Net net, const Inputs in, float *__restrict__ out, float *__restrict__ sdf) {
+sdf_eval_ts_kernel(const Net net, const Inputs in, float *__restrict__ sdf) {
     extern __shared__ __align__(1024) uint8_t smem[];
     Ctrl *ct = reinterpret_cast<Ctrl *>(smem + CTRL_OFF);
     float *sb1 = reinterpret_cast<float *>(smem + BIAS_OFF), *sb2 = sb1 + 128, *sb3 = sb2 + 128, *sw30 = sb3 + 64;
@@ -145,15 +145,11 @@ sdf_eval_ts_kernel(const Net net, const Inputs in, float *__restrict__ out, floa
         const uint32_t tm = tmem + GRP_COLS * g;
         const tc::Operand B1 = tc::op_kmajor(tc::smem_u32(smem + W1_OFF), W1_PLANE, HID);
         const tc::Operand B2 = tc::op_kmajor(tc::smem_u32(smem + W2_OFF), W2_PLANE, HID);
-        const tc::Operand B3 = tc::op_kmajor(tc::smem_u32(smem + W3_OFF), W3_PLANE, KP);
-        const uint32_t id128 = tc::instr_desc(128, HID, false, false), id48 = tc::instr_desc(128, KP, false, false);
+        const uint32_t id128 = tc::instr_desc(128, HID, false, false);
         uint32_t rpar = 0u;
         for (int tile = 2 * blockIdx.x + g; tile < n_tiles; tile += 2 * gridDim.x) {
             ISSUE(gemm3_ts<KP / 16>(tm + D0, tm + A_HI, tm + A_LO, B1, id128);)
             ISSUE(gemm3_ts<HID / 16>(tm + D0, tm + A_HI, tm + A_LO, B2, id128);)
-            if (!SDF_ONLY) {
-                ISSUE(gemm3_ts<HID / 16>(tm + D0, tm + A_HI, tm + A_LO, B3, id48);)
-            }
         }
     } else {
         // ---- epilogue group g: thread = (sample row r of the tile, feature half ch) --------------------------
@@ -210,59 +206,22 @@ sdf_eval_ts_kernel(const Net net, const Inputs in, float *__restrict__ out, floa
             }
             EPI_DONE()
             EPI_WAIT()
-            if (SDF_ONLY) {
-                float dot = 0.0f;
+            float dot = 0.0f;
 #pragma unroll
-                for (int c = 0; c < 4; ++c) {             // w3[0, :] . softplus(Z2 + b2) over this thread's half row
-                    float v[16];
-                    tc::tmem_ld16(tl + D0 + 64 * ch + 16 * c, v);
-                    tc::tmem_ld_wait();
+            for (int c = 0; c < 4; ++c) {             // w3[0, :] . softplus(Z2 + b2) over this thread's half row
+                float v[16];
+                tc::tmem_ld16(tl + D0 + 64 * ch + 16 * c, v);
+                tc::tmem_ld_wait();
 #pragma unroll
-                    for (int j = 0; j < 16; ++j) {
-                        const int f = 64 * ch + 16 * c + j;
-                        dot = fmaf(sw30[f], sp_act(v[j] + sb2[f]), dot);
-                    }
-                }
-                if (ch == 1) sdot[128 * g + r] = dot;
-                tc::tc_fence_before();
-                grp_sync(g);
-                if (ch == 0 && s < in.S) sdf[s] = dot + sdot[128 * g + r] + sb3[0];
-            } else {
-#pragma unroll
-                for (int c = 0; c < 4; ++c) {             // a2 = softplus(Z2 + b2)
-                    float v[16];
-                    tc::tmem_ld16(tl + D0 + 64 * ch + 16 * c, v);
-                    tc::tmem_ld_wait();
-                    uint32_t hi[8], lo[8];
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) {
-                        const int f = 64 * ch + 16 * c + 2 * j;
-                        tc::split2(sp_act(v[2 * j] + sb2[f]), sp_act(v[2 * j + 1] + sb2[f + 1]), hi[j], lo[j]);
-                    }
-                    tmem_st8(tl + A_HI + 32 * ch + 8 * c, hi);
-                    tmem_st8(tl + A_LO + 32 * ch + 8 * c, lo);
-                }
-                EPI_DONE()
-                EPI_WAIT()
-                // out[s, :] = Z3 + b3: 48 columns -> ch 0 takes [0, 32), ch 1 [32, 48)
-                const int c_begin = ch == 0 ? 0 : 2, c_end = ch == 0 ? 2 : 3;
-                for (int c = c_begin; c < c_end; ++c) {
-                    float v[16];
-                    tc::tmem_ld16(tl + D0 + 16 * c, v);
-                    tc::tmem_ld_wait();
-                    if (s < in.S) {
-#pragma unroll
-                        for (int j = 0; j < 16; ++j) {
-                            const int f = 16 * c + j;
-                            if (f < net.n_out) {
-                                const float o = v[j] + sb3[f];
-                                if (out) out[(size_t)s * net.n_out + f] = o;
-                                if (sdf && f == 0) sdf[s] = o;
-                            }
-                        }
-                    }
+                for (int j = 0; j < 16; ++j) {
+                    const int f = 64 * ch + 16 * c + j;
+                    dot = fmaf(sw30[f], sp_act(v[j] + sb2[f]), dot);
                 }
             }
+            if (ch == 1) sdot[128 * g + r] = dot;
+            tc::tc_fence_before();
+            grp_sync(g);
+            if (ch == 0 && s < in.S) sdf[s] = dot + sdot[128 * g + r] + sb3[0];
             tc::tc_fence_before();
             grp_sync(g);                                  // this group's TMEM columns / sdot are reused next tile
         }
@@ -277,10 +236,10 @@ sdf_eval_ts_kernel(const Net net, const Inputs in, float *__restrict__ out, floa
 extern "C" {
 
 int rsdf_sdf_mlp_eval(const rsdf_sdf_mlp *n, const float *in0, int w0, float scale0, float shift0, const float *in1,
-                      int w1, int n_samples, float *out, float *sdf, void *stream) {
+                      int w1, int n_samples, float *sdf, void *stream) {
     if (n_samples == 0) return 0;
     if (!n || !n->w1_blob || !n->w2_blob || !n->w3_blob || !n->b1 || !n->b2 || !n->b3 || !n->w3_row0 || n->n_in < 1 ||
-        n->n_in > KP || n->n_out < 1 || n->n_out > KP || !in0 || (!out && !sdf) || w0 < 1 || w1 < 0 || (w1 > 0 && !in1) ||
+        n->n_in > KP || n->n_out < 1 || n->n_out > KP || !in0 || !sdf || w0 < 1 || w1 < 0 || (w1 > 0 && !in1) ||
         w0 + w1 != n->n_in)
         return RSDF_EBADARG;
     const Net net{(const uint8_t *)n->w1_blob, (const uint8_t *)n->w2_blob, (const uint8_t *)n->w3_blob,
@@ -288,16 +247,10 @@ int rsdf_sdf_mlp_eval(const rsdf_sdf_mlp *n, const float *in0, int w0, float sca
     const Inputs in{in0, in1, w0, w1, scale0, shift0, n_samples};
     const int n_tiles = (n_samples + TS_M - 1) / TS_M, pairs = (n_tiles + 1) / 2;
     const int grid = pairs < RSDF_NUM_SMS ? pairs : RSDF_NUM_SMS;
-    cudaError_t e;
-    if (!out) {
-        e = cudaFuncSetAttribute(sdf_eval_ts_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
-        if (e != cudaSuccess) return (int)e;
-        sdf_eval_ts_kernel<true><<<grid, THREADS, SMEM_BYTES, (cudaStream_t)stream>>>(net, in, out, sdf);
-    } else {
-        e = cudaFuncSetAttribute(sdf_eval_ts_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_BYTES);
-        if (e != cudaSuccess) return (int)e;
-        sdf_eval_ts_kernel<false><<<grid, THREADS, SMEM_BYTES, (cudaStream_t)stream>>>(net, in, out, sdf);
-    }
+    const cudaError_t e = cudaFuncSetAttribute(sdf_eval_ts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                               (int)SMEM_BYTES);
+    if (e != cudaSuccess) return (int)e;
+    sdf_eval_ts_kernel<<<grid, THREADS, SMEM_BYTES, (cudaStream_t)stream>>>(net, in, sdf);
     RSDF_LAUNCH_CHECK();
     return 0;
 }

@@ -844,10 +844,11 @@ sdf_bwd_kernel(const Net net, const Inputs in, const Grads g_) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// inference forward (out and/or sdf only): eval / relighting render, occupancy update, and the 7 evaluations per
-// sample behind the finite-difference normals of the split-sum config -- by far the most-called kernel of a relit
-// frame.  Without the gradient chain only ONE [128 x 64] activation image is live per tile, so two tiles fit next
-// to the 112 KB of weights, and the kernel runs as TWO INDEPENDENT HALF-CTAs: epilogue group g (8 warps, named
+// inference forward of the full output (out, and sdf = out[:,0] once more when asked): eval / relighting render and
+// occupancy update.  The sdf-only evaluations (the finite-difference neighbours of the split-sum config) run on the
+// TMEM-operand kernel of csrc/sdf_eval_ts.cu, the faster of the two there and the slower one for the full output
+// (DESIGN.md §4).  Without the gradient chain only ONE [128 x 64] activation image is live per tile, so two tiles
+// fit next to the 112 KB of weights, and the kernel runs as TWO INDEPENDENT HALF-CTAs: epilogue group g (8 warps, named
 // barrier 1 + g) works through its own stream of 64-sample tiles with its own images and TMEM columns, and MMA-
 // issuer warp 16 + g serves it (tcgen05.mma issue blocks the issuing warp while the tensor pipe's queue is full,
 // so issuing is that warp's only job).  Group g announces "operands of the next GEMM are in place" on mbarrier
@@ -880,11 +881,6 @@ __device__ __forceinline__ void ev_arrive(uint64_t *bar) {
 #define EV_DONE() { tc::fence_async_smem(); tc::tc_fence_before(); ev_sync(g); if (tg == 0) ev_arrive(&ct->ready[g]); }
 #define EV_WAIT() { tc::mbar_wait(&ct->done[g], dpar); dpar ^= 1u; tc::tc_fence_after(); }
 
-// SDF_ONLY (6 of every 7 evaluations of a relit frame: the finite-difference neighbours): only out[:, 0] is wanted,
-// so the third GEMM -- 42 % of the kernel's tensor work for one useful row of 128 -- is replaced by an fp32 dot
-// product on the CUDA cores: the a2 epilogue writes w3[0,f] * a2[f,s] into the (now idle) image buffer as
-// [sample][feature] floats and every warp sums 128 features for 8 samples with one 16-byte load and 5 shuffles.
-template <bool SDF_ONLY>
 __global__ void __launch_bounds__(EV_THREADS, 1)
 sdf_eval_kernel(const Net net, const Inputs in, float *__restrict__ out, float *__restrict__ sdf) {
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -919,9 +915,7 @@ sdf_eval_kernel(const Net net, const Inputs in, float *__restrict__ out, float *
         for (int tile = 2 * blockIdx.x + g; tile < n_tiles; tile += 2 * gridDim.x) {
             EV_ISSUE(gemm3<KP / 16>(tm + 0, tc::op_kmajor(sW1, W1_PLANE, HID), tc::op_mnmajor(sH0, IMG_S_PLANE, KP), id_kn, false);)
             EV_ISSUE(gemm3<HID / 16>(tm + 64, tc::op_kmajor(sW2, W2_PLANE, HID), tc::op_mnmajor(sA, IMG_B_PLANE, HID), id_kn, false);)
-            if (!SDF_ONLY) {
-                EV_ISSUE(gemm3<HID / 16>(tm + 128, tc::op_kmajor(sW3, W3_PLANE, KP), tc::op_mnmajor(sA, IMG_B_PLANE, HID), id_kn, false);)
-            }
+            EV_ISSUE(gemm3<HID / 16>(tm + 128, tc::op_kmajor(sW3, W3_PLANE, KP), tc::op_mnmajor(sA, IMG_B_PLANE, HID), id_kn, false);)
         }
     } else {
         // ---- epilogue group g: thread = feature row f x the 32 sample columns [32*cg, +32) -----------
@@ -929,7 +923,7 @@ sdf_eval_kernel(const Net net, const Inputs in, float *__restrict__ out, float *
         const int cg = (t.warp >> 2) & 1;
         t.tl = tmem + ((uint32_t)(t.q * 32) << 16) + (uint32_t)(192 * g);
         uint8_t *h0_img = smem + EV_H0 + g * IMG_S_BYTES, *a_img = smem + EV_A + g * IMG_B_BYTES;
-        const float b1f = net.b1[t.f], b2f = net.b2[t.f], w30f = net.w3r0[t.f], b30 = net.b3[0];
+        const float b1f = net.b1[t.f], b2f = net.b2[t.f];
         const float b3f = t.f < net.n_out ? net.b3[t.f] : 0.0f;
         // staging: feature row fs = tg % 64 (< 48), chunks cs and cs + 4 of the tile
         const int fs = tg & 63, cs = tg >> 6;
@@ -965,27 +959,6 @@ sdf_eval_kernel(const Net net, const Inputs in, float *__restrict__ out, float *
             }
             EV_DONE()
             EV_WAIT()
-            if (SDF_ONLY) {
-                float *prod = reinterpret_cast<float *>(a_img);        // [64 samples][128 features] fp32 = 32 KB
-#pragma unroll
-                for (int cc = 0; cc < 2; ++cc) {          // w3[0,f] * softplus(Z2 + b2)
-                    t.col0 = 32 * cg + 16 * cc;
-                    float v[16];
-                    ld16(t, 64, v);
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) prod[(t.col0 + j) * HID + t.f] = w30f * sp_act(v[j] + b2f);
-                }
-                tc::tc_fence_before();
-                ev_sync(g);
-                const int wg = t.warp & 7;                // 8 warps x 8 samples
-#pragma unroll
-                for (int i = 0; i < 8; ++i) {
-                    const int sl = 8 * wg + i;
-                    const float4 q = *reinterpret_cast<const float4 *>(prod + sl * HID + 4 * t.lane);
-                    const float sum = warp_sum((q.x + q.y) + (q.z + q.w));
-                    if (t.lane == 0 && s0 + sl < in.S) sdf[s0 + sl] = sum + b30;
-                }
-            } else {
 #pragma unroll
             for (int cc = 0; cc < 2; ++cc) {              // a2 = softplus(Z2 + b2)  (a1's GEMM has drained)
                 t.col0 = 32 * cg + 16 * cc;
@@ -1011,7 +984,6 @@ sdf_eval_kernel(const Net net, const Inputs in, float *__restrict__ out, float *
                             if (sb + j < in.S) sdf[sb + j] = v[j] + b3f;
                     }
                 }
-            }
             }
             tc::tc_fence_before();
             ev_sync(g);                                   // this group's images / TMEM columns are reused next tile
@@ -1095,19 +1067,13 @@ int rsdf_sdf_mlp_fwd(const rsdf_sdf_mlp *net, const float *in0, int w0, float sc
     if (g0a) {
         if (net->precision) RSDF_FWD(true, false) else RSDF_FWD(true, true)
     } else if (net->precision) {
-        RSDF_FWD(false, false)          // (the two-group inference kernels below are fp32-class only)
+        RSDF_FWD(false, false)          // (the two-group inference kernel below is fp32-class only)
     } else {
         const int pairs = (n_tiles + 1) / 2;
         const int eg = pairs < RSDF_NUM_SMS ? pairs : RSDF_NUM_SMS;
-        if (!out) {
-            e = cudaFuncSetAttribute(sdf_eval_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EV_SMEM);
-            if (e != cudaSuccess) return (int)e;
-            sdf_eval_kernel<true><<<eg, EV_THREADS, EV_SMEM, (cudaStream_t)stream>>>(to_net(net), in, out, sdf);
-        } else {
-            e = cudaFuncSetAttribute(sdf_eval_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EV_SMEM);
-            if (e != cudaSuccess) return (int)e;
-            sdf_eval_kernel<false><<<eg, EV_THREADS, EV_SMEM, (cudaStream_t)stream>>>(to_net(net), in, out, sdf);
-        }
+        e = cudaFuncSetAttribute(sdf_eval_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EV_SMEM);
+        if (e != cudaSuccess) return (int)e;
+        sdf_eval_kernel<<<eg, EV_THREADS, EV_SMEM, (cudaStream_t)stream>>>(to_net(net), in, out, sdf);
     }
     RSDF_LAUNCH_CHECK();
     return 0;

@@ -30,6 +30,13 @@ def pad16(n):
     return (n + 15) // 16 * 16
 
 
+def fp16_variant():
+    """1 when VanillaMLP.mlp_precision selects the reduced-precision variant of the sdf_field and relu_mlp kernels
+    (single fp16 plane, one product per GEMM), else 0."""
+    from .network_utils import VanillaMLP
+    return 1 if VanillaMLP.mlp_precision == "fp16" else 0
+
+
 def pack_weight(W, n_pad=None, k_pad=None):
     """fp32 [N,K] (CUDA) -> uint8 blob of 4*N_pad*K_pad bytes (pads default to the next multiple of 16)."""
     W = W.detach().contiguous().float()

@@ -45,15 +45,13 @@ class VolumeSDF(nn.Module):
         # fused kernels (which return the raw network outputs) off.
         self._post_activations = "sdf_activation" in config or "feature_activation" in config
 
-    fused_analytic = True       # class-wide switch (tests compare the fused and the op-by-op paths)
-
     def _fused_parts(self):
         """(hash-grid Encoding, level mask or None) when the analytic-normal path can run on the fused
         SDF-field kernels (csrc/sdf_train.cu): include_xyz composite over a HashGrid, SDF-shaped MLP."""
         from . import sdf_field, tinycudann as tcnn
         from .network_utils import CompositeEncoding, ProgressiveBandHashGrid, VanillaMLP
         comp = self.encoding
-        if not (VolumeSDF.fused_analytic and isinstance(comp, CompositeEncoding) and comp.include_xyz
+        if not (isinstance(comp, CompositeEncoding) and comp.include_xyz
                 and isinstance(self.network, VanillaMLP) and sdf_field.supports(self.network, comp.n_output_dims)
                 and self.network.config_output_activation_is_identity and not self._post_activations):
             return None
@@ -91,81 +89,49 @@ class VolumeSDF(nn.Module):
         no_grad (eval / relighting / occupancy update / the 7 finite-difference evaluations per sample of
         the split-sum config) no autograd bookkeeping either."""
         from . import sdf_field
-        from .network_utils import VanillaMLP
         parts = self._fused_parts() if (x01.is_cuda and not x01.requires_grad and x01.shape[0] > 0) else None
-        if parts is not None:
-            inner, mask = parts
-            comp = self.encoding
-            if torch.is_grad_enabled():
-                if VanillaMLP.tc_training and VanillaMLP.fused_training:
-                    y = inner(x01)
-                    out, sdf, _, _ = sdf_field.fused_sdf_parts(self.network, x01, comp.xyz_scale, comp.xyz_offset,
-                                                               y if mask is None else y * mask, want_g0=False,
-                                                               sdf_only=sdf_only)
-                    return sdf if sdf_only else out        # (_fused_parts: the output activation is the identity)
-            elif VanillaMLP.fused_inference:
-                y = inner(x01)
-                if mask is not None:
-                    if self._mask_ones is None:            # one host sync; update_step refreshes the cache
-                        self._mask_ones = bool((mask == 1).all())
-                    if not self._mask_ones:
-                        y = y * mask
-                if self._packed_sdf is None:
-                    self._packed_sdf = sdf_field.PackedSDF(self.network)
-                identity = self.network.config_output_activation_is_identity
-                if sdf_only and identity:                 # only the sdf head is written: 4 B instead of 192 B per point
-                    return self._packed_sdf(x01, comp.xyz_scale, comp.xyz_offset, y, sdf_only=True)
-                out = self.network.output_activation(self._packed_sdf(x01, comp.xyz_scale, comp.xyz_offset, y))
-                return out[..., 0] if sdf_only else out
-        out = self.network(self.encoding(x01))
-        return out[..., 0] if sdf_only else out
+        if parts is None:
+            out = self.network(self.encoding(x01))
+            return out[..., 0] if sdf_only else out
+        inner, mask = parts
+        comp = self.encoding
+        y = inner(x01)
+        if mask is not None:
+            y = y * mask
+        # (_fused_parts: the output activation is the identity; sdf_only writes just the sdf head, 4 B instead of 192 B
+        # per point)
+        if not torch.is_grad_enabled():
+            return self.network.packed()(x01, comp.xyz_scale, comp.xyz_offset, y, sdf_only=sdf_only)
+        out, sdf, _, _ = sdf_field.fused_sdf_parts(self.network, x01, comp.xyz_scale, comp.xyz_offset, y, want_g0=False,
+                                                   sdf_only=sdf_only)
+        return sdf if sdf_only else out
 
     def _fd6_sdf(self, points, eps):
         """sdf at the six finite-difference neighbours of `points` [..., 3] -> [..., 6], or None when the fused
-        inference path does not apply.  One hash-grid launch builds the neighbours exactly as the reference
-        does (add, clamp, scale: models/geometry.py:229-237) and re-gathers corners only when a neighbour leaves
-        the previous one's cell; the MLP then writes just the sdf head."""
+        path does not apply.  One hash-grid launch builds the neighbours exactly as the reference does (add, clamp,
+        scale: models/geometry.py:229-237) and re-gathers corners only when a neighbour leaves the previous one's
+        cell; the MLP then writes just the sdf head.  Under autograd the hash-grid launch is differentiable w.r.t. the
+        table and the MLP is the sdf-only fused node -- instead of building the 6S neighbour positions with torch ops
+        and running the generic hash-grid forward over them."""
         from . import sdf_field, tinycudann as tcnn
-        from .network_utils import VanillaMLP
-        if torch.is_grad_enabled() or not (points.is_cuda and VanillaMLP.fused_inference and points.numel() > 0):
-            return None
-        parts = self._fused_parts()
-        if parts is None or not self.network.config_output_activation_is_identity:
-            return None
-        inner, mask = parts
-        comp = self.encoding
-        x01, y = tcnn.hashgrid_fd6(inner, points.reshape(-1, 3), eps, self.radius)
-        if mask is not None:
-            if self._mask_ones is None:
-                self._mask_ones = bool((mask == 1).all())
-            if not self._mask_ones:
-                y = y * mask
-        if self._packed_sdf is None:
-            self._packed_sdf = sdf_field.PackedSDF(self.network)
-        sdf = self._packed_sdf(x01, comp.xyz_scale, comp.xyz_offset, y, sdf_only=True)
-        return sdf.view(*points.shape[:-1], 6)
-
-    def _fd6_sdf_train(self, points, eps):
-        """`_fd6_sdf` under autograd (training): the same single hash-grid launch for the six neighbours, differentiable
-        w.r.t. the table, followed by the sdf-only fused MLP node -- instead of building the 6S neighbour positions with
-        torch ops and running the generic hash-grid forward over them.  None when the fused path does not apply."""
-        from . import sdf_field, tinycudann as tcnn
-        from .network_utils import VanillaMLP
-        if not (torch.is_grad_enabled() and points.is_cuda and not points.requires_grad and points.numel() > 0
-                and VanillaMLP.tc_training and VanillaMLP.fused_training):
+        grad = torch.is_grad_enabled()
+        if not points.is_cuda or points.numel() == 0 or (grad and points.requires_grad):
             return None
         parts = self._fused_parts()
         if parts is None:
             return None
         inner, mask = parts
         comp = self.encoding
-        x01, y = tcnn.hashgrid_fd6_train(inner, points.reshape(-1, 3), eps, self.radius)
-        _, sdf, _, _ = sdf_field.fused_sdf_parts(self.network, x01, comp.xyz_scale, comp.xyz_offset,
-                                                 y if mask is None else y * mask, want_g0=False, sdf_only=True)
+        fd6 = tcnn.hashgrid_fd6_train if grad else tcnn.hashgrid_fd6
+        x01, y = fd6(inner, points.reshape(-1, 3), eps, self.radius)
+        if mask is not None:
+            y = y * mask
+        if grad:
+            _, sdf, _, _ = sdf_field.fused_sdf_parts(self.network, x01, comp.xyz_scale, comp.xyz_offset, y,
+                                                     want_g0=False, sdf_only=True)
+        else:
+            sdf = self.network.packed()(x01, comp.xyz_scale, comp.xyz_offset, y, sdf_only=True)
         return sdf.view(*points.shape[:-1], 6)
-
-    _packed_sdf = None
-    _mask_ones = None           # cached "progressive level mask is all ones" (refreshed in update_step)
 
     def forward(self, points, with_grad=True, with_feature=True, with_laplace=False):
         analytic = with_grad and self.grad_type == "analytic"
@@ -203,8 +169,6 @@ class VolumeSDF(nn.Module):
                 elif self.grad_type == "finite_difference":
                     eps = self._finite_difference_eps
                     points_d_sdf = self._fd6_sdf(points_, eps)
-                    if points_d_sdf is None:
-                        points_d_sdf = self._fd6_sdf_train(points_, eps)
                     if points_d_sdf is None:
                         offsets = torch.as_tensor([[eps, 0.0, 0.0], [-eps, 0.0, 0.0], [0.0, eps, 0.0],
                                                    [0.0, -eps, 0.0], [0.0, 0.0, eps], [0.0, 0.0, -eps]]).to(points_)
@@ -304,8 +268,6 @@ class VolumeSDF(nn.Module):
     def update_step(self, epoch, global_step):
         update_module_step(self.encoding, epoch, global_step)
         update_module_step(self.network, epoch, global_step)
-        parts = self._fused_parts()
-        self._mask_ones = None if (parts is None or parts[1] is None) else bool((parts[1] == 1).all())
         if self.grad_type == "finite_difference":
             if isinstance(self.finite_difference_eps, float):
                 self._finite_difference_eps = self.finite_difference_eps

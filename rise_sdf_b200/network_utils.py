@@ -15,7 +15,9 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
+from . import relu_mlp, sdf_field, tc_autograd as tca
 from . import tinycudann as tcnn
+from .fused_mlp import PackedMLP
 
 
 class Config(dict):
@@ -227,57 +229,50 @@ class VanillaMLP(nn.Module):
     _folded = None
 
     def forward(self, x):
-        if x.is_cuda and not torch.is_grad_enabled() and x.dim() == 2 and VanillaMLP.fused_inference:
-            # inference: the whole chain runs in one fused tcgen05 kernel (csrc/mlp_tc.cu)
-            if self._packed is None:
-                from . import sdf_field
-                from .fused_mlp import PackedMLP
-                # SDF-shaped nets run on the features-on-lanes kernel (csrc/sdf_train.cu, ~2x the rows/s of
-                # the generic chain kernel); everything else on csrc/mlp_fwd.cu
-                self._packed = sdf_field.PackedSDF(self) if sdf_field.supports(self) else PackedMLP(self)
-            return self.output_activation(self._packed(x))
-        if x.is_cuda and x.dim() == 2 and VanillaMLP.tc_training and VanillaMLP.fused_training:
-            from . import sdf_field
-            if sdf_field.supports(self):
-                # SDF-shaped net (finite-difference evaluations of the split-sum config): one fused
-                # forward node / one fused backward kernel (csrc/sdf_train.cu)
-                out, _ = sdf_field.fused_sdf(self, x, want_g0=False)
-                return self.output_activation(out)
-            from . import relu_mlp
-            if relu_mlp.supports(self):
-                # ReLU texture networks: one tcgen05 launch per layer, fp16 hi/lo operand-image streams
-                # between layers (csrc/relu_mlp.cu)
-                return self.output_activation(relu_mlp.relu_mlp(self, x))
-        if x.is_cuda and x.dim() == 2 and VanillaMLP.tc_training:
-            # training: every GEMM of forward / backward / double-backward runs on tcgen05
-            # (csrc/gemm_stream.cu) through differentiable primitives; activations stay in torch
-            from . import tc_autograd as tca
-            h = x.float()
+        return self._forward([x])
+
+    def forward_segments(self, segs):
+        """forward(cat(segs, -1)) without materialising the concatenation when a fused kernel takes the
+        segments directly (models/texture.py builds its network inputs with torch.cat)."""
+        return self._forward([s.reshape(-1, s.shape[-1]) for s in segs])
+
+    def _forward(self, segs):
+        """output_activation(network(cat(segs, -1))); the kernels follow from the inputs and the net's shape:
+          CPU or non-2-D input: the nn.Linear stack;
+          no grad: one fused tcgen05 inference launch -- SDF-shaped nets on the features-on-lanes kernels of
+                   sdf_field (~2x the rows/s of the generic chain kernel), every other net on csrc/mlp_fwd.cu;
+          grad:    SDF-shaped nets as one fused forward node / one fused backward kernel (sdf_field), ReLU nets of
+                   width 128 as one tcgen05 launch per layer (relu_mlp), every other shape through the tcgen05 GEMM
+                   primitives of tc_autograd (closed under differentiation; activations stay in torch).
+        mlp_precision picks the operand precision of the sdf_field and relu_mlp kernels.  Only the kernels of ReLU
+        nets read up to 3 input segments; everything else gets their concatenation."""
+        if len(segs) > 1 and (len(segs) > 3 or self.sphere_init or not segs[0].is_cuda):
+            segs = [torch.cat(segs, dim=-1)]
+        x = segs[0]
+        sdf_net = sdf_field.supports(self)
+        if not (x.is_cuda and x.dim() == 2):
+            h = self.layers(x.float())
+        elif not torch.is_grad_enabled():
+            h = self.packed()(x if sdf_net else segs)
+        elif sdf_net:
+            h, _ = sdf_field.fused_sdf(self, x, want_g0=False)
+        elif relu_mlp.supports(self):
+            h = relu_mlp.relu_mlp(self, segs)
+        else:
+            h = (x if len(segs) == 1 else torch.cat(segs, dim=-1)).float()
             ws = self.effective_weights()
             for i, (W, b) in enumerate(ws):
                 h = tca.linear(h, W, b)
                 if i + 1 < len(ws):
                     h = F.softplus(h, beta=100) if self.sphere_init else F.relu(h)
-            return self.output_activation(h)
-        x = self.layers(x.float())
-        return self.output_activation(x)
+        return self.output_activation(h)
 
-    def forward_segments(self, segs):
-        """forward(cat(segs, -1)) without materialising the concatenation when a fused kernel takes the
-        segments directly (models/texture.py builds its network inputs with torch.cat)."""
-        segs = [s.reshape(-1, s.shape[-1]) for s in segs]
-        x0 = segs[0]
-        if x0.is_cuda and len(segs) <= 3 and not self.sphere_init:
-            if not torch.is_grad_enabled() and VanillaMLP.fused_inference:
-                if self._packed is None:
-                    from .fused_mlp import PackedMLP
-                    self._packed = PackedMLP(self)
-                return self.output_activation(self._packed(segs))
-            if torch.is_grad_enabled() and VanillaMLP.tc_training and VanillaMLP.fused_training:
-                from . import relu_mlp
-                if relu_mlp.supports(self):
-                    return self.output_activation(relu_mlp.relu_mlp(self, segs))
-        return self.forward(torch.cat(segs, dim=-1))
+    def packed(self):
+        """The inference launcher with this net's packed weights (PackedSDF for an SDF-shaped net, PackedMLP
+        otherwise), made once; it re-packs when a parameter changes."""
+        if self._packed is None:
+            self._packed = sdf_field.PackedSDF(self) if sdf_field.supports(self) else PackedMLP(self)
+        return self._packed
 
     _packed = None
     # "fp32": every GEMM as three fp16 products of hi|lo operands with fp32 accumulation -- fp32-class, the parity path.
@@ -285,9 +280,6 @@ class VanillaMLP(nn.Module):
     #         the activation-stream bytes (fused SDF field fwd/bwd and the ReLU training nets).  Stated tolerance:
     #         tests/test_gpu_mlp_fp16.py (outputs 2e-3 of their scale; end to end: images 5e-3, gradients 3e-2 rel-L2).
     mlp_precision = "fp32"
-    fused_inference = True      # class-wide switches (tests compare the kernel and the torch paths)
-    tc_training = True
-    fused_training = True
 
     def make_linear(self, dim_in, dim_out, is_first, is_last):
         layer = nn.Linear(dim_in, dim_out, bias=True)

@@ -13,7 +13,7 @@ import ctypes
 import torch
 
 from . import _lib as L
-from .fused_mlp import pack_weight, pad16
+from .fused_mlp import fp16_variant, pack_weight, pad16
 
 NS = 64
 HID = 128
@@ -22,11 +22,6 @@ HID = 128
 def supports(mlp, n_in=None):
     return (not getattr(mlp, "sphere_init", False) and mlp.n_neurons == HID and mlp.n_hidden_layers >= 1
             and (n_in or mlp.dim_in) <= 128 and mlp.dim_out <= 16)
-
-
-def _fp16():
-    from .network_utils import VanillaMLP
-    return 1 if VanillaMLP.mlp_precision == "fp16" else 0
 
 
 def _stream(n_tiles, rows, device, fp16=0):
@@ -50,7 +45,7 @@ class _ReluMLP(torch.autograd.Function):
         out = torch.empty(S, n_out, device=dev, dtype=torch.float32)
         blobs = [pack_weight(W, HID if i + 1 < len(Ws) else 16, k0 if i == 0 else HID) for i, W in enumerate(Ws)]
         acts = []                                                        # a_0 (input image stream), a_1, ..., a_L
-        fp16 = ctx.fp16 = _fp16()
+        fp16 = ctx.fp16 = fp16_variant()
         if S:
             a0 = _stream(n_tiles, k0, dev, fp16)
             acts.append(a0)
@@ -85,8 +80,8 @@ class _ReluMLP(torch.autograd.Function):
             # `once_differentiable` only raises when the cotangent requires grad and otherwise hands back constants:
             # a caller differentiating through this backward (create_graph=True) would silently lose terms.  Nothing
             # on the render path does (the texture nets are first order), so refuse loudly.
-            raise NotImplementedError("relu_mlp is first-order only: VanillaMLP.fused_training = False routes the "
-                                      "network through the twice-differentiable GEMM primitives (tc_autograd)")
+            raise NotImplementedError("relu_mlp is first-order only: build a network that must be differentiated "
+                                      "twice from tc_autograd.linear, which is closed under differentiation")
         params = ctx.saved_tensors
         Ws, bs = params[0::2], params[1::2]
         S, dev = ctx.S, g_out.device

@@ -15,15 +15,9 @@ import ctypes
 import torch
 
 from . import _lib as L
-from .fused_mlp import pack_weight
+from .fused_mlp import fp16_variant, pack_weight
 
 HID, KP = 128, 48
-
-
-def _fp16():
-    """The reduced-precision MLP variant (VanillaMLP.mlp_precision = "fp16"): single fp16 plane, one product."""
-    from .network_utils import VanillaMLP
-    return 1 if VanillaMLP.mlp_precision == "fp16" else 0
 
 
 def supports(mlp, dim_in=None):
@@ -40,8 +34,23 @@ def _net_struct(W1, b1, W2, b2, W3, b3):
     c.w1_blob, c.w2_blob, c.w3_blob = (k.data_ptr() for k in keep[:3])
     c.b1, c.b2, c.b3, c.w3_row0 = (k.data_ptr() for k in keep[3:])
     c.n_in, c.n_out = W1.shape[1], W3.shape[0]
-    c.precision = _fp16()
+    c.precision = fp16_variant()
     return c, keep
+
+
+def _forward(net, in0, scale0, shift0, in1, out, sdf, g0a=None, g0b=None):
+    """Launch the forward of S > 0 samples: sdf-only (out is None) in fp32 on the TMEM-operand kernel
+    (rsdf_sdf_mlp_eval), everything else on rsdf_sdf_mlp_fwd.  Measured at 3.34 M evaluations on a B200 (DESIGN.md
+    §4): sdf-only 0.79 ms on the TMEM-operand kernel vs 1.14 ms on the shared-memory-operand one; the full 48-wide
+    output 1.50 vs 1.38 ms."""
+    S, w0 = in0.shape
+    w1 = 0 if in1 is None else in1.shape[1]
+    if out is None and not net.precision:
+        L.call("rsdf_sdf_mlp_eval", ctypes.byref(net), L.ptr(in0), w0, float(scale0), float(shift0), L.ptr(in1), w1, S,
+               L.ptr(sdf), L.stream())
+    else:
+        L.call("rsdf_sdf_mlp_fwd", ctypes.byref(net), L.ptr(in0), w0, float(scale0), float(shift0), L.ptr(in1), w1, S,
+               L.ptr(out), L.ptr(sdf), L.ptr(g0a), L.ptr(g0b), L.stream())
 
 
 def _absmax(tensors, dev):
@@ -77,12 +86,8 @@ class _FusedSDF(torch.autograd.Function):
         sdf = torch.empty(S, device=dev, dtype=torch.float32)
         g0a = torch.empty(S, w0, device=dev, dtype=torch.float32) if want_g0 else None
         g0b = torch.empty(S, w1, device=dev, dtype=torch.float32) if (want_g0 and w1) else None
-        if S and sdf_only and not net.precision and PackedSDF.tensor_memory_operands:
-            L.call("rsdf_sdf_mlp_eval", ctypes.byref(net), L.ptr(in0), w0, float(scale0), float(shift0), L.ptr(in1), w1, S,
-                   None, L.ptr(sdf), L.stream())
-        elif S:
-            L.call("rsdf_sdf_mlp_fwd", ctypes.byref(net), L.ptr(in0), w0, float(scale0), float(shift0), L.ptr(in1), w1,
-                   S, L.ptr(out), L.ptr(sdf), L.ptr(g0a), L.ptr(g0b), L.stream())
+        if S:
+            _forward(net, in0, scale0, shift0, in1, out, sdf, g0a, g0b)
         ctx.save_for_backward(in0, in1, W1, b1, W2, b2, W3, b3)
         ctx.net, ctx.keep, ctx.scale0, ctx.shift0, ctx.want_g0 = net, keep, float(scale0), float(shift0), bool(want_g0)
         empty = []
@@ -196,7 +201,7 @@ class PackedSDF:
         self.mlp, self._key, self._net, self._keep = mlp, None, None, None
 
     def _struct(self):
-        key = tuple((p.data_ptr(), p._version) for p in self.mlp.parameters()) + (_fp16(),)
+        key = tuple((p.data_ptr(), p._version) for p in self.mlp.parameters()) + (fp16_variant(),)
         if key != self._key:
             with torch.no_grad():
                 (W1, b1), (W2, b2), (W3, b3) = self.mlp.effective_weights()
@@ -214,17 +219,5 @@ class PackedSDF:
         out = None if sdf_only else torch.empty(S, self.mlp.dim_out, device=in0.device, dtype=torch.float32)
         sdf = torch.empty(S, device=in0.device, dtype=torch.float32) if sdf_only else None
         if S:
-            # measured (3.34 M evaluations): sdf-only 0.79 ms on the TMEM-operand kernel vs 1.14 ms on the smem-operand
-            # one; full 48-wide output 1.50 vs 1.38 ms (row-per-thread output stores) -> each variant on its faster kernel
-            if PackedSDF.tensor_memory_operands and (sdf_only or PackedSDF.tensor_memory_full_output) and not _fp16():
-                L.call("rsdf_sdf_mlp_eval", ctypes.byref(self._struct()), L.ptr(in0), in0.shape[1], float(scale0),
-                       float(shift0), L.ptr(in1), 0 if in1 is None else in1.shape[1], S, L.ptr(out), L.ptr(sdf), L.stream())
-            else:
-                L.call("rsdf_sdf_mlp_fwd", ctypes.byref(self._struct()), L.ptr(in0), in0.shape[1], float(scale0),
-                       float(shift0), L.ptr(in1), 0 if in1 is None else in1.shape[1], S, L.ptr(out), L.ptr(sdf), None,
-                       None, L.stream())
+            _forward(self._struct(), in0, scale0, shift0, in1, out, sdf)
         return sdf if sdf_only else out
-
-    # True: csrc/sdf_eval_ts.cu (A operand in tensor memory); False: sdf_eval_kernel of csrc/sdf_train.cu
-    tensor_memory_operands = True
-    tensor_memory_full_output = False

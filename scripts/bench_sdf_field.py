@@ -29,9 +29,7 @@ f_fwd = 2 * (35 * 128 + 128 * 128 + 128 * 48)
 f_chain = 2 * (128 * 128 + 128 * 35)
 t("fwd (out only)", lambda: L.call("rsdf_sdf_mlp_fwd", ctypes.byref(net), L.ptr(x01), 3, 2.0, -1.0, L.ptr(enc), 32, S, L.ptr(out), None, None, None, st), f_fwd)
 sdf1 = torch.empty(S, device='cuda')
-t("eval TS (out)", lambda: L.call("rsdf_sdf_mlp_eval", ctypes.byref(net), L.ptr(x01), 3, 2.0, -1.0, L.ptr(enc), 32, S, L.ptr(out), None, st), f_fwd)
-t("eval TS (sdf only)", lambda: L.call("rsdf_sdf_mlp_eval", ctypes.byref(net), L.ptr(x01), 3, 2.0, -1.0, L.ptr(enc), 32, S, None, L.ptr(sdf1), st), f_fwd)
-t("eval SS (sdf only)", lambda: L.call("rsdf_sdf_mlp_fwd", ctypes.byref(net), L.ptr(x01), 3, 2.0, -1.0, L.ptr(enc), 32, S, None, L.ptr(sdf1), None, None, st), f_fwd)
+t("eval TS (sdf only)", lambda: L.call("rsdf_sdf_mlp_eval", ctypes.byref(net), L.ptr(x01), 3, 2.0, -1.0, L.ptr(enc), 32, S, L.ptr(sdf1), st), f_fwd)
 t("fwd (out + g0)", lambda: L.call("rsdf_sdf_mlp_fwd", ctypes.byref(net), L.ptr(x01), 3, 2.0, -1.0, L.ptr(enc), 32, S, L.ptr(out), None, L.ptr(g0a), L.ptr(g0b), st), f_fwd + f_chain)
 f_bwd = 2 * (35 * 128 + 128 * 128) + f_chain + 2 * (35 * 128 + 128 * 128 + 48 * 128 + 128 * 128 + 128 * 35) + 2 * (2 * 35 * 128 + 2 * 128 * 128 + 48 * 128)
 t("absmax2", lambda: L.call("rsdf_absmax2", L.ptr(go), go.numel(), L.ptr(gg), gg.numel(), L.ptr(amax), 0, st), 0)

@@ -1,7 +1,6 @@
 import sys, time, numpy as np, torch
 sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tests')
 from rise_sdf_b200 import synthetic as syn
-from rise_sdf_b200.network_utils import VanillaMLP
 from rise_sdf_b200.split_mixed_occ import SplitMixedOCCModel, split_mixed_occ_config
 from oracle import split as osplit
 from helpers import split_oracle_params
@@ -21,12 +20,10 @@ P = split_oracle_params(m)
 # use the product's own prefiltered maps in the oracle so that only the render path is compared
 P.specular = [t.detach().cpu() for t in m.emitter.specular]; P.diffuse = m.emitter.diffuse.detach().cpu()
 ref = osplit.forward(P, rays, grid.numpy(), m.render_step_size, stage=1, relighting=False, background=bg)
-for fused in (True, False):
-    VanillaMLP.fused_inference = fused
-    with torch.no_grad(): out = m(rays.cuda(), relighting=False)
-    print('fused', fused, 'samples', ref['num_samples'], int(out['num_samples'].sum()))
-    for k in ('comp_rgb', 'comp_rgb_phys', 'comp_normal', 'opacity', 'depth', 'comp_albedo', 'comp_spec_rgb'):
-        a, b = out[k].cpu().numpy(), ref[k].numpy(); e = np.abs(a - b).max(-1)
-        print(f'  {k:18s} max {e.max():.2e} mean {e.mean():.2e} p99 {np.quantile(e, .99):.2e} argmax {e.argmax()} n>1e-3 {(e>1e-3).sum()}')
-    bad = np.abs(out['comp_rgb'].cpu().numpy() - ref['comp_rgb'].numpy()).max(-1).argmax()
-    print('  worst ray', bad, 'opacity', float(out['opacity'][bad]), float(ref['opacity'][bad]), 'in valid(ref)', bad in ref['valid_indices'].tolist())
+with torch.no_grad(): out = m(rays.cuda(), relighting=False)
+print('samples', ref['num_samples'], int(out['num_samples'].sum()))
+for k in ('comp_rgb', 'comp_rgb_phys', 'comp_normal', 'opacity', 'depth', 'comp_albedo', 'comp_spec_rgb'):
+    a, b = out[k].cpu().numpy(), ref[k].numpy(); e = np.abs(a - b).max(-1)
+    print(f'  {k:18s} max {e.max():.2e} mean {e.mean():.2e} p99 {np.quantile(e, .99):.2e} argmax {e.argmax()} n>1e-3 {(e>1e-3).sum()}')
+bad = np.abs(out['comp_rgb'].cpu().numpy() - ref['comp_rgb'].numpy()).max(-1).argmax()
+print('  worst ray', bad, 'opacity', float(out['opacity'][bad]), float(ref['opacity'][bad]), 'in valid(ref)', bad in ref['valid_indices'].tolist())

@@ -5,6 +5,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+from rise_sdf_b200 import _lib as L
 from rise_sdf_b200 import sdf_field
 from rise_sdf_b200.network_utils import VanillaMLP
 
@@ -106,23 +107,19 @@ def test_plain_input_segment():
         assert rel(a, b) <= 2e-5
 
 
-@pytest.mark.parametrize("ts", [True, False])
-@pytest.mark.parametrize("S", [1, 64, 65, 129, 2 * 148 * 128 + 77])
-def test_inference_kernel_out_and_sdf_only(S, ts):
-    """PackedSDF (two-group inference kernel): full output == the training forward, and the sdf-only variant
-    (third GEMM replaced by an fp32 dot product) == channel 0, both against fp64."""
+@pytest.mark.parametrize("S", [1, 63, 64, 65, 127, 128, 129, 257, 148 * 128 + 1, 2 * 148 * 128 + 77])
+def test_inference_kernel_out_and_sdf_only(S):
+    """PackedSDF: the full output (two-group shared-memory-operand kernel, two segments and one) and the sdf-only
+    output (TMEM-operand kernel, output layer replaced by an fp32 dot product) against fp64."""
     m = make_mlp(seed=3)
     g = torch.Generator().manual_seed(S)
     x01 = torch.rand(S, 3, generator=g).cuda()
     enc = (torch.randn(S, 32, generator=g) * 0.1).cuda()
-    sdf_field.PackedSDF.tensor_memory_operands = ts       # both inference kernels: TMEM-operand and smem-operand
-    sdf_field.PackedSDF.tensor_memory_full_output = ts
     packed = sdf_field.PackedSDF(m)
     out = packed(x01, 2.0, -1.0, enc)
     sdf = packed(x01, 2.0, -1.0, enc, sdf_only=True)
     h0 = torch.cat([x01 * 2 - 1, enc], -1)
     out1 = packed(h0)                                     # single input segment
-    sdf_field.PackedSDF.tensor_memory_operands, sdf_field.PackedSDF.tensor_memory_full_output = True, False
     ro, _ = ref64(m, x01.double(), enc.double(), want_g0=False)
     assert out.shape == (S, 48) and sdf.shape == (S,)
     assert rel(out, ro.detach()) <= 2e-6 and rel(out1, ro.detach()) <= 2e-6
@@ -187,3 +184,44 @@ def test_sdf_only_training_node(S):
     assert len(pa) == len(pb) > 0
     for x, y in zip(pa, pb):
         assert rel(x, y) <= 1e-5
+
+
+@pytest.mark.parametrize("precision", ["fp32", "fp16"])
+def test_forward_kernel_selection(precision, monkeypatch):
+    """Which entry point each forward runs: the SDF field's sdf-only output in fp32 on the TMEM-operand kernel, every
+    other SDF-field forward on rsdf_sdf_mlp_fwd; VanillaMLP under grad by net shape (fused SDF node, per-layer ReLU
+    kernels, tc_autograd GEMMs for any other shape) and under no_grad on the fused inference kernels."""
+    monkeypatch.setattr(VanillaMLP, "mlp_precision", precision)
+    calls = []
+    real = L.call
+    monkeypatch.setattr(L, "call", lambda name, *a: (calls.append(name), real(name, *a))[1])
+
+    def run(fn, *a, **k):
+        calls.clear()
+        fn(*a, **k)
+        return [c for c in calls if c not in ("rsdf_mlp_pack_weight", "rsdf_absmax2")]
+
+    sdf_only_kernel = "rsdf_sdf_mlp_eval" if precision == "fp32" else "rsdf_sdf_mlp_fwd"
+    m = make_mlp(seed=5)
+    g = torch.Generator().manual_seed(5)
+    x01 = torch.rand(300, 3, generator=g).cuda()
+    enc = (torch.randn(300, 32, generator=g) * 0.1).cuda()
+    packed = sdf_field.PackedSDF(m)
+    assert run(packed, x01, 2.0, -1.0, enc) == ["rsdf_sdf_mlp_fwd"]
+    assert run(packed, x01, 2.0, -1.0, enc, sdf_only=True) == [sdf_only_kernel]
+    assert run(sdf_field.fused_sdf_parts, m, x01, 2.0, -1.0, enc, want_g0=False, sdf_only=True) == [sdf_only_kernel]
+    assert run(sdf_field.fused_sdf_parts, m, x01, 2.0, -1.0, enc, want_g0=False) == ["rsdf_sdf_mlp_fwd"]
+
+    h0 = torch.cat([x01 * 2 - 1, enc], -1)
+    relu = VanillaMLP(67, 3, {"n_neurons": 128, "n_hidden_layers": 4, "output_activation": "none"}).cuda()
+    narrow = VanillaMLP(35, 48, {"n_neurons": 64, "n_hidden_layers": 2, "sphere_init": True, "weight_norm": True,
+                                 "output_activation": "none"}).cuda()
+    segs = [torch.randn(300, 48, device="cuda"), torch.randn(300, 16, device="cuda"), torch.randn(300, 3, device="cuda")]
+    assert run(m, h0) == ["rsdf_sdf_mlp_fwd"]
+    assert run(relu, torch.cat(segs, -1)) == ["rsdf_relu_layer_fwd"] * 5
+    assert run(relu.forward_segments, segs) == ["rsdf_relu_layer_fwd"] * 5
+    assert run(narrow, h0) == ["rsdf_mm_stream"] * 3
+    with torch.no_grad():
+        assert run(m, h0) == ["rsdf_sdf_mlp_fwd"]
+        assert run(relu.forward_segments, segs) == ["rsdf_mlp_fwd"]
+        assert run(narrow, h0) == ["rsdf_mlp_fwd"]

@@ -176,7 +176,6 @@ def test_fused_analytic_field_is_differentiable_wrt_the_points():
     one fused MLP node -> dy_dx^T g0) must give the same first and second-order gradients as the op-by-op autograd
     path (tcnn.Encoding double backward + the MLP's twice-differentiable GEMM primitives) and as float64 torch."""
     from oracle import fields as ofields
-    from rise_sdf_b200.geometry import VolumeSDF
     m = split_model(64).train()
     geo = m.geometry
     g = torch.Generator().manual_seed(3)
@@ -186,16 +185,12 @@ def test_fused_analytic_field_is_differentiable_wrt_the_points():
 
     def run(fused):
         p = pts.clone().requires_grad_(True)
-        VolumeSDF.fused_analytic = fused
-        try:
-            if fused:
-                sdf, grad, feat = geo._forward_fused_analytic(p, geo._fused_parts())
-            else:
-                x01 = (p + 1.5) * float(np.float32(1.0) / np.float32(3.0))
-                sdf = geo.network(geo.encoding(x01))[..., 0]
-                (grad,) = torch.autograd.grad(sdf, p, torch.ones_like(sdf), create_graph=True)
-        finally:
-            VolumeSDF.fused_analytic = True
+        if fused:
+            sdf, grad, feat = geo._forward_fused_analytic(p, geo._fused_parts())
+        else:
+            x01 = (p + 1.5) * float(np.float32(1.0) / np.float32(3.0))
+            sdf = geo.network(geo.encoding(x01))[..., 0]
+            (grad,) = torch.autograd.grad(sdf, p, torch.ones_like(sdf), create_graph=True)
         loss = (grad * c).sum() + ((grad.norm(dim=-1) - 1.0) ** 2).mean() + sdf.mean()
         return [sdf, grad] + list(torch.autograd.grad(loss, [p] + params))
 
