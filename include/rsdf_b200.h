@@ -496,6 +496,25 @@ typedef struct rsdf_adam_groups {
 int rsdf_adam_step(float *params, float *grads, float *exp_avg, float *exp_avg_sq, long long n,
                    const rsdf_adam_groups *groups_host, int zero_grad, void *stream);
 
+/* ---------------------------------------------------------------- isosurface mesh (SURVEY §8f f4) */
+/* PyMCubes `mcubes.marching_cubes(volume, iso)` as `MarchingCubeHelper` calls it (models/geometry.py:60, there on
+ * `-level`): marching cubes over a contiguous fp32 volume[nx, ny, nz] (x-major), nx, ny, nz >= 2 and
+ * 3 * nx * ny * nz <= INT32_MAX (the number of grid edges, which bounds every vertex id), else -1.
+ *   - a grid vertex is inside when value > iso, value = negate ? -volume : volume (no negated copy is made);
+ *   - one welded vertex per grid edge whose ends differ, interpolated once from its lower end a:
+ *     t = (iso - va) / (vb - va), p = pa + t (pb - pa), fp32; negating both volume and iso gives the same bits;
+ *   - faces are wound so that right-hand normals point towards decreasing value (out of the object for -sdf);
+ *   - vertex order: lower grid corner's linear index, then axis x < y < z; face order: the cell's linear index, then
+ *     triangle-table order (rise_sdf_b200/csrc/mcubes_table.cuh, at most 5 triangles per cell).
+ * Output is deterministic.  Count pass: fills `scratch` and writes totals2[0] = V, totals2[1] = F (device int64; the
+ * caller reads them back once to size the outputs).  scratch: 1048 * ceil(nx * ny * nz / 2048) bytes, 16-byte
+ * aligned (0.51 bytes per grid vertex).  Emit pass (same volume, iso, negate and scratch): verts float32[V, 3] in
+ * index space, faces int64[F, 3]; call it only when V > 0. */
+int rsdf_mc_count(const float *volume, int nx, int ny, int nz, float iso, int negate, void *scratch,
+                  int64_t *totals2, void *stream);
+int rsdf_mc_emit(const float *volume, int nx, int ny, int nz, float iso, int negate, const void *scratch,
+                 float *verts, int64_t *faces, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -136,6 +136,8 @@ _SIGS = {
     "rsdf_vis_round_fill": [c_p, c_p, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p, c_p],
     "rsdf_vis_round_scatter": [c_p, c_p, ctypes.c_longlong, ctypes.c_longlong, c_p, c_p, c_p],
     "rsdf_tc_gemm_test": [c_i, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_p],
+    "rsdf_mc_count": [c_p, c_i, c_i, c_i, c_f, c_i, c_p, c_p, c_p],
+    "rsdf_mc_emit": [c_p, c_i, c_i, c_i, c_f, c_i, c_p, c_p, c_p, c_p],
 }
 
 
@@ -181,7 +183,7 @@ def stream():
 
 # kernels launched per C-ABI entry point (for bench.py's gpu_launches count)
 LAUNCHES = {"rsdf_march_count": 4, "rsdf_march_count_keep": 4, "rsdf_sdf_reg_fwd": 2, "rsdf_neus_loss_fwd": 2,
-            "rsdf_occ_update": 2, "rsdf_occ_threshold": 3}
+            "rsdf_occ_update": 2, "rsdf_occ_threshold": 3, "rsdf_mc_count": 2}
 SDF_REG_BLOCKS = 1184
 LOSS_BLOCKS = 296
 STATS = {"enabled": False, "launches": 0, "timed": set(), "events": {}}

@@ -277,6 +277,24 @@ def save_exr_or_hdr(path, img):
         raise RuntimeError(f"OpenCV could not write {path}")
 
 
+def save_mesh_obj(path, v_pos, t_pos_idx, v_rgb=None):
+    """Wavefront OBJ of a triangle mesh (`VolumeSDF.isosurface` / `NeuSModel.export`): one `v x y z` line per vertex,
+    `v x y z r g b` with vertex colours in [0, 1], then one 1-based `f a b c` line per face -- the plain layout mesh
+    viewers and trimesh read."""
+    host = lambda t: t.detach().cpu().numpy() if hasattr(t, "detach") else np.asarray(t)
+    v = host(v_pos).astype(np.float64).reshape(-1, 3)
+    f = host(t_pos_idx).astype(np.int64).reshape(-1, 3) + 1
+    if v_rgb is not None:
+        v = np.concatenate([v, host(v_rgb).astype(np.float64).reshape(-1, 3)], 1)
+    vfmt = "v" + " %.9g" * v.shape[1]                 # 9 significant digits: float32 round-trips exactly
+    with open(path, "w") as fh:
+        if len(v):
+            np.savetxt(fh, v, fmt=vfmt)
+        if len(f):
+            np.savetxt(fh, f, fmt="f %d %d %d")
+    return path
+
+
 def save_level_grid(path, level):
     """The isosurface level grid (VolumeSDF.isosurface_level) as a raw .npy volume for an external marching-cubes tool."""
     import numpy as np

@@ -2,7 +2,8 @@
 geometry of both configs) with the reference's call signature
     forward(points, with_grad=True, with_feature=True, with_laplace=False)
 (models/geometry.py:206-292).  Encoding and scan kernels come from librsdf_b200.so.
-Isosurface extraction (models/geometry.py:31-191) is out of scope (SURVEY.md §2.1 row 6).
+Isosurface extraction (models/geometry.py:31-112) runs on the device: the level grid on the sdf-only inference kernel,
+marching cubes on csrc/mcubes.cu (`MarchingCubeHelper`, `VolumeSDF.isosurface`).
 """
 import numpy as np
 import torch
@@ -26,6 +27,23 @@ def contract_to_unisphere(x, radius, contraction_type):
     if contraction_type == ContractionType.AABB:
         return scale_anything(x, (-radius, radius), (0, 1))
     raise NotImplementedError("unbounded contraction belongs to the learned-background branch")
+
+
+class MarchingCubeHelper(nn.Module):
+    """models/geometry.py:31-68 (`isosurface.method: mc`): the surface `-level = threshold` of a [res, res, res] level
+    grid, vertices scaled to [0, 1].  PyMCubes on `.cpu()` copies there, rise_sdf_b200.mcubes on the device here: the
+    negation is folded into the kernel, and the outputs stay on the level's device."""
+
+    def __init__(self, resolution):
+        super().__init__()
+        self.resolution = resolution
+
+    def forward(self, level, threshold=0.0):
+        from .mcubes import marching_cubes
+        r = self.resolution
+        level = level.float().view(r, r, r)
+        verts, faces = marching_cubes(level, threshold, negate=True)
+        return {"v_pos": verts / (r - 1.0), "t_pos_idx": faces}
 
 
 class VolumeSDF(nn.Module):
@@ -264,6 +282,28 @@ class VolumeSDF(nn.Module):
         bmin, bmax = mn * (hi - lo) + lo, mx * (hi - lo) + lo
         pad = (bmax - bmin) * 0.1                                                  # :106-107
         return (bmin - pad).clamp(-self.radius, self.radius), (bmax + pad).clamp(-self.radius, self.radius)
+
+    @torch.no_grad()
+    def isosurface(self, resolution=512, threshold=0.0):
+        """`BaseImplicitGeometry.isosurface` (models/geometry.py:76-112): a coarse mesh over the whole [-radius, radius]^3
+        box places a fine grid on its bounding box padded by 10 % and clamped to the radius; returns the fine mesh
+        {'v_pos' [V,3] world space, 't_pos_idx' [F,3] int64} on the device.  Both level grids share one buffer.  An
+        empty coarse mesh (no surface in the box) gives an empty mesh."""
+        helper = MarchingCubeHelper(resolution)
+        dev = next(self.parameters()).device
+        buf = torch.empty(resolution ** 3, device=dev, dtype=torch.float32)
+        r = self.radius
+        vmin = torch.full((3,), -r, dtype=torch.float32, device=dev)
+        vmax = torch.full((3,), r, dtype=torch.float32, device=dev)
+        for fine in (False, True):
+            level = self.isosurface_level(resolution, vmin, vmax, out=buf)
+            mesh = helper(level, threshold)
+            mesh["v_pos"] = mesh["v_pos"] * (vmax - vmin) + vmin           # scale_anything((0, 1) -> (vmin, vmax))
+            if fine or mesh["v_pos"].shape[0] == 0:
+                return mesh
+            lo, hi = mesh["v_pos"].amin(dim=0), mesh["v_pos"].amax(dim=0)
+            vmin = (lo - (hi - lo) * 0.1).clamp(-r, r)
+            vmax = (hi + (hi - lo) * 0.1).clamp(-r, r)
 
     def update_step(self, epoch, global_step):
         update_module_step(self.encoding, epoch, global_step)

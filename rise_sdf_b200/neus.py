@@ -321,6 +321,22 @@ class NeuSModel(nn.Module):
     def regularizations(self, out):
         return {}
 
+    @torch.no_grad()
+    def export(self, chunk_size=1 << 20, resolution=512, threshold=0.0):
+        """`NeuSModel.export` of models/neus.py (instant-nsr-pl), with vertex colours: the isosurface mesh, then the
+        geometry at its vertices (chunked, analytic normals), normal = normalize(grad) and
+        v_rgb = texture(feature, -normal, normal), i.e. the colour seen looking straight at the surface.  Returns
+        {'v_pos', 't_pos_idx', 'v_rgb'} on the device (formats.save_mesh_obj writes it)."""
+        mesh = self.geometry.isosurface(resolution, threshold)
+        v_pos = mesh["v_pos"]
+        if v_pos.shape[0] == 0:
+            mesh["v_rgb"] = torch.zeros(0, 3, device=v_pos.device)
+            return mesh
+        _, sdf_grad, feature = chunk_batch(self.geometry, chunk_size, False, v_pos, with_grad=True, with_feature=True)
+        normal = F.normalize(sdf_grad, p=2, dim=-1)
+        mesh["v_rgb"] = self.texture(feature, -normal, normal)
+        return mesh
+
 
 def chunk_batch(func, chunk_size, move_to_cpu, *args, **kwargs):
     """models/utils.py:14-51: run `func` over the leading dim in chunks and merge dict/tuple/
