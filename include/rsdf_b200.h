@@ -514,6 +514,27 @@ int rsdf_mc_count(const float *volume, int nx, int ny, int nz, float iso, int ne
                   int64_t *totals2, void *stream);
 int rsdf_mc_emit(const float *volume, int nx, int ny, int nz, float iso, int negate, const void *scratch,
                  float *verts, int64_t *faces, void *stream);
+/* The same mesher over one x-slab of a volume of nx layers, so that a volume of any size can be meshed in pieces that
+ * each meet the int32 bound, with output identical to the dense call's.  `slab` is the contiguous sub-volume
+ * [p, ny, nz] that starts at global layer x0; its first `own` layers (1 <= own <= p) are owned, the others are a
+ * read-only halo.  The caller presents p = min(own + 2, nx - x0) layers: one halo layer closes the cells of the last
+ * owned layer, and a second is needed for the x-edge bits of the first halo layer, on which the ids of the next
+ * slab's first-layer vertices depend.  p >= 2, ny, nz >= 2, 3 * p * ny * nz <= INT32_MAX (else -1); slabs are
+ * x0 = 0, x0 + own(0), ... up to nx.
+ *   - Count pass: fills `scratch` over all p layers (1048 * ceil(p * ny * nz / 2048) bytes, 16-byte aligned) and
+ *     writes totals2[0] = V, the vertices owned by grid vertices of local layers [0, own), and totals2[1] = F, the
+ *     triangles of cells whose lower corner lies in local layers [0, own).
+ *   - Emit pass (same slab, p, ny, nz, own, iso, negate and scratch): verts float32[V, 3] at global index-space
+ *     positions (x0 + x, exact while x0 + p <= 2^24; x0, vbase >= 0), faces int64[F, 3] with vertex ids
+ *     vbase + local id.
+ *     With vbase = the sum of V over the slabs before this one, the concatenation of all slabs' outputs in x order
+ *     is the dense call's output, bit for bit; a face of the last owned layer may use a vertex that the next slab
+ *     emits.  Call it only when V > 0 (F > 0 implies V > 0).
+ * rsdf_mc_count / rsdf_mc_emit are the slab x0 = 0, own = p = nx, vbase = 0. */
+int rsdf_mc_slab_count(const float *slab, int p, int ny, int nz, int own, float iso, int negate, void *scratch,
+                       int64_t *totals2, void *stream);
+int rsdf_mc_slab_emit(const float *slab, int p, int ny, int nz, int own, int x0, int64_t vbase, float iso, int negate,
+                      const void *scratch, float *verts, int64_t *faces, void *stream);
 
 #ifdef __cplusplus
 }

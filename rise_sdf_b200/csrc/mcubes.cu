@@ -19,6 +19,17 @@
 //          is no per-cell offset array, no atomic and no hash map.
 // Scratch: 1048 bytes per tile (0.51 bytes per grid vertex).  Vertex ids and linear indices are int32: the caller
 // guarantees 3 * nx * ny * nz <= INT32_MAX (every vertex id is below the edge count); triangle offsets are int64.
+//
+// Slabs.  The same passes run on a sub-volume of p consecutive x layers starting at global layer x0, of which the
+// first `own` are owned and the rest are a read-only halo (p = min(own + 2, nx - x0)).  Both orders are x-major, so
+// the owned vertices of a slab are a prefix of its local vertex order and its owned cells a prefix of its cells:
+//   count  fills the bit planes of all p layers as above, counts the triangles of owned cells only, and reports
+//          V = the local id of the first vertex of layer `own` (the owned vertices) and F;
+//   emit   writes owned vertices at x0 + x and owned cells' triangles with ids vbase + local id.
+// A triangle of the last owned layer may use an edge owned by layer `own`, the next slab's first layer.  Its local id
+// here is V + (crossing edges of layer `own` before it), and it is exactly what the next slab assigns, with
+// vbase(k + 1) = vbase(k) + V(k), as long as layer `own`'s bits are right: its x bits need layer own + 1, hence the
+// second halo layer.  The dense volume is the slab x0 = 0, own = p = nx, vbase = 0.
 #include "common.cuh"
 #include "mcubes_table.cuh"
 
@@ -33,7 +44,8 @@ constexpr long long MC_SCRATCH_PER_TILE = MC_WORDS * 16 + 3 * 8;   // words, vba
 
 struct McVolume {
     const float *v;
-    int nx, ny, nz, syz, n;
+    int nx, ny, nz, syz, n;   // nx: layers present; n = nx * syz
+    int n_own;                // owned grid vertices: own * syz, a prefix of the n
     float iso;
     int negate;
 };
@@ -114,7 +126,7 @@ __global__ void __launch_bounds__(MC_T) mc_count_kernel(const McVolume g, uint4 
         int x, y, z, cs = 0;
         unsigned e = 0;
         if (i < g.n) classify(g, i, x, y, z, e, cs);
-        ntri += RSDF_MC_NTRI[cs];
+        if (i < g.n_own) ntri += RSDF_MC_NTRI[cs];
         const unsigned bx = __ballot_sync(0xffffffffu, e & 1u);
         const unsigned by = __ballot_sync(0xffffffffu, e & 2u);
         const unsigned bz = __ballot_sync(0xffffffffu, e & 4u);
@@ -150,8 +162,10 @@ __global__ void __launch_bounds__(MC_T) mc_count_kernel(const McVolume g, uint4 
     }
 }
 
-// one block: thread t scans tiles [t * per, (t + 1) * per) sequentially around one block-wide scan
+// one block: thread t scans tiles [t * per, (t + 1) * per) sequentially around one block-wide scan.  totals2[0] is
+// the number of owned vertices: the local id of grid vertex n_own (all vertices when n_own == n).
 __global__ void __launch_bounds__(MC_SCAN_T, 1) mc_scan_kernel(const int2 *__restrict__ tile_tot, int nt,
+                                                            const uint4 *__restrict__ words, int n, int n_own,
                                                             long long *__restrict__ vbase,
                                                             long long *__restrict__ fbase,
                                                             long long *__restrict__ totals2) {
@@ -174,8 +188,15 @@ __global__ void __launch_bounds__(MC_SCAN_T, 1) mc_scan_kernel(const int2 *__res
         ev += c.x;
         ef += c.y;
     }
+    __syncthreads();                                   // vbase of every tile written
     if (threadIdx.x == 0) {
-        totals2[0] = sv_.total;
+        long long v_own = sv_.total;
+        if (n_own < n) {
+            const uint4 w = words[n_own >> 5];
+            const unsigned lt = (1u << (n_own & 31)) - 1u;
+            v_own = vbase[n_own / MC_TILE] + w.w + __popc(w.x & lt) + __popc(w.y & lt) + __popc(w.z & lt);
+        }
+        totals2[0] = v_own;
         totals2[1] = sf_.total;
     }
 }
@@ -191,7 +212,9 @@ __device__ __forceinline__ int vertex_id(const uint4 *__restrict__ words, const 
     return id;
 }
 
-__global__ void __launch_bounds__(MC_T) mc_emit_kernel(const McVolume g, const uint4 *__restrict__ words,
+// launched over the tiles that hold owned vertices; x0: global layer of local layer 0, vid0: global id of local id 0
+__global__ void __launch_bounds__(MC_T) mc_emit_kernel(const McVolume g, int x0, long long vid0,
+                                                       const uint4 *__restrict__ words,
                                                        const long long *__restrict__ vbase,
                                                        const long long *__restrict__ fbase, float *__restrict__ verts,
                                                        long long *__restrict__ faces) {
@@ -202,7 +225,7 @@ __global__ void __launch_bounds__(MC_T) mc_emit_kernel(const McVolume g, const u
         const int i = base + k * MC_T + threadIdx.x;
         int x = 0, y = 0, z = 0, cs = 0;
         unsigned e = 0;
-        if (i < g.n) classify(g, i, x, y, z, e, cs);
+        if (i < g.n_own) classify(g, i, x, y, z, e, cs);
         if (e) {
             int id = vertex_id(words, vbase, i, 0);
             const float va = value_at(g, i);
@@ -212,7 +235,7 @@ __global__ void __launch_bounds__(MC_T) mc_emit_kernel(const McVolume g, const u
                 if (!((e >> a) & 1u)) continue;
                 const float vb = value_at(g, i + step[a]);
                 const float t = __fdiv_rn(__fsub_rn(g.iso, va), __fsub_rn(vb, va));
-                float p[3] = {(float)x, (float)y, (float)z};
+                float p[3] = {(float)(x0 + x), (float)y, (float)z};      // exact while x0 + x <= 2^24
                 p[a] = __fadd_rn(p[a], t);
                 float *o = verts + 3 * (long long)id;
                 o[0] = p[0];
@@ -229,20 +252,22 @@ __global__ void __launch_bounds__(MC_T) mc_emit_kernel(const McVolume g, const u
             const int ed = tri[q];
             const int c = RSDF_MC_EDGE_CORNER[ed];
             const int j = i + (c & 1) * g.syz + ((c >> 1) & 1) * g.nz + ((c >> 2) & 1);
-            f[q] = vertex_id(words, vbase, j, RSDF_MC_EDGE_AXIS[ed]);
+            f[q] = vid0 + vertex_id(words, vbase, j, RSDF_MC_EDGE_AXIS[ed]);
         }
         fcarry += off.total;
     }
 }
 
-int mc_setup(const float *volume, int nx, int ny, int nz, float iso, int negate, McVolume &g, int &nt) {
-    if (!volume || nx < 2 || ny < 2 || nz < 2 || 3LL * nx * ny * nz > 0x7fffffffLL) return RSDF_EBADARG;
-    g.v = volume;
-    g.nx = nx;
+int mc_setup(const float *slab, int p, int ny, int nz, int own, float iso, int negate, McVolume &g, int &nt) {
+    if (!slab || p < 2 || ny < 2 || nz < 2 || own < 1 || own > p || 3LL * p * ny * nz > 0x7fffffffLL)
+        return RSDF_EBADARG;
+    g.v = slab;
+    g.nx = p;
     g.ny = ny;
     g.nz = nz;
     g.syz = ny * nz;
-    g.n = nx * ny * nz;
+    g.n = p * ny * nz;
+    g.n_own = own * ny * nz;
     g.iso = iso;
     g.negate = negate != 0;
     nt = rsdf_div_up(g.n, MC_TILE);
@@ -269,33 +294,47 @@ McScratch mc_scratch(void *scratch, int nt) {
 
 extern "C" {
 
-int rsdf_mc_count(const float *volume, int nx, int ny, int nz, float iso, int negate, void *scratch,
-                  int64_t *totals2, void *stream) {
+int rsdf_mc_slab_count(const float *slab, int p, int ny, int nz, int own, float iso, int negate, void *scratch,
+                       int64_t *totals2, void *stream) {
     McVolume g;
     int nt;
-    const int rc = mc_setup(volume, nx, ny, nz, iso, negate, g, nt);
+    const int rc = mc_setup(slab, p, ny, nz, own, iso, negate, g, nt);
     if (rc) return rc;
     if (!scratch || !totals2 || (((uintptr_t)scratch) & 15)) return RSDF_EBADARG;
     cudaStream_t st = (cudaStream_t)stream;
     const McScratch s = mc_scratch(scratch, nt);
     mc_count_kernel<<<nt, MC_T, 0, st>>>(g, s.words, s.tile_tot);
     RSDF_LAUNCH_CHECK();
-    mc_scan_kernel<<<1, MC_SCAN_T, 0, st>>>(s.tile_tot, nt, s.vbase, s.fbase, (long long *)totals2);
+    mc_scan_kernel<<<1, MC_SCAN_T, 0, st>>>(s.tile_tot, nt, s.words, g.n, g.n_own, s.vbase, s.fbase,
+                                            (long long *)totals2);
     RSDF_LAUNCH_CHECK();
     return 0;
 }
 
-int rsdf_mc_emit(const float *volume, int nx, int ny, int nz, float iso, int negate, const void *scratch,
-                 float *verts, int64_t *faces, void *stream) {
+int rsdf_mc_slab_emit(const float *slab, int p, int ny, int nz, int own, int x0, int64_t vbase, float iso, int negate,
+                      const void *scratch, float *verts, int64_t *faces, void *stream) {
     McVolume g;
     int nt;
-    const int rc = mc_setup(volume, nx, ny, nz, iso, negate, g, nt);
+    const int rc = mc_setup(slab, p, ny, nz, own, iso, negate, g, nt);
     if (rc) return rc;
+    if (x0 < 0 || vbase < 0) return RSDF_EBADARG;
     if (!scratch || !verts || !faces || (((uintptr_t)scratch) & 15)) return RSDF_EBADARG;
     const McScratch s = mc_scratch(const_cast<void *>(scratch), nt);
-    mc_emit_kernel<<<nt, MC_T, 0, (cudaStream_t)stream>>>(g, s.words, s.vbase, s.fbase, verts, (long long *)faces);
+    mc_emit_kernel<<<rsdf_div_up(g.n_own, MC_TILE), MC_T, 0, (cudaStream_t)stream>>>(g, x0, (long long)vbase, s.words,
+                                                                                     s.vbase, s.fbase, verts,
+                                                                                     (long long *)faces);
     RSDF_LAUNCH_CHECK();
     return 0;
+}
+
+int rsdf_mc_count(const float *volume, int nx, int ny, int nz, float iso, int negate, void *scratch,
+                  int64_t *totals2, void *stream) {
+    return rsdf_mc_slab_count(volume, nx, ny, nz, nx, iso, negate, scratch, totals2, stream);
+}
+
+int rsdf_mc_emit(const float *volume, int nx, int ny, int nz, float iso, int negate, const void *scratch,
+                 float *verts, int64_t *faces, void *stream) {
+    return rsdf_mc_slab_emit(volume, nx, ny, nz, nx, 0, 0, iso, negate, scratch, verts, faces, stream);
 }
 
 }  // extern "C"

@@ -295,6 +295,39 @@ def save_mesh_obj(path, v_pos, t_pos_idx, v_rgb=None):
     return path
 
 
+def save_mesh_ply(path, v_pos, t_pos_idx, v_rgb=None):
+    """Binary little-endian PLY of a triangle mesh, for meshes too large for text (`VolumeSDF.isosurface` at 1024^3 and
+    beyond): `float x, y, z` per vertex, plus `float red, green, blue` in [0, 1] when `v_rgb` is given (float, not
+    uchar, so the colours are stored as computed), and `list uchar int vertex_indices` (0-based) per face.  The body is
+    two numpy records written as they are; an empty mesh writes a header with zero counts."""
+    host = lambda t: t.detach().cpu().numpy() if hasattr(t, "detach") else np.asarray(t)
+    v = host(v_pos).reshape(-1, 3)
+    f = host(t_pos_idx).reshape(-1, 3)
+    if len(v) > np.iinfo(np.int32).max:
+        raise ValueError(f"{len(v)} vertices: PLY face indices are int32")
+    names = ["x", "y", "z"] + ([] if v_rgb is None else ["red", "green", "blue"])
+    vert = np.empty(len(v), dtype=[(n, "<f4") for n in names])
+    for k in range(3):
+        vert[names[k]] = v[:, k]
+    if v_rgb is not None:
+        c = host(v_rgb).reshape(-1, 3)
+        if len(c) != len(v):
+            raise ValueError(f"v_rgb has {len(c)} rows for {len(v)} vertices")
+        for k in range(3):
+            vert[names[3 + k]] = c[:, k]
+    face = np.empty(len(f), dtype=[("n", "u1"), ("idx", "<i4", (3,))])
+    face["n"] = 3
+    face["idx"] = f
+    header = (["ply", "format binary_little_endian 1.0", f"element vertex {len(v)}"]
+              + [f"property float {n}" for n in names]
+              + [f"element face {len(f)}", "property list uchar int vertex_indices", "end_header"])
+    with open(path, "wb") as fh:
+        fh.write(("\n".join(header) + "\n").encode("ascii"))
+        fh.write(vert.tobytes())
+        fh.write(face.tobytes())
+    return path
+
+
 def save_level_grid(path, level):
     """The isosurface level grid (VolumeSDF.isosurface_level) as a raw .npy volume for an external marching-cubes tool."""
     import numpy as np

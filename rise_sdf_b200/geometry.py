@@ -240,24 +240,32 @@ class VolumeSDF(nn.Module):
         return sdf
 
     @torch.no_grad()
-    def isosurface_level(self, resolution=512, vmin=None, vmax=None, chunk=1 << 22, out=None):
+    def isosurface_level(self, resolution=512, vmin=None, vmax=None, chunk=1 << 22, out=None, x0=0, n_layers=None):
         """The level grid `BaseImplicitGeometry.isosurface_` evaluates before marching cubes (models/geometry.py:76-91):
         sdf at the resolution^3 vertices of linspace(0, 1, resolution)^3 scaled into [vmin, vmax] (default: the whole
         [-radius, radius]^3 box), x-major like `MarchingCubeHelper.grid_vertices` (:43-49).  The reference moves 2 M-point
         chunks to the GPU and back (`.cpu()` per chunk); here the vertices are generated on the device chunk by chunk
-        (nothing but the [resolution^3] result is ever materialised: 512 MB at 512^3) and each chunk is one hash-grid
-        launch + one sdf-only tcgen05 inference launch.  Returns a float32 tensor [resolution, resolution, resolution]."""
+        (nothing but the result is ever materialised: 512 MB at 512^3) and each chunk is one hash-grid launch + one
+        sdf-only tcgen05 inference launch.  `x0`, `n_layers` select the x layers [x0, x0 + n_layers) (default: all);
+        their values are those of the same points in the whole grid, bit for bit.  `out`, if given, is a float32
+        buffer of at least n_layers * resolution^2 elements whose head receives the values.  Returns a float32 tensor
+        [n_layers, resolution, resolution]."""
         r = int(resolution)
+        n = r - x0 if n_layers is None else int(n_layers)
+        if not (0 <= x0 and 0 <= n and x0 + n <= r):
+            raise ValueError(f"layers [{x0}, {x0 + n}) are outside the grid's {r} layers")
         dev = next(self.parameters()).device
         lo = torch.as_tensor([-self.radius] * 3 if vmin is None else vmin, dtype=torch.float32, device=dev)
         hi = torch.as_tensor([self.radius] * 3 if vmax is None else vmax, dtype=torch.float32, device=dev)
-        level = out if out is not None else torch.empty(r ** 3, device=dev, dtype=torch.float32)
+        begin, end = x0 * r * r, (x0 + n) * r * r
+        level = out.view(-1)[:end - begin] if out is not None else torch.empty(end - begin, device=dev,
+                                                                               dtype=torch.float32)
         lin = torch.linspace(0.0, 1.0, r, device=dev)
-        for s in range(0, r ** 3, chunk):
-            idx = torch.arange(s, min(s + chunk, r ** 3), device=dev)
+        for s in range(begin, end, chunk):
+            idx = torch.arange(s, min(s + chunk, end), device=dev)
             v = torch.stack([lin[idx // (r * r)], lin[(idx // r) % r], lin[idx % r]], -1)
-            level[s:s + idx.numel()] = self.forward_level(v * (hi - lo) + lo)       # scale_anything((0,1) -> (vmin, vmax))
-        return level.view(r, r, r)
+            level[s - begin:s - begin + idx.numel()] = self.forward_level(v * (hi - lo) + lo)   # scale_anything
+        return level.view(n, r, r)
 
     @torch.no_grad()
     def isosurface_bounds(self, level, vmin=None, vmax=None, threshold=0.0):
@@ -287,23 +295,38 @@ class VolumeSDF(nn.Module):
     def isosurface(self, resolution=512, threshold=0.0):
         """`BaseImplicitGeometry.isosurface` (models/geometry.py:76-112): a coarse mesh over the whole [-radius, radius]^3
         box places a fine grid on its bounding box padded by 10 % and clamped to the radius; returns the fine mesh
-        {'v_pos' [V,3] world space, 't_pos_idx' [F,3] int64} on the device.  Both level grids share one buffer.  An
-        empty coarse mesh (no surface in the box) gives an empty mesh."""
-        helper = MarchingCubeHelper(resolution)
+        {'v_pos' [V,3] world space, 't_pos_idx' [F,3] int64} on the device.  An empty coarse mesh (no surface in the
+        box) gives an empty mesh.  Both grids are evaluated and meshed one x-slab at a time (`mcubes.SLAB_BYTES` of
+        level values; a 512^3 grid is one slab), so any resolution works and the level grid is never whole in memory:
+        one slab buffer serves both stages, and the coarse stage keeps only the running bounds of its vertices."""
+        from .mcubes import marching_cubes_slab_iter, marching_cubes_slabs, plan_slabs
+        res = int(resolution)
+        shape = (res, res, res)
         dev = next(self.parameters()).device
-        buf = torch.empty(resolution ** 3, device=dev, dtype=torch.float32)
+        buf = torch.empty(max((p for _, _, p in plan_slabs(shape)), default=0) * res * res, device=dev,
+                          dtype=torch.float32)
         r = self.radius
         vmin = torch.full((3,), -r, dtype=torch.float32, device=dev)
         vmax = torch.full((3,), r, dtype=torch.float32, device=dev)
-        for fine in (False, True):
-            level = self.isosurface_level(resolution, vmin, vmax, out=buf)
-            mesh = helper(level, threshold)
-            mesh["v_pos"] = mesh["v_pos"] * (vmax - vmin) + vmin           # scale_anything((0, 1) -> (vmin, vmax))
-            if fine or mesh["v_pos"].shape[0] == 0:
-                return mesh
-            lo, hi = mesh["v_pos"].amin(dim=0), mesh["v_pos"].amax(dim=0)
-            vmin = (lo - (hi - lo) * 0.1).clamp(-r, r)
-            vmax = (hi + (hi - lo) * 0.1).clamp(-r, r)
+
+        def layers(vmin, vmax):
+            return lambda x0, n: self.isosurface_level(res, vmin, vmax, out=buf, x0=x0, n_layers=n)
+
+        # coarse: bounds of the mesh's index-space vertices.  v -> v / (res - 1) * (vmax - vmin) + vmin is monotone in
+        # each coordinate in fp32 as well, so it maps these bounds onto those of the world-space mesh exactly.
+        lo = hi = None
+        for verts, _ in marching_cubes_slab_iter(layers(vmin, vmax), shape, threshold, negate=True):
+            if verts.shape[0]:
+                a, b = verts.amin(dim=0), verts.amax(dim=0)
+                lo, hi = (a, b) if lo is None else (torch.minimum(lo, a), torch.maximum(hi, b))
+        if lo is None:
+            return {"v_pos": torch.zeros(0, 3, device=dev), "t_pos_idx": torch.zeros(0, 3, dtype=torch.int64, device=dev)}
+        lo = lo / (res - 1.0) * (vmax - vmin) + vmin
+        hi = hi / (res - 1.0) * (vmax - vmin) + vmin
+        vmin = (lo - (hi - lo) * 0.1).clamp(-r, r)
+        vmax = (hi + (hi - lo) * 0.1).clamp(-r, r)
+        verts, faces = marching_cubes_slabs(layers(vmin, vmax), shape, threshold, negate=True)
+        return {"v_pos": verts / (res - 1.0) * (vmax - vmin) + vmin, "t_pos_idx": faces}
 
     def update_step(self, epoch, global_step):
         update_module_step(self.encoding, epoch, global_step)
