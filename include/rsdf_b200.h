@@ -536,6 +536,30 @@ int rsdf_mc_slab_count(const float *slab, int p, int ny, int nz, int own, float 
 int rsdf_mc_slab_emit(const float *slab, int p, int ny, int nz, int own, int x0, int64_t vbase, float iso, int negate,
                       const void *scratch, float *verts, int64_t *faces, void *stream);
 
+/* ---------------------------------------------------------------- material baking (SplitMixedOCCModel.export) */
+/* Texture atlas of one-triangle charts for a mesh of n_faces faces in a texture_size^2 texture (T in [16, 16384]).
+ * Faces go in pairs: P = ceil(F / 2) pairs, cols = ceil(sqrt(P)), cell size C = T / cols (integer division), C >= 4
+ * (else -1; the smallest T that fits is 4 * cols).  Pair p's C x C cell has its top-left texel at (column, row) =
+ * ((p % cols) * C, (p / cols) * C); face 2p is triangle A, face 2p + 1 triangle B.  Cell-local (x, y) is in texel
+ * centres, row 0 on top; corners in the face's vertex order: A (0,0) (C-3,0) (0,C-3), B (C-1,C-1) (1,C-1) (C-1,1).
+ * Texel (i, j) of a cell belongs to A when i + j <= C - 2, else to B; texels of a face that does not exist are
+ * unowned.  Its surface point: (s, t) = (x, y) / (C-3) for A, ((C-1-x), (C-1-y)) / (C-2) for B; if s + t > 1 both
+ * lose (s + t - 1) / 2; clamp to [0, 1]; b0 = 1 - s - t; p = (b0 p0 + s p1) + t p2, each operation rounded (fp32,
+ * no contraction).
+ * rsdf_bake_uv: t_uv float32[F, 3, 2] = ((col0 + x + 0.5) / T, (row0 + y + 0.5) / T) per face corner (glTF UVs, origin
+ * at the top-left of the image). */
+int rsdf_bake_uv(int64_t n_faces, int texture_size, float *t_uv, void *stream);
+/* The atlas rows [row0, row0 + n_rows): face_id int32[n_rows * T] (owning face, -1 if unowned) and points
+ * float32[n_rows * T, 3] (the surface point, 0 if unowned), row-major.  v_pos float32[V, 3], t_pos_idx int64[F, 3]. */
+int rsdf_bake_texels(const float *v_pos, const int64_t *t_pos_idx, int64_t n_faces, int texture_size, int row0,
+                     int n_rows, int32_t *face_id, float *points, void *stream);
+/* models/texture.py `material` activations for n rows of raw network outputs: out float32[n, 5] =
+ * (sigmoid(raw_albedo[:, 3:6]), sigmoid(raw_roughness[:, 0]), sigmoid(raw_metallic[:, 1])), from raw_albedo
+ * float32[n, 6], raw_roughness float32[n, 1], raw_metallic float32[n, 2].  face_id int32[n] may be NULL; rows whose
+ * face id is -1 are written as 0 (an atlas band of rsdf_bake_texels, or per-vertex rows with face_id = NULL). */
+int rsdf_material_pack(const float *raw_albedo, const float *raw_roughness, const float *raw_metallic,
+                       const int32_t *face_id, int64_t n, float *out, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

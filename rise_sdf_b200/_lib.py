@@ -140,6 +140,9 @@ _SIGS = {
     "rsdf_mc_emit": [c_p, c_i, c_i, c_i, c_f, c_i, c_p, c_p, c_p, c_p],
     "rsdf_mc_slab_count": [c_p, c_i, c_i, c_i, c_i, c_f, c_i, c_p, c_p, c_p],
     "rsdf_mc_slab_emit": [c_p, c_i, c_i, c_i, c_i, c_i, ctypes.c_int64, c_f, c_i, c_p, c_p, c_p, c_p],
+    "rsdf_bake_uv": [ctypes.c_int64, c_i, c_p, c_p],
+    "rsdf_bake_texels": [c_p, c_p, ctypes.c_int64, c_i, c_i, c_i, c_p, c_p, c_p],
+    "rsdf_material_pack": [c_p, c_p, c_p, c_p, ctypes.c_int64, c_p, c_p],
 }
 
 

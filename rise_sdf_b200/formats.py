@@ -13,8 +13,10 @@ BSDF table and HDR environment maps run through the B200 path unchanged.
 
 Pure host code (numpy + torch serialization): nothing here touches the device.
 """
+import json
 import os
 import struct
+import zlib
 
 import numpy as np
 import torch
@@ -245,23 +247,25 @@ def load_env_latlong(fn, device="cuda"):
 def save_png(path, img):
     """utils/mixins.py `save_image_grid` / `save_rgb_image` write 8-bit PNGs through cv2; this is a dependency-free
     writer (zlib from the standard library) for rendered frames: img [H, W, 3|1] float in [0, 1] (torch or numpy)."""
-    import struct
-    import zlib
-    import numpy as np
     a = img.detach().cpu().numpy() if hasattr(img, "detach") else np.asarray(img)
     if a.ndim == 2:
         a = a[..., None]
     a = (np.clip(a, 0.0, 1.0) * 255.0 + 0.5).astype(np.uint8)
+    with open(path, "wb") as f:
+        f.write(png_bytes(a))
+
+
+def png_bytes(a):
+    """8-bit PNG file contents of a uint8 image [H, W, 3|1] (RGB or grey, row 0 on top, no filter, zlib level 6)."""
+    a = np.ascontiguousarray(a, dtype=np.uint8)
     h, w, c = a.shape
     assert c in (1, 3)
     raw = b"".join(b"\x00" + a[y].tobytes() for y in range(h))
 
     def chunk(tag, data):
         return struct.pack(">I", len(data)) + tag + data + struct.pack(">I", zlib.crc32(tag + data) & 0xFFFFFFFF)
-    png = (b"\x89PNG\r\n\x1a\n" + chunk(b"IHDR", struct.pack(">IIBBBBB", w, h, 8, 2 if c == 3 else 0, 0, 0, 0))
-           + chunk(b"IDAT", zlib.compress(raw, 6)) + chunk(b"IEND", b""))
-    with open(path, "wb") as f:
-        f.write(png)
+    return (b"\x89PNG\r\n\x1a\n" + chunk(b"IHDR", struct.pack(">IIBBBBB", w, h, 8, 2 if c == 3 else 0, 0, 0, 0))
+            + chunk(b"IDAT", zlib.compress(raw, 6)) + chunk(b"IEND", b""))
 
 
 def save_exr_or_hdr(path, img):
@@ -325,6 +329,114 @@ def save_mesh_ply(path, v_pos, t_pos_idx, v_rgb=None):
         fh.write(("\n".join(header) + "\n").encode("ascii"))
         fh.write(vert.tobytes())
         fh.write(face.tobytes())
+    return path
+
+
+GLB_MAGIC, GLB_JSON, GLB_BIN = 0x46546C67, 0x4E4F534A, 0x004E4942
+GLB_MAX_BYTES = 2 ** 32 - 1           # glTF binary lengths are uint32
+_FLOAT, _UINT32 = 5126, 5125
+_ARRAY_BUFFER, _ELEMENT_ARRAY_BUFFER = 34962, 34963
+_LINEAR, _CLAMP_TO_EDGE = 9729, 33071
+
+
+def _glb_textures(atlas):
+    """(base colour, metallic-roughness) uint8 [T, T, 3] images of a material atlas [T, T, 5] (albedo rgb linear,
+    roughness, metallic): round(255 * srgb(albedo)) and (0, round(255 * roughness), round(255 * metallic))."""
+    from .light import rgb_to_srgb
+    q = lambda x: torch.round(x.clamp(0.0, 1.0) * 255.0).to(torch.uint8)
+    atlas = (atlas.detach().cpu() if hasattr(atlas, "detach") else torch.as_tensor(atlas)).float()
+    base = q(rgb_to_srgb(atlas[..., 0:3]))
+    mr = torch.zeros_like(base)
+    mr[..., 1:3] = q(atlas[..., 3:5])
+    return base.numpy(), mr.numpy()
+
+
+def save_mesh_glb(path, mesh):
+    """glTF 2.0 binary (`.glb`) of a mesh dict.  Textured mode, when `t_uv` [F,3,2] and `material_atlas` [T,T,5] are
+    present (`SplitMixedOCCModel.export`): 3F unwelded corners with POSITION, NORMAL (the welded `v_nrm`, if given) and
+    TEXCOORD_0, and one `pbrMetallicRoughness` material whose base-colour texture is the sRGB-encoded albedo and whose
+    metallic-roughness texture is (0, roughness, metallic), both factors 1, embedded PNGs sampled LINEAR without mipmaps
+    and clamped to the edge.  Plain mode otherwise (`NeuSModel.export`, `VolumeSDF.isosurface`): the welded mesh, with
+    NORMAL and COLOR_0 from `v_nrm` / `v_rgb` when given.  POSITION carries its exact min / max; indices are uint32.  An
+    empty mesh writes an empty scene.  Raises ValueError when the file would exceed glTF's 32-bit lengths."""
+    host = lambda t: t.detach().cpu().numpy() if hasattr(t, "detach") else np.asarray(t)
+    v_pos = host(mesh["v_pos"]).astype(np.float32).reshape(-1, 3)
+    faces = host(mesh["t_pos_idx"]).astype(np.int64).reshape(-1, 3)
+    textured = mesh.get("t_uv") is not None and mesh.get("material_atlas") is not None
+    gltf = {"asset": {"version": "2.0", "generator": "rise_sdf_b200"}, "scene": 0, "scenes": [{"nodes": []}]}
+    chunks, views, accessors = [], [], []
+    offset = [0]
+
+    def add_view(data, target=None):
+        views.append({"buffer": 0, "byteOffset": offset[0], "byteLength": len(data)})
+        if target is not None:
+            views[-1]["target"] = target
+        pad = -len(data) % 4
+        chunks.append(data + b"\0" * pad)
+        offset[0] += len(data) + pad
+        return len(views) - 1
+
+    def add_accessor(a, kind, target, comp=_FLOAT, bounds=False):
+        acc = {"bufferView": add_view(a.tobytes(), target), "componentType": comp, "count": len(a), "type": kind}
+        if bounds:
+            acc["min"], acc["max"] = [float(x) for x in a.min(0)], [float(x) for x in a.max(0)]
+        accessors.append(acc)
+        return len(accessors) - 1
+
+    if len(faces):
+        if textured:
+            corners = faces.reshape(-1)
+            uv = host(mesh["t_uv"]).astype(np.float32).reshape(-1, 2)
+            if len(uv) != len(corners):
+                raise ValueError(f"t_uv has {len(uv)} corners for {len(faces)} faces")
+            n_vert = len(corners)
+        else:
+            corners = None
+            n_vert = len(v_pos)
+        n_attr = 3 + 3 * (mesh.get("v_nrm") is not None) + (2 if textured else 3 * (mesh.get("v_rgb") is not None))
+        need = 12 + 8 + 8 + 4 * n_attr * n_vert + 4 * 3 * len(faces)         # before the PNGs and the JSON
+        if need > GLB_MAX_BYTES:
+            raise ValueError(f"the mesh needs at least {need} bytes; a .glb holds at most {GLB_MAX_BYTES}")
+        vert = (lambda a: a[corners]) if textured else (lambda a: a)
+        attrs = {"POSITION": add_accessor(vert(v_pos), "VEC3", _ARRAY_BUFFER, bounds=True)}
+        if mesh.get("v_nrm") is not None:
+            attrs["NORMAL"] = add_accessor(vert(host(mesh["v_nrm"]).astype(np.float32).reshape(-1, 3)), "VEC3",
+                                           _ARRAY_BUFFER)
+        prim = {"attributes": attrs, "mode": 4}
+        if textured:
+            attrs["TEXCOORD_0"] = add_accessor(uv, "VEC2", _ARRAY_BUFFER)
+            idx = np.arange(n_vert, dtype=np.uint32)
+        else:
+            if mesh.get("v_rgb") is not None:
+                attrs["COLOR_0"] = add_accessor(host(mesh["v_rgb"]).astype(np.float32).reshape(-1, 3), "VEC3",
+                                                _ARRAY_BUFFER)
+            idx = faces.reshape(-1).astype(np.uint32)
+        prim["indices"] = add_accessor(idx, "SCALAR", _ELEMENT_ARRAY_BUFFER, comp=_UINT32)
+        if textured:
+            base, mr = _glb_textures(mesh["material_atlas"])
+            gltf["images"] = [{"bufferView": add_view(png_bytes(img)), "mimeType": "image/png"} for img in (base, mr)]
+            gltf["samplers"] = [{"magFilter": _LINEAR, "minFilter": _LINEAR, "wrapS": _CLAMP_TO_EDGE,
+                                 "wrapT": _CLAMP_TO_EDGE}]
+            gltf["textures"] = [{"sampler": 0, "source": 0}, {"sampler": 0, "source": 1}]
+            gltf["materials"] = [{"pbrMetallicRoughness": {
+                "baseColorFactor": [1.0, 1.0, 1.0, 1.0], "baseColorTexture": {"index": 0, "texCoord": 0},
+                "metallicFactor": 1.0, "roughnessFactor": 1.0,
+                "metallicRoughnessTexture": {"index": 1, "texCoord": 0}}}]
+            prim["material"] = 0
+        gltf.update(scenes=[{"nodes": [0]}], nodes=[{"mesh": 0}], meshes=[{"primitives": [prim]}],
+                    buffers=[{"byteLength": offset[0]}], bufferViews=views, accessors=accessors)
+    js = json.dumps(gltf, separators=(",", ":")).encode("utf-8")
+    js += b" " * (-len(js) % 4)
+    total = 12 + 8 + len(js) + (8 + offset[0] if chunks else 0)
+    if total > GLB_MAX_BYTES:
+        raise ValueError(f"the .glb would be {total} bytes; glTF binary holds at most {GLB_MAX_BYTES}")
+    with open(path, "wb") as fh:
+        fh.write(struct.pack("<III", GLB_MAGIC, 2, total))
+        fh.write(struct.pack("<II", len(js), GLB_JSON) + js)
+        if chunks:
+            fh.write(struct.pack("<II", offset[0], GLB_BIN))
+            for c in chunks:
+                fh.write(c)
     return path
 
 

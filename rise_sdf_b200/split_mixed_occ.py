@@ -377,3 +377,32 @@ class SplitMixedOCCModel(nn.Module):
     def eval(self):
         self.randomized = False
         return super().eval()
+
+    @torch.no_grad()
+    def export(self, chunk_size=1 << 20, resolution=512, threshold=0.0, texture_size=8192):
+        """The recovered geometry and PBR materials as a textured mesh (formats.save_mesh_glb writes it as glTF).
+        Like `NeuSModel.export`: the isosurface mesh, then normal = normalize(grad) at its vertices (chunked).
+        Materials (linear albedo, roughness, metallic; view-independent, so defined in every stage) are evaluated at
+        the vertices and baked into a texture_size^2 atlas of one-triangle charts (rise_sdf_b200/bake.py).  Returns, on
+        the device: v_pos [V,3], t_pos_idx [F,3], v_nrm [V,3], v_albedo [V,3], v_roughness [V,1], v_metallic [V,1],
+        t_uv [F,3,2] and material_atlas [T,T,5] (albedo rgb, roughness, metallic; 0 where no face owns the texel).
+        Raises ValueError when the mesh has too many faces for `texture_size` (the message names the smallest size
+        that fits)."""
+        from . import _lib as L
+        from .bake import atlas_uv, bake_material_atlas, material_at
+        L.require_cuda(self.scene_aabb)
+        mesh = self.geometry.isosurface(resolution, threshold)
+        v_pos, t_pos_idx = mesh["v_pos"], mesh["t_pos_idx"]
+        dev = v_pos.device
+        t_uv = atlas_uv(t_pos_idx.shape[0], texture_size, dev)         # a too-small atlas raises before the materials
+        if v_pos.shape[0] == 0:
+            mats = torch.zeros(0, 5, device=dev)
+            mesh["v_nrm"] = torch.zeros(0, 3, device=dev)
+        else:
+            _, sdf_grad = chunk_batch(self.geometry, chunk_size, False, v_pos, with_grad=True, with_feature=False)
+            mesh["v_nrm"] = F.normalize(sdf_grad, p=2, dim=-1)
+            mats = material_at(self, v_pos, chunk_size)
+        mesh.update(v_albedo=mats[:, :3].contiguous(), v_roughness=mats[:, 3:4].contiguous(),
+                    v_metallic=mats[:, 4:5].contiguous(), t_uv=t_uv,
+                    material_atlas=bake_material_atlas(self, v_pos, t_pos_idx, texture_size, chunk_size))
+        return mesh

@@ -83,6 +83,17 @@ class VolumeMixedMipSplitOcc(nn.Module):
         return dr.texture(self.FG_LUT, fg_uv.reshape(1, pn, 1, 2).contiguous(), filter_mode="linear",
                           boundary_mode="clamp").reshape(pn, 2)
 
+    def material_nets(self, features, positions):
+        """Raw outputs of the three view-independent material networks on [feature, VanillaFrequency(position)]:
+        albedo [..., 6] (diffuse rgb | albedo), roughness [..., 1], metallic [..., 2] (blend | metallic).  `material`
+        and the atlas baker (`bake.material_at`) both start from these."""
+        xyz_embd = self.xyz_encoding(positions.view(-1, self.n_pos_dims))
+        network_inp = [features.view(-1, features.shape[-1]), xyz_embd]
+        raw6 = self.albedo_network.forward_segments(network_inp).view(*features.shape[:-1], 6).float()
+        roughness = self.roughness_network.forward_segments(network_inp).view(*features.shape[:-1], 1).float()
+        raw2 = self.metallic_network.forward_segments(network_inp).view(*features.shape[:-1], 2).float()
+        return raw6, roughness, raw2
+
     def material(self, features, dirs, normals, positions, stage=0):
         """The light-independent half of `forward` (models/texture.py:330-377 up to the emitter lookups): material
         networks, activations, reflection direction, FG lookup.  A relighting render under several environment
@@ -90,12 +101,8 @@ class VolumeMixedMipSplitOcc(nn.Module):
         wi = -dirs
         wo = torch.sum(wi * normals, -1, keepdim=True) * normals * 2 - wi
         NoV = torch.sum(normals * wi, -1, keepdim=True)
-        xyz_embd = self.xyz_encoding(positions.view(-1, self.n_pos_dims))
-        network_inp = [features.view(-1, features.shape[-1]), xyz_embd]
-        raw6 = self.albedo_network.forward_segments(network_inp).view(*features.shape[:-1], 6).float()
+        raw6, roughness, raw2 = self.material_nets(features, positions)
         diff_rgb, albedo = raw6[..., :3], raw6[..., 3:]
-        roughness = self.roughness_network.forward_segments(network_inp).view(*features.shape[:-1], 1).float()
-        raw2 = self.metallic_network.forward_segments(network_inp).view(*features.shape[:-1], 2).float()
         blend, metallic = raw2[..., :1], raw2[..., 1:]
         wo_enc = self.dir_encoding(((wo + 1.0) / 2.0).view(-1, self.n_dir_dims))
         spec_rgb = self.env_network.forward_segments([features, wo_enc]).view(*features.shape[:-1], 3).float()
