@@ -559,6 +559,25 @@ int rsdf_bake_texels(const float *v_pos, const int64_t *t_pos_idx, int64_t n_fac
  * face id is -1 are written as 0 (an atlas band of rsdf_bake_texels, or per-vertex rows with face_id = NULL). */
 int rsdf_material_pack(const float *raw_albedo, const float *raw_roughness, const float *raw_metallic,
                        const int32_t *face_id, int64_t n, float *out, void *stream);
+/* Normal map of the atlas above (fp32, every product, sum, quotient and square root rounded on its own, no contraction;
+ * dot(a, b) = (a.x b.x + a.y b.y) + a.z b.z, normalize(v) = v / sqrt(dot(v, v))).
+ * rsdf_bake_tangents: t_tangent float32[F, 3, 4], a glTF TANGENT (xyz unit, w = +-1) per face corner.  With
+ * e1 = p1 - p0, e2 = p2 - p0 the atlas's +u direction is u = e1 for A and -e1 for B, image-up (decreasing v) is -e2
+ * for A and +e2 for B.  Corner k: n = normalize(N_k) (v_nrm float32[V, 3]), t1 = u - n dot(n, u), t = t1 - n dot(n, t1),
+ * tangent = normalize(t).  Fallback, when N_k is 0 or not finite (n = 0), e1 is 0 or u is (nearly) parallel to N_k
+ * (dot(t1, t1) <= 1e-6 dot(u, u)): t = a - n dot(n, a) for the world axis a least aligned with n (smallest |n_c|, the
+ * first of equal ones; x when n = 0).  w is one value per face: -1 when dot((N0 + N1) + N2, cross(e1, e2)) > 0, else
+ * +1, so that w cross(N, T) points image-up (glTF's normal texture: +X right, +Y up). */
+int rsdf_bake_tangents(const float *v_pos, const int64_t *t_pos_idx, const float *v_nrm, int64_t n_faces,
+                       int texture_size, float *t_tangent, void *stream);
+/* The normal atlas rows [row0, row0 + n_rows): out float32[n_rows * T, 3] = (dot(n, T'), dot(n, B), dot(n, N)), the
+ * field normal n = normalize(grad) (grad float32[n_rows * T, 3], one row per texel, e.g. at the points of
+ * rsdf_bake_texels) in the texel's tangent frame.  The texel's face and barycentrics b are recomputed as in
+ * rsdf_bake_texels; N = normalize((b0 N0 + b1 N1) + b2 N2), t = (b0 t0 + b1 t1) + b2 t2 of the corner tangents' xyz,
+ * T' = normalize(t - N dot(N, t)), B = w cross(N, T') (each product w B_c rounded).  (0, 0, 1) for unowned texels,
+ * a gradient whose length is 0 or not finite, and a zero N or T'. */
+int rsdf_normal_pack(const float *v_nrm, const int64_t *t_pos_idx, const float *t_tangent, int64_t n_faces,
+                     int texture_size, int row0, int n_rows, const float *grad, float *out, void *stream);
 
 #ifdef __cplusplus
 }

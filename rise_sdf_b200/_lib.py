@@ -143,6 +143,8 @@ _SIGS = {
     "rsdf_bake_uv": [ctypes.c_int64, c_i, c_p, c_p],
     "rsdf_bake_texels": [c_p, c_p, ctypes.c_int64, c_i, c_i, c_i, c_p, c_p, c_p],
     "rsdf_material_pack": [c_p, c_p, c_p, c_p, ctypes.c_int64, c_p, c_p],
+    "rsdf_bake_tangents": [c_p, c_p, c_p, ctypes.c_int64, c_i, c_p, c_p],
+    "rsdf_normal_pack": [c_p, c_p, c_p, ctypes.c_int64, c_i, c_i, c_i, c_p, c_p, c_p],
 }
 
 

@@ -10,6 +10,12 @@ face's UV triangle reads only texels of that face, so the atlas needs no gutters
 The atlas is evaluated in bands of texel rows: csrc/bake.cu gives each texel of the band its face and surface point,
 the geometry feature and the three material networks run on the existing no-grad kernels, and `rsdf_material_pack`
 applies the sigmoid and writes the band's rows of the atlas.  Device memory beyond the atlas is bounded by the band.
+
+The optional normal map carries the surface detail the mesh is too coarse for: every texel holds the model's own
+shading normal, normalize(grad) of the SDF at its surface point (finite differences or analytic, as the model's
+`grad_type` says), in the tangent frame a glTF viewer builds from the mesh's NORMAL and TANGENT (`atlas_tangents`,
+`rsdf_bake_tangents`; `rsdf_normal_pack` writes the band's rows).  `bake_atlases` evaluates the field once per band for
+both atlases: the geometry call that returns the gradient returns the feature the material networks read.
 """
 import math
 
@@ -53,9 +59,11 @@ def _check_model(model):
                          f"texture has {model.texture.config.get('color_activation', None)!r}")
 
 
-def _materials(model, points, face_id, out):
-    """materials of `points` [n, 3] into `out` [n, 5] (rows with face id -1 are 0)"""
-    _, feature = model.geometry(points, with_grad=False, with_feature=True)
+def _materials(model, points, face_id, out, feature=None):
+    """materials of `points` [n, 3] into `out` [n, 5] (rows with face id -1 are 0); `feature`: the geometry feature at
+    `points` when the caller has it"""
+    if feature is None:
+        _, feature = model.geometry(points, with_grad=False, with_feature=True)
     raw6, raw1, raw2 = model.texture.material_nets(feature, points)
     raw6, raw1, raw2 = raw6.contiguous(), raw1.contiguous(), raw2.contiguous()
     L.call("rsdf_material_pack", L.ptr(raw6), L.ptr(raw1), L.ptr(raw2), L.ptr(face_id), points.shape[0], L.ptr(out),
@@ -84,29 +92,90 @@ def material_at(model, points, chunk_size=1 << 20):
 
 
 @torch.no_grad()
-def bake_material_atlas(model, v_pos, t_pos_idx, texture_size=8192, chunk_size=1 << 20):
-    """The material atlas of the mesh (v_pos float32 [V, 3], t_pos_idx int64 [F, 3], CUDA): float32 [T, T, 5] of
-    (albedo rgb, roughness, metallic), row 0 on top, 0 where no face owns the texel; UVs from `atlas_uv`.  Bands of
-    max(1, chunk_size // T) texel rows are evaluated one at a time, over the rows that hold cells only."""
+def atlas_tangents(v_pos, t_pos_idx, v_nrm, texture_size):
+    """glTF TANGENTs float32 [F, 3, 4] of the atlas layout, one per face corner (`rsdf_bake_tangents`): the atlas's +u
+    direction made orthogonal to the corner's normal `v_nrm` [V, 3], and w = +-1 per face so that w cross(N, T) points
+    image-up.  Raises ValueError like `atlas_layout`."""
+    L.require_cuda(v_pos, t_pos_idx, v_nrm)
+    F = t_pos_idx.shape[0]
+    atlas_layout(F, texture_size)
+    t_tangent = torch.empty(F, 3, 4, dtype=torch.float32, device=v_pos.device)
+    if F:
+        v_pos = v_pos.detach().float().contiguous()
+        v_nrm = v_nrm.detach().float().contiguous()
+        t_pos_idx = t_pos_idx.detach().to(torch.int64).contiguous()
+        L.call("rsdf_bake_tangents", L.ptr(v_pos), L.ptr(t_pos_idx), L.ptr(v_nrm), F, int(texture_size),
+               L.ptr(t_tangent), L.stream())
+    return t_tangent
+
+
+def _bake_bands(model, v_pos, t_pos_idx, texture_size, chunk_size, materials, normals):
+    """(material atlas [T, T, 5] if `materials` else None, normal atlas [T, T, 3] if `normals` = (v_nrm, t_tangent)
+    else None), one geometry call per band of texel rows"""
     L.require_cuda(v_pos, t_pos_idx)
-    _check_model(model)
+    if materials:
+        _check_model(model)
     T = int(texture_size)
     F = t_pos_idx.shape[0]
     C, cols = atlas_layout(F, T)
     dev = v_pos.device
-    atlas = torch.zeros(T, T, 5, dtype=torch.float32, device=dev)
+    atlas = torch.zeros(T, T, 5, dtype=torch.float32, device=dev) if materials else None
+    normal_atlas = None
+    if normals is not None:
+        v_nrm, t_tangent = normals
+        L.require_cuda(v_nrm, t_tangent)
+        if tuple(t_tangent.shape) != (F, 3, 4):
+            raise ValueError(f"t_tangent must be [{F}, 3, 4] for {F} faces, got {list(t_tangent.shape)}")
+        v_nrm = v_nrm.detach().float().contiguous()
+        t_tangent = t_tangent.detach().float().contiguous()
+        normal_atlas = torch.zeros(T, T, 3, dtype=torch.float32, device=dev)
+        normal_atlas[..., 2] = 1.0                                   # unowned texels: flat
     if F == 0:
-        return atlas
+        return atlas, normal_atlas
     v_pos = v_pos.detach().float().contiguous()
     t_pos_idx = t_pos_idx.detach().to(torch.int64).contiguous()
     rows = -(-((F + 1) // 2) // cols) * C                    # texel rows that hold cells
     band = min(max(1, _chunk(chunk_size) // T), rows)
     face_id = torch.empty(band * T, dtype=torch.int32, device=dev)
     points = torch.empty(band * T, 3, dtype=torch.float32, device=dev)
-    flat = atlas.view(T * T, 5)
+    # the analytic gradient's feature comes from the training kernels; bake_material_atlas's from the inference ones
+    shared = normals is None or model.geometry.grad_type == "finite_difference"
     for r0 in range(0, rows, band):
         n = min(band, rows - r0)
-        L.call("rsdf_bake_texels", L.ptr(v_pos), L.ptr(t_pos_idx), F, T, r0, n, L.ptr(face_id), L.ptr(points),
+        pts = points[:n * T]
+        L.call("rsdf_bake_texels", L.ptr(v_pos), L.ptr(t_pos_idx), F, T, r0, n, L.ptr(face_id), L.ptr(pts),
                L.stream())
-        _materials(model, points[:n * T], face_id[:n * T], flat[r0 * T:(r0 + n) * T])
-    return atlas
+        feature = None
+        if normals is not None:
+            _, grad, feature = model.geometry(pts, with_grad=True, with_feature=True)
+            grad = grad.float().contiguous()
+            L.call("rsdf_normal_pack", L.ptr(v_nrm), L.ptr(t_pos_idx), L.ptr(t_tangent), F, T, r0, n, L.ptr(grad),
+                   L.ptr(normal_atlas.view(T * T, 3)[r0 * T:(r0 + n) * T]), L.stream())
+        if materials:
+            _materials(model, pts, face_id[:n * T], atlas.view(T * T, 5)[r0 * T:(r0 + n) * T],
+                       feature if shared else None)
+    return atlas, normal_atlas
+
+
+@torch.no_grad()
+def bake_material_atlas(model, v_pos, t_pos_idx, texture_size=8192, chunk_size=1 << 20):
+    """The material atlas of the mesh (v_pos float32 [V, 3], t_pos_idx int64 [F, 3], CUDA): float32 [T, T, 5] of
+    (albedo rgb, roughness, metallic), row 0 on top, 0 where no face owns the texel; UVs from `atlas_uv`.  Bands of
+    max(1, chunk_size // T) texel rows are evaluated one at a time, over the rows that hold cells only."""
+    return _bake_bands(model, v_pos, t_pos_idx, texture_size, chunk_size, True, None)[0]
+
+
+@torch.no_grad()
+def bake_normal_atlas(model, v_pos, t_pos_idx, v_nrm, t_tangent, texture_size=8192, chunk_size=1 << 20):
+    """The tangent-space normal atlas of the mesh: float32 [T, T, 3], per texel the unit field normal
+    normalize(model.geometry(point, with_grad=True)) at its surface point in the frame of the interpolated vertex
+    normal `v_nrm` [V, 3] and corner tangents `t_tangent` [F, 3, 4] (`atlas_tangents`): (x along T, y along
+    B = w cross(N, T), z along N); (0, 0, 1) where no face owns the texel.  Banded like `bake_material_atlas`."""
+    return _bake_bands(model, v_pos, t_pos_idx, texture_size, chunk_size, False, (v_nrm, t_tangent))[1]
+
+
+@torch.no_grad()
+def bake_atlases(model, v_pos, t_pos_idx, v_nrm, t_tangent, texture_size=8192, chunk_size=1 << 20):
+    """(`bake_material_atlas`, `bake_normal_atlas`) of the mesh from one geometry evaluation per band.  With the
+    split-sum config's finite-difference gradient the material atlas is bit-identical to `bake_material_atlas`'s."""
+    return _bake_bands(model, v_pos, t_pos_idx, texture_size, chunk_size, True, (v_nrm, t_tangent))

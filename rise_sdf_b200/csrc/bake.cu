@@ -15,6 +15,10 @@
 //     triangle, the nearest point on the triangle (a one-texel dilation for bilinear samples at the edges).
 // Positions are evaluated as (b0 p0 + b1 p1) + b2 p2 with every product and sum rounded separately (no contraction),
 // so the float32 numpy oracle reproduces them bit for bit.
+//
+// The normal map (`export(normal_map=True)`) adds glTF tangents per face corner (`rsdf_bake_tangents`) and a
+// tangent-space normal atlas of the field's gradient (`rsdf_normal_pack`), in the same atlas and with the same rounding
+// rule.
 #include "common.cuh"
 
 namespace {
@@ -146,6 +150,137 @@ __global__ void __launch_bounds__(BAKE_T) material_pack_kernel(const float *__re
     for (int c = 0; c < 5; ++c) out[5 * k + c] = v[c];
 }
 
+// ---- tangent frames for the normal atlas: fp32, every product, sum, quotient and root rounded on its own
+// (dot = (x x' + y y') + z z'), so the float32 numpy oracle restates them bit for bit
+
+__device__ __forceinline__ float dot3(const float *a, const float *b) {
+    return __fadd_rn(__fadd_rn(__fmul_rn(a[0], b[0]), __fmul_rn(a[1], b[1])), __fmul_rn(a[2], b[2]));
+}
+
+__device__ __forceinline__ void cross3(const float *a, const float *b, float *o) {
+    o[0] = __fsub_rn(__fmul_rn(a[1], b[2]), __fmul_rn(a[2], b[1]));
+    o[1] = __fsub_rn(__fmul_rn(a[2], b[0]), __fmul_rn(a[0], b[2]));
+    o[2] = __fsub_rn(__fmul_rn(a[0], b[1]), __fmul_rn(a[1], b[0]));
+}
+
+// v /= |v| in place; false (v unchanged) when |v| is 0 or not finite
+__device__ __forceinline__ bool unit3(float *v) {
+    const float l = __fsqrt_rn(dot3(v, v));
+    if (!(l > 0.0f) || isinf(l)) return false;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) v[c] = __fdiv_rn(v[c], l);
+    return true;
+}
+
+// v - n (n . v)
+__device__ __forceinline__ void reject3(const float *v, const float *n, float *o) {
+    const float d = dot3(n, v);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) o[c] = __fsub_rn(v[c], __fmul_rn(n[c], d));
+}
+
+// (b0 a + b1 b) + b2 c
+__device__ __forceinline__ void bary3(float b0, float b1, float b2, const float *a, const float *b, const float *c,
+                                      float *o) {
+#pragma unroll
+    for (int k = 0; k < 3; ++k)
+        o[k] = __fadd_rn(__fadd_rn(__fmul_rn(b0, a[k]), __fmul_rn(b1, b[k])), __fmul_rn(b2, c[k]));
+}
+
+// One thread per face: the atlas's +u direction (e1 for A, -e1 for B) made orthogonal to each corner's unit normal
+// (rejected twice) and normalised; where that fails (zero e1 or normal, or |t1|^2 <= 1e-6 |u|^2 after one rejection)
+// the world axis least aligned with the normal (first of equal ones) is used instead.  w = -1 when (N0 + N1) + N2 . cross(e1, e2) > 0, else +1: image-up
+// is -e2 for A and +e2 for B, and both give cross(u, up) = -cross(e1, e2), so w cross(N, T) points image-up.
+__global__ void __launch_bounds__(BAKE_T) bake_tangents_kernel(long long n_faces, const float *__restrict__ v_pos,
+                                                               const long long *__restrict__ t_pos_idx,
+                                                               const float *__restrict__ v_nrm,
+                                                               float *__restrict__ t_tangent) {
+    const long long f = (long long)blockIdx.x * BAKE_T + threadIdx.x;
+    if (f >= n_faces) return;
+    long long idx[3];
+    float p[3][3], n[3][3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        idx[k] = t_pos_idx[3 * f + k];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            p[k][c] = v_pos[3 * idx[k] + c];
+            n[k][c] = v_nrm[3 * idx[k] + c];
+        }
+    }
+    float e1[3], e2[3], u[3], ns[3], fn[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        e1[c] = __fsub_rn(p[1][c], p[0][c]);
+        e2[c] = __fsub_rn(p[2][c], p[0][c]);
+        u[c] = (f & 1) ? -e1[c] : e1[c];
+        ns[c] = __fadd_rn(__fadd_rn(n[0][c], n[1][c]), n[2][c]);
+    }
+    cross3(e1, e2, fn);
+    const float w = dot3(ns, fn) > 0.0f ? -1.0f : 1.0f;
+    const float uu = dot3(u, u);
+    float *o = t_tangent + 12 * f;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        float nk[3] = {n[k][0], n[k][1], n[k][2]}, t[3];
+        const bool has_n = unit3(nk);
+        if (!has_n) nk[0] = nk[1] = nk[2] = 0.0f;
+        float t1[3];
+        reject3(u, nk, t1);
+        reject3(t1, nk, t);                           // twice: orthogonal to rounding even when t1 is short
+        if (!has_n || !(dot3(t1, t1) > __fmul_rn(1e-6f, uu))) {
+            const float ax = fabsf(nk[0]), ay = fabsf(nk[1]), az = fabsf(nk[2]);
+            const int a = (ax <= ay && ax <= az) ? 0 : (ay <= az ? 1 : 2);
+            float e[3] = {0.0f, 0.0f, 0.0f};
+            e[a] = 1.0f;
+            reject3(e, nk, t);
+        }
+        unit3(t);
+        o[4 * k] = t[0];
+        o[4 * k + 1] = t[1];
+        o[4 * k + 2] = t[2];
+        o[4 * k + 3] = w;
+    }
+}
+
+// One thread per texel of rows [row0, row0 + n / T): the field normal grad / |grad| in the texel's tangent frame,
+// (n . T', n . B, n . N) with N = normalize(sum b_k N_k), T' = normalize(t - N (N . t)) for t = sum b_k t_k,
+// B = w cross(N, T'); (0, 0, 1) for unowned texels, a gradient whose length is 0 or not finite, or a zero N or T'.
+__global__ void __launch_bounds__(BAKE_T) normal_pack_kernel(BakeLayout l, int row0, long long n,
+                                                             const float *__restrict__ v_nrm,
+                                                             const long long *__restrict__ t_pos_idx,
+                                                             const float *__restrict__ t_tangent,
+                                                             const float *__restrict__ grad, float *__restrict__ out) {
+    const long long k = (long long)blockIdx.x * BAKE_T + threadIdx.x;
+    if (k >= n) return;
+    const int gj = row0 + (int)(k / l.T), gi = (int)(k % l.T);
+    float b0, b1, b2;
+    const long long face = bake_texel(l, gi, gj, b0, b1, b2);
+    float r[3] = {0.0f, 0.0f, 1.0f};
+    if (face >= 0) {
+        float g[3] = {grad[3 * k], grad[3 * k + 1], grad[3 * k + 2]};
+        const long long i0 = t_pos_idx[3 * face], i1 = t_pos_idx[3 * face + 1], i2 = t_pos_idx[3 * face + 2];
+        const float *tg = t_tangent + 12 * face;
+        float N[3], t[3], T[3], B[3];
+        bary3(b0, b1, b2, v_nrm + 3 * i0, v_nrm + 3 * i1, v_nrm + 3 * i2, N);
+        bary3(b0, b1, b2, tg, tg + 4, tg + 8, t);
+        if (unit3(g) && unit3(N)) {
+            reject3(t, N, T);
+            if (unit3(T)) {
+                const float w = tg[3];
+                cross3(N, T, B);
+#pragma unroll
+                for (int c = 0; c < 3; ++c) B[c] = __fmul_rn(w, B[c]);
+                r[0] = dot3(g, T);
+                r[1] = dot3(g, B);
+                r[2] = dot3(g, N);
+            }
+        }
+    }
+#pragma unroll
+    for (int c = 0; c < 3; ++c) out[3 * k + c] = r[c];
+}
+
 int blocks_for(long long n) { return (int)((n + BAKE_T - 1) / BAKE_T); }
 
 }  // namespace
@@ -183,6 +318,32 @@ int rsdf_material_pack(const float *raw_albedo, const float *raw_roughness, cons
     if (!raw_albedo || !raw_roughness || !raw_metallic || !out) return RSDF_EBADARG;
     material_pack_kernel<<<blocks_for(n), BAKE_T, 0, (cudaStream_t)stream>>>(raw_albedo, raw_roughness, raw_metallic,
                                                                              (const int *)face_id, n, out);
+    RSDF_LAUNCH_CHECK();
+    return 0;
+}
+
+int rsdf_bake_tangents(const float *v_pos, const int64_t *t_pos_idx, const float *v_nrm, int64_t n_faces,
+                       int texture_size, float *t_tangent, void *stream) {
+    BakeLayout l;
+    if (!bake_layout(n_faces, texture_size, l)) return RSDF_EBADARG;
+    if (n_faces == 0) return 0;
+    if (!v_pos || !t_pos_idx || !v_nrm || !t_tangent) return RSDF_EBADARG;
+    bake_tangents_kernel<<<blocks_for(n_faces), BAKE_T, 0, (cudaStream_t)stream>>>(
+        n_faces, v_pos, (const long long *)t_pos_idx, v_nrm, t_tangent);
+    RSDF_LAUNCH_CHECK();
+    return 0;
+}
+
+int rsdf_normal_pack(const float *v_nrm, const int64_t *t_pos_idx, const float *t_tangent, int64_t n_faces,
+                     int texture_size, int row0, int n_rows, const float *grad, float *out, void *stream) {
+    BakeLayout l;
+    if (!bake_layout(n_faces, texture_size, l)) return RSDF_EBADARG;
+    if (row0 < 0 || n_rows < 0 || row0 + (long long)n_rows > texture_size) return RSDF_EBADARG;
+    const long long n = (long long)n_rows * texture_size;
+    if (n == 0) return 0;
+    if (!grad || !out || (n_faces > 0 && (!v_nrm || !t_pos_idx || !t_tangent))) return RSDF_EBADARG;
+    normal_pack_kernel<<<blocks_for(n), BAKE_T, 0, (cudaStream_t)stream>>>(
+        l, row0, n, v_nrm, (const long long *)t_pos_idx, t_tangent, grad, out);
     RSDF_LAUNCH_CHECK();
     return 0;
 }

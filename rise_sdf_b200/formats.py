@@ -351,6 +351,13 @@ def _glb_textures(atlas):
     return base.numpy(), mr.numpy()
 
 
+def _glb_normal_texture(normal_atlas):
+    """uint8 [T, T, 3] image of a tangent-space normal atlas [T, T, 3] in [-1, 1]: round(255 * (0.5 x + 0.5)),
+    clamped (glTF's linear normal texture encoding)."""
+    a = (normal_atlas.detach().cpu() if hasattr(normal_atlas, "detach") else torch.as_tensor(normal_atlas)).float()
+    return torch.round((a * 0.5 + 0.5).clamp(0.0, 1.0) * 255.0).to(torch.uint8).numpy()
+
+
 def save_mesh_glb(path, mesh):
     """glTF 2.0 binary (`.glb`) of a mesh dict.  Textured mode, when `t_uv` [F,3,2] and `material_atlas` [T,T,5] are
     present (`SplitMixedOCCModel.export`): 3F unwelded corners with POSITION, NORMAL (the welded `v_nrm`, if given) and
@@ -358,11 +365,15 @@ def save_mesh_glb(path, mesh):
     metallic-roughness texture is (0, roughness, metallic), both factors 1, embedded PNGs sampled LINEAR without mipmaps
     and clamped to the edge.  Plain mode otherwise (`NeuSModel.export`, `VolumeSDF.isosurface`): the welded mesh, with
     NORMAL and COLOR_0 from `v_nrm` / `v_rgb` when given.  POSITION carries its exact min / max; indices are uint32.  An
-    empty mesh writes an empty scene.  Raises ValueError when the file would exceed glTF's 32-bit lengths."""
+    empty mesh writes an empty scene.  Raises ValueError when the file would exceed glTF's 32-bit lengths.
+    A textured mesh that also has `t_tangent` [F,3,4] and `normal_atlas` [T,T,3] (`export(normal_map=True)`) gets a
+    TANGENT attribute per corner and the material a `normalTexture`: the tangent-space normals as a linear PNG,
+    round(255 * (0.5 x + 0.5)) per channel."""
     host = lambda t: t.detach().cpu().numpy() if hasattr(t, "detach") else np.asarray(t)
     v_pos = host(mesh["v_pos"]).astype(np.float32).reshape(-1, 3)
     faces = host(mesh["t_pos_idx"]).astype(np.int64).reshape(-1, 3)
     textured = mesh.get("t_uv") is not None and mesh.get("material_atlas") is not None
+    normal_map = textured and mesh.get("t_tangent") is not None and mesh.get("normal_atlas") is not None
     gltf = {"asset": {"version": "2.0", "generator": "rise_sdf_b200"}, "scene": 0, "scenes": [{"nodes": []}]}
     chunks, views, accessors = [], [], []
     offset = [0]
@@ -394,6 +405,7 @@ def save_mesh_glb(path, mesh):
             corners = None
             n_vert = len(v_pos)
         n_attr = 3 + 3 * (mesh.get("v_nrm") is not None) + (2 if textured else 3 * (mesh.get("v_rgb") is not None))
+        n_attr += 4 * normal_map
         need = 12 + 8 + 8 + 4 * n_attr * n_vert + 4 * 3 * len(faces)         # before the PNGs and the JSON
         if need > GLB_MAX_BYTES:
             raise ValueError(f"the mesh needs at least {need} bytes; a .glb holds at most {GLB_MAX_BYTES}")
@@ -405,6 +417,11 @@ def save_mesh_glb(path, mesh):
         prim = {"attributes": attrs, "mode": 4}
         if textured:
             attrs["TEXCOORD_0"] = add_accessor(uv, "VEC2", _ARRAY_BUFFER)
+            if normal_map:
+                tangent = host(mesh["t_tangent"]).astype(np.float32).reshape(-1, 4)
+                if len(tangent) != len(corners):
+                    raise ValueError(f"t_tangent has {len(tangent)} corners for {len(faces)} faces")
+                attrs["TANGENT"] = add_accessor(tangent, "VEC4", _ARRAY_BUFFER)
             idx = np.arange(n_vert, dtype=np.uint32)
         else:
             if mesh.get("v_rgb") is not None:
@@ -413,15 +430,19 @@ def save_mesh_glb(path, mesh):
             idx = faces.reshape(-1).astype(np.uint32)
         prim["indices"] = add_accessor(idx, "SCALAR", _ELEMENT_ARRAY_BUFFER, comp=_UINT32)
         if textured:
-            base, mr = _glb_textures(mesh["material_atlas"])
-            gltf["images"] = [{"bufferView": add_view(png_bytes(img)), "mimeType": "image/png"} for img in (base, mr)]
+            images = _glb_textures(mesh["material_atlas"])
+            if normal_map:
+                images += (_glb_normal_texture(mesh["normal_atlas"]),)
+            gltf["images"] = [{"bufferView": add_view(png_bytes(img)), "mimeType": "image/png"} for img in images]
             gltf["samplers"] = [{"magFilter": _LINEAR, "minFilter": _LINEAR, "wrapS": _CLAMP_TO_EDGE,
                                  "wrapT": _CLAMP_TO_EDGE}]
-            gltf["textures"] = [{"sampler": 0, "source": 0}, {"sampler": 0, "source": 1}]
+            gltf["textures"] = [{"sampler": 0, "source": i} for i in range(len(images))]
             gltf["materials"] = [{"pbrMetallicRoughness": {
                 "baseColorFactor": [1.0, 1.0, 1.0, 1.0], "baseColorTexture": {"index": 0, "texCoord": 0},
                 "metallicFactor": 1.0, "roughnessFactor": 1.0,
                 "metallicRoughnessTexture": {"index": 1, "texCoord": 0}}}]
+            if normal_map:
+                gltf["materials"][0]["normalTexture"] = {"index": 2, "texCoord": 0}
             prim["material"] = 0
         gltf.update(scenes=[{"nodes": [0]}], nodes=[{"mesh": 0}], meshes=[{"primitives": [prim]}],
                     buffers=[{"byteLength": offset[0]}], bufferViews=views, accessors=accessors)

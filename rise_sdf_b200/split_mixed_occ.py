@@ -379,17 +379,20 @@ class SplitMixedOCCModel(nn.Module):
         return super().eval()
 
     @torch.no_grad()
-    def export(self, chunk_size=1 << 20, resolution=512, threshold=0.0, texture_size=8192):
+    def export(self, chunk_size=1 << 20, resolution=512, threshold=0.0, texture_size=8192, normal_map=False):
         """The recovered geometry and PBR materials as a textured mesh (formats.save_mesh_glb writes it as glTF).
         Like `NeuSModel.export`: the isosurface mesh, then normal = normalize(grad) at its vertices (chunked).
         Materials (linear albedo, roughness, metallic; view-independent, so defined in every stage) are evaluated at
         the vertices and baked into a texture_size^2 atlas of one-triangle charts (rise_sdf_b200/bake.py).  Returns, on
         the device: v_pos [V,3], t_pos_idx [F,3], v_nrm [V,3], v_albedo [V,3], v_roughness [V,1], v_metallic [V,1],
         t_uv [F,3,2] and material_atlas [T,T,5] (albedo rgb, roughness, metallic; 0 where no face owns the texel).
+        With `normal_map`, also t_tangent [F,3,4] (glTF TANGENTs per face corner) and normal_atlas [T,T,3]: the shading
+        normal normalize(grad) at every texel's surface point in tangent space, so detail finer than the mesh survives
+        the export (the same band pass evaluates both atlases; the other entries do not change).
         Raises ValueError when the mesh has too many faces for `texture_size` (the message names the smallest size
         that fits)."""
         from . import _lib as L
-        from .bake import atlas_uv, bake_material_atlas, material_at
+        from .bake import atlas_tangents, atlas_uv, bake_atlases, bake_material_atlas, material_at
         L.require_cuda(self.scene_aabb)
         mesh = self.geometry.isosurface(resolution, threshold)
         v_pos, t_pos_idx = mesh["v_pos"], mesh["t_pos_idx"]
@@ -402,7 +405,14 @@ class SplitMixedOCCModel(nn.Module):
             _, sdf_grad = chunk_batch(self.geometry, chunk_size, False, v_pos, with_grad=True, with_feature=False)
             mesh["v_nrm"] = F.normalize(sdf_grad, p=2, dim=-1)
             mats = material_at(self, v_pos, chunk_size)
+        if normal_map:
+            t_tangent = atlas_tangents(v_pos, t_pos_idx, mesh["v_nrm"], texture_size)
+            atlas, normal_atlas = bake_atlases(self, v_pos, t_pos_idx, mesh["v_nrm"], t_tangent, texture_size,
+                                               chunk_size)
+        else:
+            atlas = bake_material_atlas(self, v_pos, t_pos_idx, texture_size, chunk_size)
         mesh.update(v_albedo=mats[:, :3].contiguous(), v_roughness=mats[:, 3:4].contiguous(),
-                    v_metallic=mats[:, 4:5].contiguous(), t_uv=t_uv,
-                    material_atlas=bake_material_atlas(self, v_pos, t_pos_idx, texture_size, chunk_size))
+                    v_metallic=mats[:, 4:5].contiguous(), t_uv=t_uv, material_atlas=atlas)
+        if normal_map:
+            mesh.update(t_tangent=t_tangent, normal_atlas=normal_atlas)
         return mesh

@@ -1,6 +1,7 @@
 """Textured export timing (`SplitMixedOCCModel.export` and its phases); prints one JSON line.
 
     python scripts/bench_bake.py [--reps 3] [--resolution 512] [--texture-size 8192] [--chunk-size 1048576]
+                                 [--normal-map]
 
 The model is the seeded split-sum test model (tests/test_gpu_splitsum.py `_split_model`: seed 0, hash-feature columns
 of the first layer ~ N(0, 0.05), table ~ U(-0.02, 0.02)) in eval mode at stage 1.  Phases, each timed with CUDA events
@@ -9,6 +10,10 @@ on the current stream after one warm-up pass of all of them, mean over `--reps`:
 * `vertex_materials`: normals (`geometry(v, with_grad=True)`) and `bake.material_at` at the vertices;
 * `texel_bands`: `bake.bake_material_atlas` (texels/s counts the texel rows that hold cells, the ones evaluated);
 * `glb_write`: `formats.save_mesh_glb` of the export to a temporary directory (host work: atlas copy, PNG encoding).
+With `--normal-map` (what `export(normal_map=True)` runs instead of `texel_bands`):
+* `normal_bands`: `bake.atlas_tangents` and `bake.bake_atlases`, the material and normal atlases from one geometry
+  evaluation (with the finite-difference gradient) per band; `normal_texels_per_s` counts the same texels as
+  `texels_per_s`, and `glb_write` then writes the normal map too.
 The card's name and power limit are read in the same run.
 """
 import argparse
@@ -65,6 +70,7 @@ def main():
     ap.add_argument("--resolution", type=int, default=512)
     ap.add_argument("--texture-size", type=int, default=8192)
     ap.add_argument("--chunk-size", type=int, default=1 << 20)
+    ap.add_argument("--normal-map", action="store_true")
     args = ap.parse_args()
     assert torch.cuda.is_available(), "bench_bake.py measures the GPU path and needs a CUDA device"
     name, power = card()
@@ -82,9 +88,16 @@ def main():
     def glb():
         mesh = state["mesh"]
         nrm, mats = state["vertex"]
+        extra = {"t_tangent": state["normals"][0], "normal_atlas": state["normals"][1]} if args.normal_map else {}
         return formats.save_mesh_glb(os.path.join(tmp, "export.glb"), {
             **mesh, "v_nrm": nrm, "t_uv": bake.atlas_uv(mesh["t_pos_idx"].shape[0], T, "cuda"),
-            "material_atlas": state["atlas"]})
+            "material_atlas": state["atlas"], **extra})
+
+    def normal_bands():
+        v, f = state["mesh"]["v_pos"], state["mesh"]["t_pos_idx"]
+        t_tangent = bake.atlas_tangents(v, f, state["vertex"][0], T)
+        _, normal_atlas = bake.bake_atlases(m, v, f, state["vertex"][0], t_tangent, T, chunk)
+        state["normals"] = (t_tangent, normal_atlas)
 
     phases = {
         "isosurface": lambda: state.__setitem__("mesh", m.geometry.isosurface(res)),
@@ -93,6 +106,9 @@ def main():
             m, state["mesh"]["v_pos"], state["mesh"]["t_pos_idx"], T, chunk)),
         "glb_write": glb,
     }
+    if args.normal_map:
+        phases = {**{k: v for k, v in phases.items() if k != "glb_write"}, "normal_bands": normal_bands,
+                  "glb_write": glb}
     for fn in phases.values():                                   # warm-up
         fn()
     ms = {k: [] for k in phases}
@@ -109,7 +125,10 @@ def main():
            "ms": {k: round(v, 2) for k, v in mean.items()},
            "ms_each": {k: [round(x, 2) for x in v] for k, v in ms.items()},
            "texels_per_s": round(texels / (mean["texel_bands"] * 1e-3)),
-           "export_ms": round(sum(mean.values()) - mean["glb_write"], 2)}
+           "export_ms": round(mean["isosurface"] + mean["vertex_materials"] + mean["texel_bands"], 2)}
+    if args.normal_map:
+        out["normal_texels_per_s"] = round(texels / (mean["normal_bands"] * 1e-3))
+        out["export_normal_map_ms"] = round(mean["isosurface"] + mean["vertex_materials"] + mean["normal_bands"], 2)
     os.remove(os.path.join(tmp, "export.glb"))
     os.rmdir(tmp)
     print(json.dumps(out))
