@@ -111,11 +111,24 @@ class _Link:
     """Shared by the two autograd nodes of the fused analytic-normal path.  The second-order node runs
     first in the backward sweep (its output feeds the MLP node) and, instead of scattering its table
     gradient right away, parks (v, g2) here; the first-order node then adds both contributions to the
-    table with ONE scatter pass (rsdf_hashgrid_bwd_table2)."""
-    __slots__ = ("v", "g2")
+    table with ONE scatter pass (rsdf_hashgrid_bwd_table2).
+
+    The pair is tagged with the autograd graph task (one backward sweep) that parked it, and only that sweep may
+    consume it: a backward that reaches the second-order node but not the first-order one (a gradient to g2 alone,
+    say) would otherwise leave a pair behind for a later, unrelated backward through the forward node to scatter."""
+    __slots__ = ("v", "g2", "task")
 
     def __init__(self):
-        self.v = self.g2 = None
+        self.v = self.g2 = self.task = None
+
+    def park(self, v, g2):
+        self.v, self.g2, self.task = v, g2, torch._C._current_graph_task_id()
+
+    def take(self):
+        """(v, g2) parked by the running backward sweep, else None; the link is empty afterwards either way."""
+        pair = (self.v, self.g2) if self.v is not None and self.task == torch._C._current_graph_task_id() else None
+        self.v = self.g2 = self.task = None
+        return pair
 
 
 class _HashGridForwardJ(torch.autograd.Function):
@@ -140,16 +153,17 @@ class _HashGridForwardJ(torch.autograd.Function):
         x, table, dy_dx = ctx.saved_tensors
         S, n_out = gy.shape
         gy = gy.contiguous()
-        link, gx, gt = ctx.link, None, None
+        gx, gt = None, None
+        parked = ctx.link.take() if ctx.link is not None else None
         if ctx.needs_input_grad[0]:
             gx = torch.empty(S, 3, device=gy.device, dtype=torch.float32)
             L.call("rsdf_hashgrid_bwd_input", L.ptr(dy_dx), L.ptr(gy), S, n_out, L.ptr(gx), L.stream())
         if ctx.needs_input_grad[1]:
             gt = torch.zeros_like(table)
-            if link is not None and link.v is not None:
-                L.call("rsdf_hashgrid_bwd_table2", L.ptr(x), L.ptr(gy), L.ptr(link.v), L.ptr(link.g2), ctx.meta.ref, S,
+            if parked is not None:
+                v, g2 = parked
+                L.call("rsdf_hashgrid_bwd_table2", L.ptr(x), L.ptr(gy), L.ptr(v), L.ptr(g2), ctx.meta.ref, S,
                        L.ptr(gt), L.stream())
-                link.v = link.g2 = None
             else:
                 L.call("rsdf_hashgrid_bwd_table", L.ptr(x), L.ptr(gy), ctx.meta.ref, S, L.ptr(gt), L.stream())
         return gx, gt, None, None
@@ -188,7 +202,7 @@ class _HashGridInputGrad(torch.autograd.Function):
             L.call("rsdf_hashgrid_bwd_bwd", L.ptr(x), L.ptr(table), L.ptr(v), L.ptr(g2), ctx.meta.ref, S,
                    None, None, L.ptr(g_x), L.stream())
         if table.requires_grad:
-            ctx.link.v, ctx.link.g2 = v, g2
+            ctx.link.park(v, g2)
         return g_g2, None, g_x, None, None, None
 
 
