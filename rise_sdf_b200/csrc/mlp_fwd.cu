@@ -39,7 +39,7 @@ static_assert(sizeof(MlpFwdParams) == sizeof(rsdf_mlp_fwd_params), "C-ABI struct
 
 template <int ACT>
 __device__ __forceinline__ float act_apply(float z) {
-    if (ACT == 1) return fmaxf(z, 0.0f);
+    if (ACT == 1) return z < 0.0f ? 0.0f : z;     // keeps NaN, as torch.relu does (fmaxf(NaN, 0) is 0)
     if (ACT == 2) {                        // torch Softplus(beta=100, threshold=20)
         const float t = 100.0f * z;
         return t > 20.0f ? z : log1pf(__expf(t)) * 0.01f;

@@ -217,7 +217,10 @@ __global__ void __launch_bounds__(THREADS, 1) relu_layer_fwd_kernel(const __grid
             float v[16];
             ld16(t, 0, v);
 #pragma unroll
-            for (int j = 0; j < 16; ++j) v[j] = fmaxf(v[j] + bf, 0.0f);
+            for (int j = 0; j < 16; ++j) {      // NaN-preserving ReLU (fmaxf(NaN, 0) is 0, torch.relu(NaN) is NaN)
+                const float z = v[j] + bf;
+                v[j] = z < 0.0f ? 0.0f : z;
+            }
             st16(out_img, t, v, p.fp16);
         } else if (t.q * 32 < p.r_real) {
             float v[16];
