@@ -579,6 +579,37 @@ int rsdf_bake_tangents(const float *v_pos, const int64_t *t_pos_idx, const float
 int rsdf_normal_pack(const float *v_nrm, const int64_t *t_pos_idx, const float *t_tangent, int64_t n_faces,
                      int texture_size, int row0, int n_rows, const float *grad, float *out, void *stream);
 
+/* ---------------------------------------------------------------- test-stage metrics (csrc/metrics.cu) */
+/* The scores of SplitOccSystem.test_step (systems/split_occ.py:417-424 with systems/criterions.py).  Images are
+ * [H, W, C] row-major fp32 with C in 1..4 and H * W * C < 2^31, masks [H, W] bytes (torch.bool, nonzero = selected);
+ * anything else is -1.  Arithmetic and sums are fp64.  partials: caller scratch of 2 * RSDF_METRIC_BLOCKS doubles,
+ * per-block sums added in a fixed order by a second one-block launch (bit-reproducible, no float atomics).
+ *   rsdf_sq_err_sum      : out2 = (sum (pred - gt)^2, number of summed elements) over the selected pixels (mask NULL:
+ *                          every pixel).
+ *   rsdf_ssim            : out[0] = mean SSIM (Wang et al. 2004) over the (H - 10) x (W - 10) valid pixels of every
+ *                          channel, no padding; H, W >= 11.  win11_host: HOST array of the 11 normalised window weights,
+ *                          applied along rows, then columns; C1 = 0.01^2, C2 = 0.03^2; population moments
+ *                          (sigma^2 = G*x^2 - mu^2, clamped at 0).
+ *   rsdf_normal_angle_sum: pred, gt [H, W, 3]: out2 = (sum of atan2(|a x b|, a . b) in degrees, count) over the
+ *                          selected pixels, a and b the two vectors divided by sqrt(max(|v|^2, 1e-20)); 90 degrees
+ *                          where a vector is zero.
+ *   rsdf_ratio_median    : out_scale[c] = the lower median (torch.median's for an even count) of the fp32 ratio
+ *                          gt / max(pred, eps) (a NaN pred stays NaN, as torch.clamp keeps it) over the selected pixels,
+ *                          bit-identical to torch.median; NaN when a selected ratio is NaN or no pixel is selected.
+ *                          Radix select on order-preserving keys in 4 passes of 8 bits (8 launches), without compacting
+ *                          the selection or reading anything back; scratch: RSDF_MEDIAN_SCRATCH_WORDS uint32 words,
+ *                          16-byte aligned. */
+#define RSDF_METRIC_BLOCKS 296
+#define RSDF_MEDIAN_SCRATCH_WORDS 4116
+int rsdf_sq_err_sum(const float *pred, const float *gt, const uint8_t *mask, int H, int W, int C, double *out2,
+                    double *partials, void *stream);
+int rsdf_ssim(const float *pred, const float *gt, int H, int W, int C, const double *win11_host, double *out,
+              double *partials, void *stream);
+int rsdf_normal_angle_sum(const float *pred, const float *gt, const uint8_t *mask, int H, int W, double *out2,
+                          double *partials, void *stream);
+int rsdf_ratio_median(const float *pred, const float *gt, const uint8_t *mask, int H, int W, int C, float eps,
+                      float *out_scale, uint32_t *scratch, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -145,6 +145,10 @@ _SIGS = {
     "rsdf_material_pack": [c_p, c_p, c_p, c_p, ctypes.c_int64, c_p, c_p],
     "rsdf_bake_tangents": [c_p, c_p, c_p, ctypes.c_int64, c_i, c_p, c_p],
     "rsdf_normal_pack": [c_p, c_p, c_p, ctypes.c_int64, c_i, c_i, c_i, c_p, c_p, c_p],
+    "rsdf_sq_err_sum": [c_p, c_p, c_p, c_i, c_i, c_i, c_p, c_p, c_p],
+    "rsdf_ssim": [c_p, c_p, c_i, c_i, c_i, c_p, c_p, c_p, c_p],
+    "rsdf_normal_angle_sum": [c_p, c_p, c_p, c_i, c_i, c_p, c_p, c_p],
+    "rsdf_ratio_median": [c_p, c_p, c_p, c_i, c_i, c_i, c_f, c_p, c_p, c_p],
 }
 
 
@@ -191,9 +195,12 @@ def stream():
 # kernels launched per C-ABI entry point (for bench.py's gpu_launches count)
 LAUNCHES = {"rsdf_march_count": 4, "rsdf_march_count_keep": 4, "rsdf_sdf_reg_fwd": 2, "rsdf_neus_loss_fwd": 2,
             "rsdf_occ_update": 2, "rsdf_occ_threshold": 3, "rsdf_mc_count": 2,
-            "rsdf_mc_slab_count": 2}
+            "rsdf_mc_slab_count": 2, "rsdf_sq_err_sum": 2, "rsdf_ssim": 2, "rsdf_normal_angle_sum": 2,
+            "rsdf_ratio_median": 8}
 SDF_REG_BLOCKS = 1184
 LOSS_BLOCKS = 296
+METRIC_BLOCKS = 296
+MEDIAN_SCRATCH_WORDS = 4116
 STATS = {"enabled": False, "launches": 0, "timed": set(), "events": {}}
 
 

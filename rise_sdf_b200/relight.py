@@ -6,6 +6,7 @@ is rendered in `tile`-ray tiles; every rank holds the full model, occupancy grid
 pyramids and LUT and keeps its result sharded (`frame[rank::world] = shard` assembles it)."""
 import torch
 
+from . import metrics
 from . import synthetic as syn
 from .light import blender_latlong_to_cubemap
 
@@ -104,6 +105,59 @@ def render_frame_shard(model, rays, envs, rank=0, world=1, tile=None, keys=("com
     out = {e: {k: torch.cat(v) if v else torch.zeros(0, 3, device=rays.device) for k, v in parts[e].items()}
            for e in range(n_env)}
     return out, tiles
+
+
+EVAL_KEYS = ("comp_rgb_phys_full", "comp_albedo", "comp_normal")
+
+
+@torch.no_grad()
+def evaluate_frame(model, rays, hw, envs, targets):
+    """Score one test view of a stage-1 SplitMixedOCCModel as SplitOccSystem.test_step does (systems/split_occ.py:
+    331-458, scores at :417-424): one render_frame_shard on this GPU (the albedo and normal keys ride along with the
+    env-shared tile cache), then the metrics of rise_sdf_b200.metrics.  rays: [H*W, 6] on the device, hw = (H, W),
+    envs: an EnvSet.  targets (every key optional): "mask" [H,W] bool, "albedo" [H,W,3] linear, "normal" [H,W,3]
+    world-space vectors in the model's frame, "relit" one [H,W,3] per env map in the model's output space (sRGB,
+    background composited with model.background_color).  Without a mask, albedo and normal scores cover every pixel.
+
+    Returns Python floats: albedo_scale (3 values: the per-channel median ratio), albedo_psnr (masked, after aligning
+    the prediction by albedo_scale, without clamping), albedo_ssim (the aligned prediction and the target, both set to 0
+    outside the mask: this project's choice), normal_mae (degrees, masked), relit_psnr / relit_ssim (one value per env
+    map, full frame).  All scalars are stacked on the device and read back once.  Averaging over views is the caller's."""
+    H, W = hw
+    relit = targets.get("relit")
+    if relit is not None and len(relit) != len(envs.maps):
+        raise ValueError(f"{len(relit)} relit targets for {len(envs.maps)} env maps")
+    out, _ = render_frame_shard(model, rays, envs, keys=EVAL_KEYS)
+    img = lambda e, k: out[e][k].view(H, W, 3)
+    mask = targets.get("mask")
+    if mask is None and ("albedo" in targets or "normal" in targets):
+        mask = torch.ones(H, W, dtype=torch.bool, device=rays.device)
+    parts = []                                    # (name, device tensor [n]), read back together
+    if "albedo" in targets:
+        gt = targets["albedo"]
+        scale = metrics.albedo_scale(img(0, "comp_albedo"), gt, mask)
+        aligned = img(0, "comp_albedo") * scale
+        m3 = mask[..., None]
+        parts += [("albedo_scale", scale.double()), ("albedo_psnr", metrics.psnr(aligned, gt, mask)),
+                  ("albedo_ssim", metrics.ssim(torch.where(m3, aligned, 0.0), torch.where(m3, gt, 0.0)))]
+    if "normal" in targets:
+        parts.append(("normal_mae", metrics.normal_mae(img(0, "comp_normal"), targets["normal"], mask)))
+    for e, gt in enumerate(relit or []):
+        rgb = img(e, "comp_rgb_phys_full")
+        parts += [("relit_psnr", metrics.psnr(rgb, gt)), ("relit_ssim", metrics.ssim(rgb, gt))]
+    if not parts:
+        return {}
+    flat = torch.cat([v.reshape(-1) for _, v in parts]).tolist()        # the frame's one device-to-host copy
+    res, i = {}, 0
+    for name, v in parts:
+        vals, i = flat[i:i + v.numel()], i + v.numel()
+        if name == "albedo_scale":
+            res[name] = vals
+        elif name in ("relit_psnr", "relit_ssim"):
+            res.setdefault(name, []).extend(vals)
+        else:
+            res[name] = vals[0]
+    return res
 
 
 def synthetic_envs():
