@@ -16,6 +16,16 @@
 
 static inline int rsdf_div_up(long long a, long long b) { return (int)((a + b - 1) / b); }
 
+// launch a kernel with `smem` bytes of dynamic shared memory (above the 48 KB default: the limit is raised first)
+template <class... P, class... A>
+static inline int rsdf_launch(void (*kernel)(P...), int grid, int block, size_t smem, void *stream, const A &...args) {
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return (int)e;
+    kernel<<<grid, block, smem, (cudaStream_t)stream>>>(args...);
+    RSDF_LAUNCH_CHECK();
+    return 0;
+}
+
 // B200: 148 SMs.  Grid-stride kernels size their grids as a multiple of this.
 #define RSDF_NUM_SMS 148
 

@@ -360,27 +360,19 @@ int rsdf_mm_stream(const float *X, const void *blob, const float *bias, float *Y
     const int k_pad = transposed ? rows_pad : cols_pad, n_pad = transposed ? cols_pad : rows_pad;
     if (K > k_pad || N > n_pad) return RSDF_EBADARG;
     const size_t sm = 196608 + sizeof(StreamSmem);
-    cudaError_t e = cudaFuncSetAttribute(mm_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-    if (e != cudaSuccess) return (int)e;
     const int n_tiles = (S + TM - 1) / TM;
     const int grid = n_tiles < RSDF_NUM_SMS ? n_tiles : RSDF_NUM_SMS;
-    mm_stream_kernel<<<grid, THREADS, sm, (cudaStream_t)stream>>>(X, (const uint8_t *)blob, bias, Y, S, K, N, rows_pad,
-                                                                 cols_pad, transposed, act);
-    RSDF_LAUNCH_CHECK();
-    return 0;
+    return rsdf_launch(mm_stream_kernel, grid, THREADS, sm, stream, X, (const uint8_t *)blob, bias, Y, S, K, N, rows_pad,
+                       cols_pad, transposed, act);
 }
 
 int rsdf_mm_tn(const float *A, const float *B, float *G, int S, int Fa, int Fb, void *stream) {
     if (S == 0) return 0;
     if (!A || !B || !G || Fa < 1 || Fa > 128 || Fb < 1 || Fb > 128) return RSDF_EBADARG;
     const size_t sm = 131072 + sizeof(StreamSmem);
-    cudaError_t e = cudaFuncSetAttribute(mm_tn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-    if (e != cudaSuccess) return (int)e;
     const int n_tiles = (S + TM - 1) / TM;
     const int grid = n_tiles < RSDF_NUM_SMS ? n_tiles : RSDF_NUM_SMS;
-    mm_tn_kernel<<<grid, THREADS, sm, (cudaStream_t)stream>>>(A, B, G, S, Fa, Fb);
-    RSDF_LAUNCH_CHECK();
-    return 0;
+    return rsdf_launch(mm_tn_kernel, grid, THREADS, sm, stream, A, B, G, S, Fa, Fb);
 }
 
 }  // extern "C"

@@ -643,13 +643,9 @@ int rsdf_hashgrid_fd6(const float *points, const float *table, const rsdf_hashgr
     if (!points || !table || !x01_out || !y || !(radius > 0.0f) || !load_meta(meta, m)) return RSDF_EBADARG;
     const int n_out = m.n_levels * NFEAT;
     const size_t sm = sizeof(float) * FD_S * 6 * (n_out + 2);
-    cudaError_t e = cudaFuncSetAttribute(hashgrid_fd6_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-    if (e != cudaSuccess) return (int)e;
     const float inv_2r = 1.0f / (radius - (-radius));          // fl32(1) / fl32(2r): torch's tensor / scalar on CUDA
-    hashgrid_fd6_kernel<<<rsdf_div_up(n_samples, FD_S), FD_THREADS, sm, (cudaStream_t)stream>>>(
-        points, table, m, n_samples, eps, radius, inv_2r, x01_out, y);
-    RSDF_LAUNCH_CHECK();
-    return 0;
+    return rsdf_launch(hashgrid_fd6_kernel, rsdf_div_up(n_samples, FD_S), FD_THREADS, sm, stream, points, table, m,
+                       n_samples, eps, radius, inv_2r, x01_out, y);
 }
 
 int rsdf_hashgrid_bwd_table2(const float *x, const float *dL_dy, const float *v, const float *g2,

@@ -119,11 +119,7 @@ __global__ void __launch_bounds__(THREADS, 1) mlp_fwd_kernel(const __grid_consta
 
     auto issue_w = [&](int job) {     // thread 0 only
         const MlpLayerDesc &L = p.layer[job % p.n_layers];
-#ifdef RSDF_EXP_NO_WLOAD             // developer experiment: only the first blobs are ever copied
-        const uint32_t bytes = job < 2 ? 4u * (uint32_t)L.n_pad * (uint32_t)L.k_pad : 16u;
-#else
         const uint32_t bytes = 4u * (uint32_t)L.n_pad * (uint32_t)L.k_pad;
-#endif
         tc::mbar_expect_tx(&sm->bar_w[job & 1], bytes);
         tc::bulk_g2s(w_img[job & 1], L.blob, bytes, &sm->bar_w[job & 1]);
     };
@@ -201,11 +197,9 @@ __global__ void __launch_bounds__(THREADS, 1) mlp_fwd_kernel(const __grid_consta
                 if (job & 1) w_phase1 ^= 1; else w_phase0 ^= 1;
                 tc::tc_fence_after();
                 const uint32_t idesc = tc::instr_desc(128, n_pad, false, false);
-#ifndef RSDF_EXP_NO_MMA
                 tc::gemm_split3(tmem, tc::op_kmajor(tc::smem_u32(a_img), TM * k_pad * 2, TM),
                                 tc::op_kmajor(tc::smem_u32(w_img[job & 1]), (uint32_t)n_pad * k_pad * 2, n_pad),
                                 k_pad / 16, idesc, false, /*keep_lo_lo=*/false);
-#endif
                 tc::mma_commit(&sm->bar_mma);
                 if (job + 1 < total_jobs) issue_w(job + 1);   // other ring slot: its last reader has drained
             }
@@ -217,10 +211,6 @@ __global__ void __launch_bounds__(THREADS, 1) mlp_fwd_kernel(const __grid_consta
             const int n_chunks = n_pad / 16, per = (n_chunks + PARTS - 1) / PARTS;
             const int c_begin = min(part * per, n_chunks), c_end = min(c_begin + per, n_chunks);
             const float *bias = sm->bias[l];
-#ifdef RSDF_EXP_NO_EPI
-            if (!last) {
-            } else
-#endif
             if (!last) {
                 const uint32_t next_plane = TM * n_pad * 2;
                 for (int c = c_begin; c < c_end; ++c)
@@ -260,13 +250,8 @@ int rsdf_mlp_fwd(const rsdf_mlp_fwd_params *params_host, void *stream) {
     }
     if (p.out_w > p.layer[p.n_layers - 1].n_pad) return RSDF_EBADARG;
     const size_t smem = 196608 + sizeof(MlpSmem);
-    cudaError_t e = cudaFuncSetAttribute(mlp_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
     const int n_tiles = (p.S + TM - 1) / TM;
-    const int grid = n_tiles < RSDF_NUM_SMS ? n_tiles : RSDF_NUM_SMS;
-    mlp_fwd_kernel<<<grid, THREADS, smem, (cudaStream_t)stream>>>(p);
-    RSDF_LAUNCH_CHECK();
-    return 0;
+    return rsdf_launch(mlp_fwd_kernel, n_tiles < RSDF_NUM_SMS ? n_tiles : RSDF_NUM_SMS, THREADS, smem, stream, p);
 }
 
 }  // extern "C"

@@ -111,14 +111,10 @@ tc_gemm_test_kernel(int mode, const float *__restrict__ A, const uint8_t *__rest
                     const float x1 = (s < S && k + 1 < d_a) ? A[(size_t)s * d_a + k + 1] : 0.0f;
                     tc::split2(x0, x1, hi[j], lo[j]);
                 }
-                asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};"
-                             ::"r"(tl + COL_AHI + c8 * 8), "r"(hi[0]), "r"(hi[1]), "r"(hi[2]), "r"(hi[3]), "r"(hi[4]),
-                               "r"(hi[5]), "r"(hi[6]), "r"(hi[7]) : "memory");
-                asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};"
-                             ::"r"(tl + COL_ALO + c8 * 8), "r"(lo[0]), "r"(lo[1]), "r"(lo[2]), "r"(lo[3]), "r"(lo[4]),
-                               "r"(lo[5]), "r"(lo[6]), "r"(lo[7]) : "memory");
+                tc::tmem_st8(tl + COL_AHI + c8 * 8, hi);
+                tc::tmem_st8(tl + COL_ALO + c8 * 8, lo);
             }
-            asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+            tc::tmem_st_wait();
             tc::tc_fence_before();
         }
         tc::fence_async_smem();
@@ -126,23 +122,10 @@ tc_gemm_test_kernel(int mode, const float *__restrict__ A, const uint8_t *__rest
         if (tid == 0) {
             tc::tc_fence_after();
             if (mode == 3) {
+                // the split GEMM and tcgen05.st / mma wrappers of sdf_eval_ts_kernel
                 const uint32_t idesc = tc::instr_desc(128, w_rows_pad, false, false);
-                const tc::Operand B = tc::op_kmajor(tc::smem_u32(b_img), b_plane, w_rows_pad);
-                const int ksteps = a_pad / 16;
-                for (int term = 0; term < 3; ++term) {
-                    const uint32_t a0 = tmem + (term == 0 ? COL_ALO : COL_AHI);
-                    const uint32_t b0 = B.addr + (term == 1 ? B.plane : 0u);
-                    for (int k = 0; k < ksteps; ++k) {
-                        const uint64_t bd = tc::smem_desc(b0 + k * B.kstep, B.lbo, B.sbo);
-                        const uint32_t acc = (term > 0 || k > 0) ? 1u : 0u, z = 0u;
-                        asm volatile(
-                            "{\n\t"
-                            ".reg .pred p;\n\t"
-                            "setp.ne.b32 p, %4, 0;\n\t"
-                            "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, {%5, %5, %5, %5}, p;\n\t"
-                            "}" ::"r"(tmem), "r"(a0 + k * 8), "l"(bd), "r"(idesc), "r"(acc), "r"(z) : "memory");
-                    }
-                }
+                tc::gemm_split3_ts(tmem, tmem + COL_AHI, tmem + COL_ALO,
+                                   tc::op_kmajor(tc::smem_u32(b_img), b_plane, w_rows_pad), a_pad / 16, idesc);
             } else if (mode == 0) {
                 // D[128 x N] = A(K-major, K=a_pad) * W(K-major: rows N_pad, K=w_cols_pad)
                 const uint32_t idesc = tc::instr_desc(128, w_rows_pad, false, false);
@@ -213,12 +196,8 @@ int rsdf_tc_gemm_test(int mode, const float *A, const void *Wblob, const float *
                       int d_b, int w_rows_pad, int w_cols_pad, int grid, void *stream) {
     if (!A || !C || S <= 0 || d_a > 128 || d_b > 128) return RSDF_EBADARG;
     const size_t sm = 131072 + 64;
-    cudaError_t e = cudaFuncSetAttribute(tc_gemm_test_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-    if (e != cudaSuccess) return (int)e;
-    tc_gemm_test_kernel<<<grid, 128, sm, (cudaStream_t)stream>>>(mode, A, (const uint8_t *)Wblob, Y, C, S, d_a,
-                                                                  d_b, w_rows_pad, w_cols_pad);
-    RSDF_LAUNCH_CHECK();
-    return 0;
+    return rsdf_launch(tc_gemm_test_kernel, grid, 128, sm, stream, mode, A, (const uint8_t *)Wblob, Y, C, S, d_a, d_b,
+                       w_rows_pad, w_cols_pad);
 }
 
 

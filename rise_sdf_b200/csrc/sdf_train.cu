@@ -31,34 +31,14 @@
 // their activation-side operand carries the complementary factor 2^(K - k_s) <= 1 (K from the launch-wide
 // cotangent maximum, rsdf_absmax2): the accumulators hold 2^K * dW, precise relative to the samples
 // that dominate the sum.
-#include "common.cuh"
-#include "tc.cuh"
+#include "sdf_net.cuh"
 
 namespace {
 
 constexpr int NS = 64;                    // samples per tile (UMMA N)
-constexpr int THREADS = 512;
-constexpr int HID = 128;
-constexpr int KP = 48;                    // padded width of the input and output sides
 constexpr uint32_t IMG_S_PLANE = KP * 128;       // [48 feature rows x 64 samples] fp16 plane
 constexpr uint32_t IMG_B_PLANE = HID * 128;      // [128 x 64]
 constexpr uint32_t IMG_S_BYTES = 2 * IMG_S_PLANE, IMG_B_BYTES = 2 * IMG_B_PLANE;
-constexpr uint32_t W1_PLANE = HID * KP * 2, W2_PLANE = HID * HID * 2, W3_PLANE = KP * HID * 2;
-constexpr uint32_t W1_OFF = 0, W2_OFF = W1_OFF + 2 * W1_PLANE, W3_OFF = W2_OFF + 2 * W2_PLANE;
-constexpr uint32_t W_END = W3_OFF + 2 * W3_PLANE;                                   // 114688
-
-struct Net {
-    const uint8_t *w1, *w2, *w3;          // blobs: [128 x 48], [128 x 128], [48 x 128] (rows x cols, padded)
-    const float *b1, *b2, *b3, *w3r0;     // fp32 biases and row 0 of W3 (the sdf head)
-    int n_in, n_out;
-    int fp16;                             // != 0: the single-plane fp16 variant
-};
-struct Inputs {
-    const float *in0, *in1;               // h0 = cat(in0 * sc0 + sh0, in1)
-    int w0, w1;
-    float sc0, sh0;
-    int S;
-};
 
 // 16 warps: warp w owns TMEM lane quadrant w%4 (feature rows 32*(w%4)..+31) and the 16 sample
 // columns [16*(w/4), +16) of the tile
@@ -68,20 +48,12 @@ struct Tid {
 };
 
 __device__ __forceinline__ void ld16(const Tid &t, int col, float *v) {
-#ifdef RSDF_EXP_NO_LDST         // developer experiment: the chain's synchronisation skeleton alone
-    for (int j = 0; j < 16; ++j) v[j] = (float)col;
-    return;
-#endif
     tc::tmem_ld16(t.tl + (uint32_t)(col + t.col0), v);
     tc::tmem_ld_wait();
 }
 // several TMEM regions wanted together: issue the loads back to back and wait once (one TMEM round trip instead of
 // one per region on the critical path of the GEMM -> epilogue chain)
 __device__ __forceinline__ void ld16_issue(const Tid &t, int col, float *v) {
-#ifdef RSDF_EXP_NO_LDST
-    for (int j = 0; j < 16; ++j) v[j] = (float)col;
-    return;
-#endif
     tc::tmem_ld16(t.tl + (uint32_t)(col + t.col0), v);
 }
 // SPLIT = true : fp32-class arithmetic, every operand an fp16 hi|lo pair and every GEMM three products (tc.cuh)
@@ -90,10 +62,6 @@ __device__ __forceinline__ void ld16_issue(const Tid &t, int col, float *v) {
 // this thread's 16 samples of feature row f -> two 16-byte chunks per plane of a [128 x 64] image
 template <bool SPLIT = true>
 __device__ __forceinline__ void st16(uint8_t *img, const Tid &t, const float *v) {
-#ifdef RSDF_EXP_NO_LDST
-    if (v[0] == 12345.678f) img[0] = 1;
-    return;
-#endif
     const int c = t.col0 >> 3;
     if (SPLIT) {
         tc::store_chunk(img, IMG_B_PLANE, HID, t.f, c, v);
@@ -104,49 +72,11 @@ __device__ __forceinline__ void st16(uint8_t *img, const Tid &t, const float *v)
     }
 }
 
-// 3-product split GEMM, fully unrolled; descriptors advance by adding to the 14-bit address field
-template <int KSTEPS, bool SPLIT = true>
+// the training issuer's GEMMs: lo*hi, hi*lo, hi*hi (hi*hi alone in the fp16 variant), one rolled k loop per product
+template <int KSTEPS, bool SPLIT>
 __device__ __forceinline__ void gemm3(uint32_t d, const tc::Operand &A, const tc::Operand &B, uint32_t idesc,
                                       bool accumulate) {
-    const uint64_t a_hi = tc::smem_desc(A.addr, A.lbo, A.sbo), a_lo = tc::smem_desc(A.addr + A.plane, A.lbo, A.sbo);
-    const uint64_t b_hi = tc::smem_desc(B.addr, B.lbo, B.sbo), b_lo = tc::smem_desc(B.addr + B.plane, B.lbo, B.sbo);
-    const uint64_t ak = A.kstep >> 4, bk = B.kstep >> 4;
-    if (SPLIT) {
-#pragma unroll
-        for (int k = 0; k < KSTEPS; ++k) tc::mma_f16(d, a_lo + k * ak, b_hi + k * bk, idesc, accumulate || k > 0);
-#pragma unroll
-        for (int k = 0; k < KSTEPS; ++k) tc::mma_f16(d, a_hi + k * ak, b_lo + k * bk, idesc, true);
-    }
-#pragma unroll
-    for (int k = 0; k < KSTEPS; ++k) tc::mma_f16(d, a_hi + k * ak, b_hi + k * bk, idesc, SPLIT || accumulate || k > 0);
-}
-
-// The same GEMM for the dedicated issuer warp of the training kernels, ROLLED: the issuer runs ~40 GEMMs per tile and a
-// fully unrolled issue stream keeps hundreds of precomputed 64-bit descriptors live -- they spill, and every spill reload
-// of the single issuing lane is an L2 round trip in front of an MMA (ncu: 1500 local loads per tile, 32 % L1 hit).
-// Rolled, a descriptor is two 64-bit adds away from its base and nothing outlives the call.
-template <int KSTEPS, bool SPLIT>
-__device__ __forceinline__ void gemm3r(uint32_t d, const tc::Operand &A, const tc::Operand &B, uint32_t idesc,
-                                       bool accumulate) {
-#ifdef RSDF_EXP_NO_MMA          // developer experiment (scripts/exp_sdf_chain.sh): the chain without tensor work
-    return;
-#endif
-    // the address is the low 14 bits of the descriptor's low word and never carries out of it: stepping a descriptor
-    // is ONE 32-bit add, the high word (LBO | SBO | version) is per-operand constant
-    const uint64_t a0 = tc::smem_desc(A.addr, A.lbo, A.sbo), b0 = tc::smem_desc(B.addr, B.lbo, B.sbo);
-    const uint32_t a_hi32 = (uint32_t)(a0 >> 32), b_hi32 = (uint32_t)(b0 >> 32);
-    const uint32_t a_lo32 = (uint32_t)a0, b_lo32 = (uint32_t)b0;
-    const uint32_t ak = A.kstep >> 4, bk = B.kstep >> 4, apl = A.plane >> 4, bpl = B.plane >> 4;
-    auto pass = [&](uint32_t a, uint32_t b, bool acc0) {
-#pragma unroll 1
-        for (int k = 0; k < KSTEPS; ++k, a += ak, b += bk)
-            tc::mma_f16(d, ((uint64_t)a_hi32 << 32) | a, ((uint64_t)b_hi32 << 32) | b, idesc, acc0 || k > 0);
-    };
-    if (SPLIT) {
-        pass(a_lo32 + apl, b_lo32, accumulate);
-        pass(a_lo32, b_lo32 + bpl, true);
-    }
-    pass(a_lo32, b_lo32, SPLIT || accumulate);
+    tc::gemm_split3<tc::ROLL_K, KSTEPS>(d, A, B, KSTEPS, idesc, accumulate, /*keep_lo_lo=*/false, SPLIT);
 }
 // a zero the compiler cannot see through: operands built from it are recomputed where they are used instead of being
 // hoisted out of the persistent tile loop (and spilled)
@@ -155,51 +85,6 @@ __device__ __forceinline__ uint32_t opaque_zero() {
     asm volatile("mov.u32 %0, 0;" : "=r"(z));
     return z;
 }
-
-__device__ __forceinline__ float exp2f_fast(float x) {
-    float y;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
-// softplus(beta=100, threshold=20) and its first two derivatives, torch semantics (aten softplus /
-// softplus_backward / its double-backward formula).  With e = exp(-|t|) in (0,1]:
-//   softplus = max(z,0) + log(1+e)/beta,  sigmoid(t) = 1/(1+e) or e/(1+e),  sigmoid' = beta e/(1+e)^2.
-// The fast intrinsics are safe here: their absolute error (~2^-22) is divided by beta = 100 in the
-// activation and enters the derivatives at <= 3e-7.
-// Branch-free: for t > 20, e < 2.1e-9 so 1 + e == 1 in fp32 and the activation / sigmoid reduce to z / 1
-// exactly as torch's threshold branch does; only sigmoid' needs the explicit select.
-constexpr float SP_K = 100.0f * 1.4426950408889634f;          // beta * log2(e)
-constexpr float SP_L = 0.01f * 0.6931471805599453f;           // ln(2) / beta
-#ifdef RSDF_EXP_NO_MATH         // developer experiment: the chain without the transcendental epilogue math
-__device__ __forceinline__ void sp_sig_dsig(float z, float &s, float &ds) { s = z; ds = z; }
-__device__ __forceinline__ void sp_all(float z, float &a, float &s, float &ds) { a = z; s = z; ds = z; }
-__device__ __forceinline__ float sp_act(float z) { return z; }
-__device__ __forceinline__ float sp_sig(float z) { return z; }
-#else
-__device__ __forceinline__ void sp_sig_dsig(float z, float &s, float &ds) {
-    const float e = exp2f_fast(-fabsf(z) * SP_K);
-    const float r = __fdividef(1.0f, 1.0f + e);
-    const float er = e * r;
-    s = z >= 0.0f ? r : er;
-    ds = z > 0.2f ? 0.0f : 100.0f * er * r;
-}
-__device__ __forceinline__ void sp_all(float z, float &a, float &s, float &ds) {
-    const float e = exp2f_fast(-fabsf(z) * SP_K);
-    const float r = __fdividef(1.0f, 1.0f + e);
-    const float er = e * r;
-    a = fmaf(SP_L, __log2f(1.0f + e), fmaxf(z, 0.0f));
-    s = z >= 0.0f ? r : er;
-    ds = z > 0.2f ? 0.0f : 100.0f * er * r;
-}
-__device__ __forceinline__ float sp_act(float z) {
-    return fmaf(SP_L, __log2f(1.0f + exp2f_fast(-fabsf(z) * SP_K)), fmaxf(z, 0.0f));
-}
-__device__ __forceinline__ float sp_sig(float z) {
-    const float e = exp2f_fast(-fabsf(z) * SP_K);
-    const float r = __fdividef(1.0f, 1.0f + e);
-    return z >= 0.0f ? r : e * r;
-}
-#endif
 
 // Row-major global -> registers: thread (f = tid % 64, c = tid / 64) fetches the 8-sample chunk
 // (samples s0 + 8c .. +7) of feature row f; a warp reads 32 consecutive floats of one sample row per
@@ -301,15 +186,6 @@ __device__ __forceinline__ Tid make_tid() {
     return t;
 }
 
-__device__ __forceinline__ void load_weights(uint8_t *smem, const Net &net, uint64_t *bar, int tid) {
-    if (tid == 0) {
-        tc::mbar_expect_tx(bar, W_END);
-        tc::bulk_g2s(smem + W1_OFF, net.w1, 2 * W1_PLANE, bar);
-        tc::bulk_g2s(smem + W2_OFF, net.w2, 2 * W2_PLANE, bar);
-        tc::bulk_g2s(smem + W3_OFF, net.w3, 2 * W3_PLANE, bar);
-    }
-}
-
 // ---- half-tile ping-pong ---------------------------------------------------------------------------
 // The per-tile work is a strict chain  GEMM -> epilogue -> GEMM -> ...  (7 links in the backward), and with one tile in
 // flight the tensor pipe idles during every epilogue and all 16 epilogue warps idle during every GEMM (measured:
@@ -325,51 +201,18 @@ constexpr int TR_GRP = 256, TR_THREADS = 2 * TR_GRP + 32, HS = NS / 2;
 // issuer's share to the epilogue warps with setmaxnreg is bounded by the CTA's LAUNCH allocation, not the SM's file --
 // 4 x 128 x 112 + 128 x 40 exceeds 640 x 96 and the last warpgroup's setmaxnreg.inc never returns -- and an issuer at
 // the 24 registers that would fit cannot hold its descriptors; not used.)
-struct TrCtrl {
-    uint64_t bar_w, done[2], ready[2];
-    uint32_t tmem_slot, pad;
-};
-__device__ __forceinline__ void grp_sync(int g) {
-    asm volatile("bar.sync %0, %1;" ::"r"(1 + g), "n"(TR_GRP) : "memory");
-}
-__device__ __forceinline__ void bar_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tc::smem_u32(bar)) : "memory");
-}
 // sample-half g of an operand: MN-major (samples on N: 4 chunks of 8) / K-major over samples (2 k-steps of 16)
 __device__ __forceinline__ tc::Operand half_n(tc::Operand o, int g) { o.addr += (uint32_t)g * 4u * o.sbo; return o; }
 __device__ __forceinline__ tc::Operand half_k(tc::Operand o, int g) { o.addr += (uint32_t)g * 2u * o.kstep; return o; }
 
-// group side: publish this group's smem image writes / TMEM reads and hand its half to the issuer; wait for the GEMMs
-// (one arrival per WARP -- ready[g] counts the group's 8 warps -- instead of a named barrier over the group followed by a
-// single arrival: the group's warps need not meet each other, only the issuer has to see all of them)
-#define TR_READY() { tc::fence_async_smem(); tc::tc_fence_before(); __syncwarp(); if (t.lane == 0) bar_arrive(&ct->ready[g]); }
-#define TR_WAIT() { tc::mbar_wait(&ct->done[g], dpar); dpar ^= 1u; tc::tc_fence_after(); }
-// issuer side: one link of the chain for half 0, then for half 1
-#define TR_ISSUE(...)                                          \
-    {                                                          \
-        _Pragma("unroll 1")                                    \
-        for (int g = 0; g < 2; ++g) {                          \
-            tc::mbar_wait(&ct->ready[g], rpar);                \
-            tc::tc_fence_after();                              \
-            if (tc::elect_one()) {                             \
-                __VA_ARGS__                                    \
-                tc::mma_commit(&ct->done[g]);                  \
-            }                                                  \
-            __syncwarp();                                      \
-        }                                                      \
-        rpar ^= 1u;                                            \
-    }
-
-__device__ __forceinline__ void tr_init(TrCtrl *ct, const Tid &t, uint32_t tmem_cols) {
-    if (t.tid == 0) {
-        tc::mbar_init(&ct->bar_w, 1);
-        for (int i = 0; i < 2; ++i) { tc::mbar_init(&ct->done[i], 1); tc::mbar_init(&ct->ready[i], TR_GRP / 32); }
-        tc::mbar_fence_init();
-    }
-    if (t.warp == 0) tc::tmem_alloc(&ct->tmem_slot, tmem_cols);
-    tc::tc_fence_before();
-    __syncthreads();
-    tc::tc_fence_after();
+// issuer side of one link of the chain: half 0's GEMMs, then half 1's.  The group side hands its half over with one
+// arrival per WARP (ready[g] counts the group's 8 warps) instead of a named barrier over the group followed by a single
+// arrival: the group's warps need not meet each other, only the issuer has to see all of them.
+template <class F>
+__device__ __forceinline__ void issue_link(tc::Pipe *ct, uint32_t &rpar, F &&body) {
+#pragma unroll 1
+    for (int g = 0; g < 2; ++g) tc::issue(ct, g, rpar, [&] { body(g); });
+    rpar ^= 1u;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -383,12 +226,12 @@ __global__ void __launch_bounds__(TR_THREADS, 1)
 sdf_fwd_kernel(const Net net, const Inputs in, float *__restrict__ out, float *__restrict__ sdf,
                float *__restrict__ g0a, float *__restrict__ g0b) {
     extern __shared__ __align__(1024) uint8_t smem[];
-    TrCtrl *ct = reinterpret_cast<TrCtrl *>(smem + F_CTRL);
+    tc::Pipe *ct = reinterpret_cast<tc::Pipe *>(smem + F_CTRL);
     uint8_t *h0_img = smem + F_H0, *big_a = smem + F_BIGA, *big_b = smem + F_BIGB;
     Tid t = make_tid();
-    tr_init(ct, t, 256);
+    tc::pipe_init(ct, TR_GRP / 32, 256);
     const uint32_t tmem = ct->tmem_slot;
-    load_weights(smem, net, &ct->bar_w, t.tid);
+    load_weights(smem, net, &ct->bar_w);
     constexpr uint32_t Z1 = 0, Z2 = 64, T0 = 128, T1 = 192;
     const int n_tiles = (in.S + NS - 1) / NS;
     if (t.warp == 2 * TR_GRP / 32) {
@@ -408,14 +251,17 @@ sdf_fwd_kernel(const Net net, const Inputs in, float *__restrict__ out, float *_
             const tc::Operand H0n = tc::op_mnmajor(sH0 + z, IMG_S_PLANE, KP), An = tc::op_mnmajor(sA + z, IMG_B_PLANE, HID),
                               Bn = tc::op_mnmajor(sB + z, IMG_B_PLANE, HID);
             // P1: Z1 = W1 h0
-            TR_ISSUE(gemm3r<KP / 16, SPLIT>(tmem + Z1 + HS * g, W1k, half_n(H0n, g), id_kn, false);)
+            issue_link(ct, rpar, [&](int g) { gemm3<KP / 16, SPLIT>(tmem + Z1 + HS * g, W1k, half_n(H0n, g), id_kn, false); });
             // P2: Z2 = W2 a1
-            TR_ISSUE(gemm3r<HID / 16, SPLIT>(tmem + Z2 + HS * g, W2k, half_n(An, g), id_kn, false);)
+            issue_link(ct, rpar, [&](int g) { gemm3<HID / 16, SPLIT>(tmem + Z2 + HS * g, W2k, half_n(An, g), id_kn, false); });
             // P3: out = W3 a2 (lanes >= 48 are don't-care);  v1 = W2^T u2
-            TR_ISSUE(gemm3r<HID / 16, SPLIT>(tmem + T0 + HS * g, W3k, half_n(An, g), id_kn, false);
-                     if (WITH_GRAD) gemm3r<HID / 16, SPLIT>(tmem + T1 + HS * g, W2t, half_n(Bn, g), id_tn, false);)
+            issue_link(ct, rpar, [&](int g) {
+                gemm3<HID / 16, SPLIT>(tmem + T0 + HS * g, W3k, half_n(An, g), id_kn, false);
+                if (WITH_GRAD) gemm3<HID / 16, SPLIT>(tmem + T1 + HS * g, W2t, half_n(Bn, g), id_tn, false);
+            });
             // P4: g0 = W1^T u1 (lanes >= 48 don't-care)
-            if (WITH_GRAD) TR_ISSUE(gemm3r<HID / 16, SPLIT>(tmem + T0 + HS * g, W1t, half_n(An, g), id_tn, false);)
+            if (WITH_GRAD)
+                issue_link(ct, rpar, [&](int g) { gemm3<HID / 16, SPLIT>(tmem + T0 + HS * g, W1t, half_n(An, g), id_tn, false); });
         }
     } else {
         // ---- epilogue group g: thread = feature row f x 16 of the half's 32 sample columns -----------------
@@ -431,10 +277,10 @@ sdf_fwd_kernel(const Net net, const Inputs in, float *__restrict__ out, float *_
             const int s0 = tile * NS;
             affine_chunk8(src_h, t.tid, s0, in.S, hv);
             store_chunk8<SPLIT>(h0_img, t, hv);
-            TR_READY()                                               // P1
+            tc::group_ready<tc::PER_WARP>(ct, g, t.lane == 0);  // P1
             // prefetch the next tile's inputs; they land while this tile computes
             if (tile + (int)gridDim.x < n_tiles) load_chunk8<false>(src_h, t.tid, (tile + gridDim.x) * NS, in.S, hv);
-            TR_WAIT()
+            tc::group_wait(ct, g, dpar);
             {
                 float v[16];
                 ld16(t, Z1, v);
@@ -442,8 +288,8 @@ sdf_fwd_kernel(const Net net, const Inputs in, float *__restrict__ out, float *_
                 for (int j = 0; j < 16; ++j) v[j] = sp_act(v[j] + b1f);
                 st16<SPLIT>(big_a, t, v);
             }
-            TR_READY()                                               // P2
-            TR_WAIT()
+            tc::group_ready<tc::PER_WARP>(ct, g, t.lane == 0);  // P2
+            tc::group_wait(ct, g, dpar);
             {
                 float v[16], u[16];
                 ld16(t, Z2, v);
@@ -457,8 +303,8 @@ sdf_fwd_kernel(const Net net, const Inputs in, float *__restrict__ out, float *_
                 st16<SPLIT>(big_a, t, v);                            // a2 (a1's MMA has drained)
                 if (WITH_GRAD) st16<SPLIT>(big_b, t, u);             // u2 = s2 . W3[0,:]
             }
-            TR_READY()                                               // P3
-            TR_WAIT()
+            tc::group_ready<tc::PER_WARP>(ct, g, t.lane == 0);  // P3
+            tc::group_wait(ct, g, dpar);
             store_rows(out, net.n_out, 1.0f, nullptr, 0, s0, in.S, t, T0, b3f, nullptr);
             if (sdf && t.q == 0) {            // the sdf head (feature row 0) once more as its own [S] array
                 float v[16];
@@ -485,8 +331,8 @@ sdf_fwd_kernel(const Net net, const Inputs in, float *__restrict__ out, float *_
 #pragma unroll
                 for (int j = 0; j < 16; ++j) v[j] *= sp_sig(z[j] + b1f);
                 st16<SPLIT>(big_a, t, v);                            // u1 = s1 . v1
-                TR_READY()                                           // P4
-                TR_WAIT()
+                tc::group_ready<tc::PER_WARP>(ct, g, t.lane == 0);  // P4
+                tc::group_wait(ct, g, dpar);
                 store_rows(g0a, in.w0, 1.0f, g0b, in.w1, s0, in.S, t, T0, 0.0f, nullptr);
             }
         }
@@ -520,7 +366,7 @@ template <bool CHAIN, bool SPLIT, bool SDF_ONLY = false>
 __global__ void __launch_bounds__(TR_THREADS, 1)
 sdf_bwd_kernel(const Net net, const Inputs in, const Grads g_) {
     extern __shared__ __align__(1024) uint8_t smem[];
-    TrCtrl *ct = reinterpret_cast<TrCtrl *>(smem + B_CTRL);
+    tc::Pipe *ct = reinterpret_cast<tc::Pipe *>(smem + B_CTRL);
     uint32_t *smax = reinterpret_cast<uint32_t *>(smem + B_CTRL + 64);   // [64] per-sample |cotangent| max (bits)
     float *ssc = reinterpret_cast<float *>(smax + NS);                    // [64] 2^k_s
     float *sinv = ssc + NS;                                               // [64] 2^-k_s
@@ -530,10 +376,10 @@ sdf_bwd_kernel(const Net net, const Inputs in, const Grads g_) {
             *big_a = smem + B_BIGA, *big_b = smem + B_BIGB;
     Tid t = make_tid();
     if (t.tid < NS) smax[t.tid] = 0u;
-    tr_init(ct, t, 512);
+    tc::pipe_init(ct, TR_GRP / 32, 512);
     const uint32_t tmem = ct->tmem_slot;
     t.tl = tmem + ((uint32_t)((t.q & 3) * 32) << 16);
-    load_weights(smem, net, &ct->bar_w, t.tid);
+    load_weights(smem, net, &ct->bar_w);
     constexpr uint32_t AW2 = 0, AW1 = 128, AW3 = 176, Z1 = 224, Z2 = 288, T0 = 352, T1 = 416;
     constexpr int KS = HS / 16;           // k-steps of a half's sample contraction
     const int n_tiles = (in.S + NS - 1) / NS;
@@ -566,32 +412,40 @@ sdf_bwd_kernel(const Net net, const Inputs in, const Grads g_) {
                               Bk = tc::op_kmajor(sB + z, IMG_B_PLANE, HID);
             const bool acc = it > 0;
             // P1: Z1 = W1 h0
-            TR_ISSUE(gemm3r<KP / 16, SPLIT>(tmem + Z1 + HS * g, W1k, half_n(H0n, g), id_kn, false);)
+            issue_link(ct, rpar, [&](int g) { gemm3<KP / 16, SPLIT>(tmem + Z1 + HS * g, W1k, half_n(H0n, g), id_kn, false); });
             // P2: Z2 = W2 a1
-            TR_ISSUE(gemm3r<HID / 16, SPLIT>(tmem + Z2 + HS * g, W2k, half_n(An, g), id_kn, false);)
+            issue_link(ct, rpar, [&](int g) { gemm3<HID / 16, SPLIT>(tmem + Z2 + HS * g, W2k, half_n(An, g), id_kn, false); });
             // P3: gW3^T += a2 g_out^T ; v1 = W2^T u2 ; ub1 = W1 g_g0   (no chain: ab2 = W3^T g_out right away)
             if (!SDF_ONLY)
-            TR_ISSUE(gemm3r<KS, SPLIT>(tmem + AW3, half_k(Ak, g), half_k(GOk, g), id_g48, acc || g);
-                     if (CHAIN) {
-                         gemm3r<HID / 16, SPLIT>(tmem + T0 + HS * g, W2t, half_n(Bn, g), id_tn, false);
-                         gemm3r<KP / 16, SPLIT>(tmem + T1 + HS * g, W1k, half_n(GGn, g), id_kn, false);
-                     } else {
-                         gemm3r<KP / 16, SPLIT>(tmem + T1 + HS * g, W3t, half_n(GOn, g), id_tn, false);
-                     })
+                issue_link(ct, rpar, [&](int g) {
+                    gemm3<KS, SPLIT>(tmem + AW3, half_k(Ak, g), half_k(GOk, g), id_g48, acc || g);
+                    if (CHAIN) {
+                        gemm3<HID / 16, SPLIT>(tmem + T0 + HS * g, W2t, half_n(Bn, g), id_tn, false);
+                        gemm3<KP / 16, SPLIT>(tmem + T1 + HS * g, W1k, half_n(GGn, g), id_kn, false);
+                    } else {
+                        gemm3<KP / 16, SPLIT>(tmem + T1 + HS * g, W3t, half_n(GOn, g), id_tn, false);
+                    }
+                });
             if (CHAIN) {
                 // P4: gW1 += u1 g_g0^T
-                TR_ISSUE(gemm3r<KS, SPLIT>(tmem + AW1, half_k(Ak, g), half_k(GGk, g), id_g48, acc || g);)
+                issue_link(ct, rpar, [&](int g) { gemm3<KS, SPLIT>(tmem + AW1, half_k(Ak, g), half_k(GGk, g), id_g48, acc || g); });
                 // P5: gW2 += u2 vb1^T ; ub2 = W2 vb1 ; ab2 = W3^T g_out
-                TR_ISSUE(gemm3r<KS, SPLIT>(tmem + AW2, half_k(Bk, g), half_k(Ak, g), id_g128, acc || g);
-                         gemm3r<HID / 16, SPLIT>(tmem + T0 + HS * g, W2k, half_n(An, g), id_kn, false);
-                         gemm3r<KP / 16, SPLIT>(tmem + T1 + HS * g, W3t, half_n(GOn, g), id_tn, false);)
+                issue_link(ct, rpar, [&](int g) {
+                    gemm3<KS, SPLIT>(tmem + AW2, half_k(Bk, g), half_k(Ak, g), id_g128, acc || g);
+                    gemm3<HID / 16, SPLIT>(tmem + T0 + HS * g, W2k, half_n(An, g), id_kn, false);
+                    gemm3<KP / 16, SPLIT>(tmem + T1 + HS * g, W3t, half_n(GOn, g), id_tn, false);
+                });
             }
             // P6: gW2 += zb2 a1^T ; ab1 = W2^T zb2
-            TR_ISSUE(gemm3r<KS, SPLIT>(tmem + AW2, half_k(Ak, g), half_k(Bk, g), id_g128, CHAIN || acc || g);
-                     gemm3r<HID / 16, SPLIT>(tmem + T0 + HS * g, W2t, half_n(An, g), id_tn, false);)
+            issue_link(ct, rpar, [&](int g) {
+                gemm3<KS, SPLIT>(tmem + AW2, half_k(Ak, g), half_k(Bk, g), id_g128, CHAIN || acc || g);
+                gemm3<HID / 16, SPLIT>(tmem + T0 + HS * g, W2t, half_n(An, g), id_tn, false);
+            });
             // P7: gW1 += zb1 h0^T ; d/d h0 = W1^T zb1
-            TR_ISSUE(gemm3r<KS, SPLIT>(tmem + AW1, half_k(Ak, g), half_k(H0Wk, g), id_g48, CHAIN || acc || g);
-                     gemm3r<HID / 16, SPLIT>(tmem + T0 + HS * g, W1t, half_n(An, g), id_tn, false);)
+            issue_link(ct, rpar, [&](int g) {
+                gemm3<KS, SPLIT>(tmem + AW1, half_k(Ak, g), half_k(H0Wk, g), id_g48, CHAIN || acc || g);
+                gemm3<HID / 16, SPLIT>(tmem + T0 + HS * g, W1t, half_n(An, g), id_tn, false);
+            });
         }
     } else {
         // ---- epilogue group g -----------------------------------------------------------------------------
@@ -645,7 +499,7 @@ sdf_bwd_kernel(const Net net, const Inputs in, const Grads g_) {
                     const uint32_t wm = __reduce_max_sync(0xffffffffu, __float_as_uint(m));
                     if (t.lane == 0 && wm != 0u) atomicMax(&smax[8 * cs + j], wm);
                 }
-                grp_sync(g);
+                tc::named_sync<TR_GRP>(1 + g);
                 if (tg < HS) {
                     const int sl = HS * g + tg;
                     const int e = (int)((smax[sl] >> 23) & 0xFFu);         // biased exponent of the sample's max
@@ -659,7 +513,7 @@ sdf_bwd_kernel(const Net net, const Inputs in, const Grads g_) {
                     ssc[sl] = sc; sinv[sl] = inv; swsc[sl] = wsc;
                     smax[sl] = 0u;
                 }
-                grp_sync(g);
+                tc::named_sync<TR_GRP>(1 + g);
                 float hw[8];
 #pragma unroll
                 for (int j = 0; j < 8; ++j) {
@@ -674,9 +528,9 @@ sdf_bwd_kernel(const Net net, const Inputs in, const Grads g_) {
                     store_chunk8<SPLIT>(gg_img, t, ggv);
                 }
             }
-            TR_READY()                                               // P1
+            tc::group_ready<tc::PER_WARP>(ct, g, t.lane == 0);  // P1
             if (tile + (int)gridDim.x < n_tiles) prefetch_tile((tile + gridDim.x) * NS);
-            TR_WAIT()
+            tc::group_wait(ct, g, dpar);
             const float *wsc = swsc + t.col0, *inv = sinv + t.col0;    // per-sample factors (smem broadcasts)
             {
                 float v[16];
@@ -685,8 +539,8 @@ sdf_bwd_kernel(const Net net, const Inputs in, const Grads g_) {
                 for (int j = 0; j < 16; ++j) v[j] = sp_act(v[j] + b1f);
                 st16<SPLIT>(big_a, t, v);                            // a1
             }
-            TR_READY()                                               // P2
-            TR_WAIT()
+            tc::group_ready<tc::PER_WARP>(ct, g, t.lane == 0);  // P2
+            tc::group_wait(ct, g, dpar);
             if (SDF_ONLY) {
                 // a2-bar = w3[0,f] g_sdf[s] and gW3[0,f] += a2[f,s] g_sdf[s] without a GEMM; z2-bar and the a1 operand
                 // of P6 right away
@@ -721,8 +575,8 @@ sdf_bwd_kernel(const Net net, const Inputs in, const Grads g_) {
                 st16<SPLIT>(big_a, t, v);                            // a2 * 2^(K-k_s)  (weight-gradient operand only)
                 if (CHAIN) st16<SPLIT>(big_b, t, u);                 // u2
             }
-            TR_READY()                                               // P3
-            TR_WAIT()
+            tc::group_ready<tc::PER_WARP>(ct, g, t.lane == 0);  // P3
+            tc::group_wait(ct, g, dpar);
             }
             float zp[16], vb[16];                             // z1-bar (chain part) and v1-bar, kept in registers
             if (CHAIN) {
@@ -744,11 +598,11 @@ sdf_bwd_kernel(const Net net, const Inputs in, const Grads g_) {
 #pragma unroll
                 for (int j = 0; j < 16; ++j) z[j] = sp_sig(z[j] + b2f) * w30f * wsc[j];
                 st16<SPLIT>(big_b, t, z);                            // u2 * 2^(K-k_s)  (v1's MMA has drained)
-                TR_READY()                                           // P4
-                TR_WAIT()
+                tc::group_ready<tc::PER_WARP>(ct, g, t.lane == 0);  // P4
+                tc::group_wait(ct, g, dpar);
                 st16<SPLIT>(big_a, t, vb);                           // v1-bar
-                TR_READY()                                           // P5
-                TR_WAIT()
+                tc::group_ready<tc::PER_WARP>(ct, g, t.lane == 0);  // P5
+                tc::group_wait(ct, g, dpar);
             }
             if (!SDF_ONLY) {
                 float ub[16], ab[16], z[16];
@@ -776,8 +630,8 @@ sdf_bwd_kernel(const Net net, const Inputs in, const Grads g_) {
                 for (int j = 0; j < 16; ++j) z[j] = sp_act(z[j] + b1f) * wsc[j];
                 st16<SPLIT>(big_b, t, z);                            // a1 * 2^(K-k_s)
             }
-            TR_READY()                                               // P6
-            TR_WAIT()
+            tc::group_ready<tc::PER_WARP>(ct, g, t.lane == 0);  // P6
+            tc::group_wait(ct, g, dpar);
             {
                 float ab[16], z[16];
                 ld16_issue(t, T0, ab);
@@ -791,10 +645,10 @@ sdf_bwd_kernel(const Net net, const Inputs in, const Grads g_) {
                 }
                 st16<SPLIT>(big_a, t, z);                            // z1-bar
             }
-            TR_READY()                                               // P7
-            TR_WAIT()
+            tc::group_ready<tc::PER_WARP>(ct, g, t.lane == 0);  // P7
+            tc::group_wait(ct, g, dpar);
             if (g_.g_in0 || g_.g_in1) store_rows(g_.g_in0, in.w0, in.sc0, g_.g_in1, in.w1, s0, in.S, t, T0, 0.0f, sinv);
-            grp_sync(g);                                      // sinv/swsc are rewritten by the next tile
+            tc::named_sync<TR_GRP>(1 + g);                    // sinv/swsc are rewritten by the next tile
         }
     }
     // every MMA has completed once group 1 is past its last wait; publish that to the whole CTA before the flush
@@ -857,51 +711,14 @@ sdf_bwd_kernel(const Net net, const Inputs in, const Grads g_) {
 constexpr int EV_GRP = 256, EV_THREADS = 2 * EV_GRP + 64;
 constexpr uint32_t EV_H0 = W_END, EV_A = EV_H0 + 2 * IMG_S_BYTES, EV_CTRL = EV_A + 2 * IMG_B_BYTES,
                    EV_SMEM = EV_CTRL + 64;
-struct EvCtrl {
-    uint64_t bar_w, done[2], ready[2];
-    uint32_t tmem_slot, pad;
-};
-__device__ __forceinline__ void ev_sync(int g) {
-    asm volatile("bar.sync %0, %1;" ::"r"(1 + g), "n"(EV_GRP) : "memory");
-}
-__device__ __forceinline__ void ev_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tc::smem_u32(bar)) : "memory");
-}
-#define EV_ISSUE(...)                                          \
-    {                                                          \
-        tc::mbar_wait(&ct->ready[g], rpar);                    \
-        rpar ^= 1u;                                            \
-        tc::tc_fence_after();                                  \
-        if (tc::elect_one()) {                                 \
-            __VA_ARGS__                                        \
-            tc::mma_commit(&ct->done[g]);                      \
-        }                                                      \
-        __syncwarp();                                          \
-    }
-#define EV_DONE() { tc::fence_async_smem(); tc::tc_fence_before(); ev_sync(g); if (tg == 0) ev_arrive(&ct->ready[g]); }
-#define EV_WAIT() { tc::mbar_wait(&ct->done[g], dpar); dpar ^= 1u; tc::tc_fence_after(); }
-
 __global__ void __launch_bounds__(EV_THREADS, 1)
 sdf_eval_kernel(const Net net, const Inputs in, float *__restrict__ out, float *__restrict__ sdf) {
     extern __shared__ __align__(1024) uint8_t smem[];
-    EvCtrl *ct = reinterpret_cast<EvCtrl *>(smem + EV_CTRL);
+    tc::Pipe *ct = reinterpret_cast<tc::Pipe *>(smem + EV_CTRL);
     Tid t = make_tid();
-    if (t.tid == 0) {
-        tc::mbar_init(&ct->bar_w, 1);
-        for (int i = 0; i < 2; ++i) { tc::mbar_init(&ct->done[i], 1); tc::mbar_init(&ct->ready[i], 1); }
-        tc::mbar_fence_init();
-    }
-    if (t.warp == 0) tc::tmem_alloc(&ct->tmem_slot, 512);
-    tc::tc_fence_before();
-    __syncthreads();
-    tc::tc_fence_after();
+    tc::pipe_init(ct, 1, 512);
     const uint32_t tmem = ct->tmem_slot;
-    if (t.tid == 0) {
-        tc::mbar_expect_tx(&ct->bar_w, W_END);
-        tc::bulk_g2s(smem + W1_OFF, net.w1, 2 * W1_PLANE, &ct->bar_w);
-        tc::bulk_g2s(smem + W2_OFF, net.w2, 2 * W2_PLANE, &ct->bar_w);
-        tc::bulk_g2s(smem + W3_OFF, net.w3, 2 * W3_PLANE, &ct->bar_w);
-    }
+    load_weights(smem, net, &ct->bar_w);
     tc::mbar_wait(&ct->bar_w, 0);
     const int n_tiles = (in.S + NS - 1) / NS;
     const uint32_t sW1 = tc::smem_u32(smem + W1_OFF), sW2 = tc::smem_u32(smem + W2_OFF), sW3 = tc::smem_u32(smem + W3_OFF);
@@ -912,10 +729,15 @@ sdf_eval_kernel(const Net net, const Inputs in, float *__restrict__ out, float *
         const uint32_t sH0 = tc::smem_u32(smem + EV_H0 + g * IMG_S_BYTES), sA = tc::smem_u32(smem + EV_A + g * IMG_B_BYTES);
         const uint32_t tm = tmem + (uint32_t)(192 * g);
         uint32_t rpar = 0u;
+        // one GEMM per hand-over, D = W x: the three products, fully unrolled
+        auto link = [&](uint32_t d, const tc::Operand &W, const tc::Operand &X, int ksteps) {
+            tc::issue(ct, g, rpar, [&] { tc::gemm_split3<tc::UNROLLED>(d, W, X, ksteps, id_kn, false, false); });
+            rpar ^= 1u;
+        };
         for (int tile = 2 * blockIdx.x + g; tile < n_tiles; tile += 2 * gridDim.x) {
-            EV_ISSUE(gemm3<KP / 16>(tm + 0, tc::op_kmajor(sW1, W1_PLANE, HID), tc::op_mnmajor(sH0, IMG_S_PLANE, KP), id_kn, false);)
-            EV_ISSUE(gemm3<HID / 16>(tm + 64, tc::op_kmajor(sW2, W2_PLANE, HID), tc::op_mnmajor(sA, IMG_B_PLANE, HID), id_kn, false);)
-            EV_ISSUE(gemm3<HID / 16>(tm + 128, tc::op_kmajor(sW3, W3_PLANE, KP), tc::op_mnmajor(sA, IMG_B_PLANE, HID), id_kn, false);)
+            link(tm + 0, tc::op_kmajor(sW1, W1_PLANE, HID), tc::op_mnmajor(sH0, IMG_S_PLANE, KP), KP / 16);
+            link(tm + 64, tc::op_kmajor(sW2, W2_PLANE, HID), tc::op_mnmajor(sA, IMG_B_PLANE, HID), HID / 16);
+            link(tm + 128, tc::op_kmajor(sW3, W3_PLANE, KP), tc::op_mnmajor(sA, IMG_B_PLANE, HID), HID / 16);
         }
     } else {
         // ---- epilogue group g: thread = feature row f x the 32 sample columns [32*cg, +32) -----------
@@ -941,13 +763,13 @@ sdf_eval_kernel(const Net net, const Inputs in, float *__restrict__ out, float *
                 tc::store_chunk(h0_img, IMG_S_PLANE, KP, fs, cs, hv[0]);
                 tc::store_chunk(h0_img, IMG_S_PLANE, KP, fs, cs + 4, hv[1]);
             }
-            EV_DONE()
+            tc::group_ready<EV_GRP>(ct, g, tg == 0);
             const int tn = tile + 2 * gridDim.x;          // prefetch this group's next tile
             if (tn < n_tiles) {
                 load_chunk8(src_h, cs << 6, tn * NS, in.S, hv[0]);
                 load_chunk8(src_h, (cs + 4) << 6, tn * NS, in.S, hv[1]);
             }
-            EV_WAIT()
+            tc::group_wait(ct, g, dpar);
 #pragma unroll
             for (int cc = 0; cc < 2; ++cc) {              // a1 = softplus(Z1 + b1)
                 t.col0 = 32 * cg + 16 * cc;
@@ -957,8 +779,8 @@ sdf_eval_kernel(const Net net, const Inputs in, float *__restrict__ out, float *
                 for (int j = 0; j < 16; ++j) v[j] = sp_act(v[j] + b1f);
                 st16(a_img, t, v);
             }
-            EV_DONE()
-            EV_WAIT()
+            tc::group_ready<EV_GRP>(ct, g, tg == 0);
+            tc::group_wait(ct, g, dpar);
 #pragma unroll
             for (int cc = 0; cc < 2; ++cc) {              // a2 = softplus(Z2 + b2)  (a1's GEMM has drained)
                 t.col0 = 32 * cg + 16 * cc;
@@ -968,8 +790,8 @@ sdf_eval_kernel(const Net net, const Inputs in, float *__restrict__ out, float *
                 for (int j = 0; j < 16; ++j) v[j] = sp_act(v[j] + b2f);
                 st16(a_img, t, v);
             }
-            EV_DONE()
-            EV_WAIT()
+            tc::group_ready<EV_GRP>(ct, g, tg == 0);
+            tc::group_wait(ct, g, dpar);
 #pragma unroll
             for (int cc = 0; cc < 2; ++cc) {              // out = W3 a2 + b3 (lanes >= n_out don't-care)
                 t.col0 = 32 * cg + 16 * cc;
@@ -986,7 +808,7 @@ sdf_eval_kernel(const Net net, const Inputs in, float *__restrict__ out, float *
                 }
             }
             tc::tc_fence_before();
-            ev_sync(g);                                   // this group's images / TMEM columns are reused next tile
+            tc::named_sync<EV_GRP>(1 + g);                // this group's images / TMEM columns are reused next tile
         }
     }
     tc::tc_fence_before();
@@ -1014,24 +836,9 @@ __global__ void absmax2_kernel(const float *__restrict__ a, size_t na, const flo
     if ((threadIdx.x & 31) == 0 && m > 0.0f && m <= 3.4e38f) atomicMax(out, __float_as_uint(m));
 }
 
-bool check_net(const rsdf_sdf_mlp *n) {
-    return n && n->w1_blob && n->w2_blob && n->w3_blob && n->b1 && n->b2 && n->b3 && n->w3_row0 && n->n_in >= 1 &&
-           n->n_in <= KP && n->n_out >= 1 && n->n_out <= KP;
-}
-Net to_net(const rsdf_sdf_mlp *n) {
-    return Net{(const uint8_t *)n->w1_blob, (const uint8_t *)n->w2_blob, (const uint8_t *)n->w3_blob,
-               n->b1, n->b2, n->b3, n->w3_row0, n->n_in, n->n_out, n->precision};
-}
-
 }  // namespace
 
 extern "C" {
-
-#ifdef RSDF_PROFILE_PHASES
-int rsdf_debug_read_prof(unsigned long long *host8) {
-    return (int)cudaMemcpyFromSymbol(host8, g_prof, sizeof(unsigned long long) * 8);
-}
-#endif
 
 int rsdf_absmax2(const float *a, long long na, const float *b, long long nb, uint32_t *out_bits, int accumulate,
                  void *stream) {
@@ -1057,26 +864,16 @@ int rsdf_sdf_mlp_fwd(const rsdf_sdf_mlp *net, const float *in0, int w0, float sc
     const Inputs in{in0, in1, w0, w1, scale0, shift0, n_samples};
     const int n_tiles = (n_samples + NS - 1) / NS;
     const int grid = n_tiles < RSDF_NUM_SMS ? n_tiles : RSDF_NUM_SMS;
-    cudaError_t e;
-#define RSDF_FWD(G, SP)                                                                                          \
-    {                                                                                                            \
-        e = cudaFuncSetAttribute(sdf_fwd_kernel<G, SP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)F_SMEM); \
-        if (e != cudaSuccess) return (int)e;                                                                     \
-        sdf_fwd_kernel<G, SP><<<grid, TR_THREADS, F_SMEM, (cudaStream_t)stream>>>(to_net(net), in, out, sdf, g0a, g0b); \
-    }
+    const Net n = to_net(net);
     if (g0a) {
-        if (net->precision) RSDF_FWD(true, false) else RSDF_FWD(true, true)
-    } else if (net->precision) {
-        RSDF_FWD(false, false)          // (the two-group inference kernel below is fp32-class only)
-    } else {
-        const int pairs = (n_tiles + 1) / 2;
-        const int eg = pairs < RSDF_NUM_SMS ? pairs : RSDF_NUM_SMS;
-        e = cudaFuncSetAttribute(sdf_eval_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EV_SMEM);
-        if (e != cudaSuccess) return (int)e;
-        sdf_eval_kernel<<<eg, EV_THREADS, EV_SMEM, (cudaStream_t)stream>>>(to_net(net), in, out, sdf);
+        auto k = net->precision ? sdf_fwd_kernel<true, false> : sdf_fwd_kernel<true, true>;
+        return rsdf_launch(k, grid, TR_THREADS, F_SMEM, stream, n, in, out, sdf, g0a, g0b);
     }
-    RSDF_LAUNCH_CHECK();
-    return 0;
+    if (net->precision)                 // (the two-group inference kernel below is fp32-class only)
+        return rsdf_launch(sdf_fwd_kernel<false, false>, grid, TR_THREADS, F_SMEM, stream, n, in, out, sdf, g0a, g0b);
+    const int pairs = (n_tiles + 1) / 2;
+    const int eg = pairs < RSDF_NUM_SMS ? pairs : RSDF_NUM_SMS;
+    return rsdf_launch(sdf_eval_kernel, eg, EV_THREADS, EV_SMEM, stream, n, in, out, sdf);
 }
 
 int rsdf_sdf_mlp_bwd(const rsdf_sdf_mlp *net, const float *in0, int w0, float scale0, float shift0,
@@ -1091,23 +888,11 @@ int rsdf_sdf_mlp_bwd(const rsdf_sdf_mlp *net, const float *in0, int w0, float sc
     const Grads g{g_out, g_sdf, g_g0a, g_g0b, amax_bits, g_in0, g_in1, gW1, gb1, gW2, gb2, gW3, gb3};
     const int n_tiles = (n_samples + NS - 1) / NS;
     const int grid = n_tiles < RSDF_NUM_SMS ? n_tiles : RSDF_NUM_SMS;
-    cudaError_t e;
-#define RSDF_BWD(C, SP, ...)                                                                                          \
-    {                                                                                                                 \
-        e = cudaFuncSetAttribute(sdf_bwd_kernel<C, SP, ##__VA_ARGS__>, cudaFuncAttributeMaxDynamicSharedMemorySize,   \
-                                 (int)B_SMEM);                                                                        \
-        if (e != cudaSuccess) return (int)e;                                                                          \
-        sdf_bwd_kernel<C, SP, ##__VA_ARGS__><<<grid, TR_THREADS, B_SMEM, (cudaStream_t)stream>>>(to_net(net), in, g); \
-    }
-    if (g_g0a || g_g0b) {
-        if (net->precision) RSDF_BWD(true, false) else RSDF_BWD(true, true)
-    } else if (!g_out) {                 // only the sdf head carries a cotangent
-        if (net->precision) RSDF_BWD(false, false, true) else RSDF_BWD(false, true, true)
-    } else {
-        if (net->precision) RSDF_BWD(false, false) else RSDF_BWD(false, true)
-    }
-    RSDF_LAUNCH_CHECK();
-    return 0;
+    auto k = net->precision ? sdf_bwd_kernel<false, false> : sdf_bwd_kernel<false, true>;
+    if (g_g0a || g_g0b) k = net->precision ? sdf_bwd_kernel<true, false> : sdf_bwd_kernel<true, true>;
+    else if (!g_out)                     // only the sdf head carries a cotangent
+        k = net->precision ? sdf_bwd_kernel<false, false, true> : sdf_bwd_kernel<false, true, true>;
+    return rsdf_launch(k, grid, TR_THREADS, B_SMEM, stream, to_net(net), in, g);
 }
 
 }  // extern "C"

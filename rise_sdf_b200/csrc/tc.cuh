@@ -59,6 +59,15 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
         : "memory");
 }
 
+__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+// named barrier `id` (1..15; 0 is __syncthreads) over NTHREADS threads
+template <int NTHREADS>
+__device__ __forceinline__ void named_sync(int id) {
+    asm volatile("bar.sync %0, %1;" ::"r"(id), "n"(NTHREADS) : "memory");
+}
+
 // ---- proxy / tcgen05 fences -------------------------------------------------------------
 // generic-proxy smem writes -> visible to the async proxy (tensor core, bulk copies)
 __device__ __forceinline__ void fence_async_smem() {
@@ -115,6 +124,16 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, float *v) {
 __device__ __forceinline__ void tmem_ld_wait() {
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
+// registers -> 32 lanes x 8 / 4 consecutive 32-bit columns (thread i <-> lane base+i)
+__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t *r) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr), "r"(r[0]),
+                 "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]) : "memory");
+}
+__device__ __forceinline__ void tmem_st4(uint32_t taddr, const uint32_t *r) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};" ::"r"(taddr), "r"(r[0]), "r"(r[1]),
+                 "r"(r[2]), "r"(r[3]) : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 // ---- descriptors ------------------------------------------------------------------------
 // shared-memory matrix descriptor, SWIZZLE_NONE, version 1 (Blackwell)
@@ -143,6 +162,17 @@ __device__ __forceinline__ void mma_f16(uint32_t tmem_d, uint64_t adesc, uint64_
         "}" ::"r"(tmem_d),
         "l"(adesc), "l"(bdesc), "r"(idesc), "r"((uint32_t)accumulate)
         : "memory");
+}
+// D[tmem] (+)= A[tmem] * B[smem]   ("TS" form: the A operand is read from tensor memory)
+__device__ __forceinline__ void mma_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc,
+                                       bool accumulate) {
+    const uint32_t z = 0u;
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, {%5, %5, %5, %5}, p;\n\t"
+        "}" ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"((uint32_t)accumulate), "r"(z) : "memory");
 }
 // make all previously issued MMAs arrive on `bar` when they complete
 __device__ __forceinline__ void mma_commit(uint64_t *bar) {
@@ -235,32 +265,130 @@ __device__ __forceinline__ void load_chunk_hi(const uint8_t *img, int rows, int 
 }
 
 // Issue the 3-product split GEMM  D[128 x N] (+)= A[128 x K] * B[N x K]^T  over tile images.
-//   a_img / b_img: smem addresses of the hi planes; *_plane: hi->lo plane stride in bytes
-//   a_lbo/a_sbo/a_kstep: descriptor strides and the byte advance per K=16 step (role dependent)
-// Must be called by ONE thread.  `first_overwrites`: the very first MMA clears D.
+//   addr: smem address of the hi plane; plane: hi->lo plane stride in bytes
+//   lbo/sbo/kstep: descriptor strides and the byte advance per K=16 step (role dependent)
+// Must be called by ONE thread.  Unless `accumulate`, the very first MMA clears D.
 struct Operand {
     uint32_t addr, plane, lbo, sbo, kstep;
 };
+// How the issue stream is laid out; it decides the issuing thread's register budget, not the result:
+//   ROLLED   : product and k loops rolled (any k-step count)
+//   ROLL_K   : one rolled k loop per product -- an issuer warp running ~40 GEMMs per tile: a fully unrolled stream
+//              keeps hundreds of precomputed 64-bit descriptors live, they spill, and every reload of the single
+//              issuing lane is an L2 round trip in front of an MMA (ncu: 1500 local loads per tile, 32 % L1 hit)
+//   UNROLLED : everything unrolled (k-step count a compile-time constant <= 8 after inlining)
+enum Unroll { ROLLED, ROLL_K, UNROLLED };
+// Products in the order lo*lo, lo*hi, hi*lo, hi*hi (small terms first into the accumulator).  The lo*lo term (~2^-22
+// of the product) halves the residual error; callers whose tensor time matters drop it (keep_lo_lo = false: the
+// training kernels' three products).  split = false: hi*hi alone, the single-plane fp16 variant.
+// KSTEPS > 0 fixes the k-step count at compile time (`ksteps` is then not read).  The training issuer needs it: with a
+// count that becomes constant only after inlining, nvcc moves the accumulate flags of its 2-step sample-contracting
+// GEMMs out of uniform predicates (R2UR per MMA) and the backward kernel runs 0.5-0.9 % slower.
+template <Unroll U = ROLLED, int KSTEPS = 0>
 __device__ __forceinline__ void gemm_split3(uint32_t tmem_d, const Operand &A, const Operand &B, int ksteps,
-                                            uint32_t idesc, bool accumulate, bool keep_lo_lo = true) {
-    // order: lo*lo, lo*hi, hi*lo, hi*hi (small terms first into the accumulator).  The lo*lo term (~2^-22 of the
-    // product) halves the residual error; callers whose tensor time matters drop it (keep_lo_lo = false: the same
-    // three products as the training kernels).
-    const int first = keep_lo_lo ? 0 : 1;
+                                            uint32_t idesc, bool accumulate, bool keep_lo_lo = true, bool split = true) {
     // the address is the low 14 bits of a descriptor's low word and never carries out of it: a K step is ONE 32-bit add
     // per operand (building a descriptor from scratch per instruction costs more issue time than the MMA takes to run)
     const uint64_t a_d = smem_desc(A.addr, A.lbo, A.sbo), b_d = smem_desc(B.addr, B.lbo, B.sbo);
     const uint32_t a_hi32 = (uint32_t)(a_d >> 32), b_hi32 = (uint32_t)(b_d >> 32);
     const uint32_t ak = A.kstep >> 4, bk = B.kstep >> 4;
+    if constexpr (U == ROLLED) {
+        const int first = !split ? 3 : keep_lo_lo ? 0 : 1;
 #pragma unroll 1
-    for (int term = first; term < 4; ++term) {
-        uint32_t a = (uint32_t)a_d + (term < 2 ? (A.plane >> 4) : 0u);
-        uint32_t b = (uint32_t)b_d + ((term == 0 || term == 2) ? (B.plane >> 4) : 0u);
+        for (int term = first; term < 4; ++term) {
+            uint32_t a = (uint32_t)a_d + (term < 2 ? (A.plane >> 4) : 0u);
+            uint32_t b = (uint32_t)b_d + ((term == 0 || term == 2) ? (B.plane >> 4) : 0u);
 #pragma unroll 1
-        for (int k = 0; k < ksteps; ++k, a += ak, b += bk)
-            mma_f16(tmem_d, ((uint64_t)a_hi32 << 32) | a, ((uint64_t)b_hi32 << 32) | b, idesc,
-                    accumulate || term > first || k > 0);
+            for (int k = 0; k < ksteps; ++k, a += ak, b += bk)
+                mma_f16(tmem_d, ((uint64_t)a_hi32 << 32) | a, ((uint64_t)b_hi32 << 32) | b, idesc,
+                        accumulate || term > first || k > 0);
+        }
+    } else {
+        const int nk = KSTEPS > 0 ? KSTEPS : ksteps;
+        auto pass = [&](uint32_t a, uint32_t b, bool acc0) {         // one product, k loop rolled or unrolled
+#pragma unroll (U == UNROLLED ? 8 : 1)
+            for (int k = 0; k < nk; ++k, a += ak, b += bk)
+                mma_f16(tmem_d, ((uint64_t)a_hi32 << 32) | a, ((uint64_t)b_hi32 << 32) | b, idesc, acc0 || k > 0);
+        };
+        const uint32_t a = (uint32_t)a_d, b = (uint32_t)b_d, apl = A.plane >> 4, bpl = B.plane >> 4;
+        if (split) {
+            if (keep_lo_lo) pass(a + apl, b + bpl, accumulate);
+            pass(a + apl, b, accumulate || keep_lo_lo);
+            pass(a, b + bpl, true);
+        }
+        pass(a, b, split || accumulate);
     }
+}
+// The same split GEMM in TS form, A planes in tensor memory (hi at tmem_a_hi, lo at tmem_a_lo, 8 32-bit columns per
+// K=16 step; B from shared memory): products lo*hi, hi*lo, hi*hi, the first one clears D, fully unrolled
+__device__ __forceinline__ void gemm_split3_ts(uint32_t tmem_d, uint32_t tmem_a_hi, uint32_t tmem_a_lo, const Operand &B,
+                                               int ksteps, uint32_t idesc) {
+    const uint64_t b_hi = smem_desc(B.addr, B.lbo, B.sbo), b_lo = smem_desc(B.addr + B.plane, B.lbo, B.sbo);
+    const uint64_t bk = B.kstep >> 4;
+#pragma unroll
+    for (int k = 0; k < ksteps; ++k) mma_ts(tmem_d, tmem_a_lo + 8 * k, b_hi + k * bk, idesc, k > 0);
+#pragma unroll
+    for (int k = 0; k < ksteps; ++k) mma_ts(tmem_d, tmem_a_hi + 8 * k, b_lo + k * bk, idesc, true);
+#pragma unroll
+    for (int k = 0; k < ksteps; ++k) mma_ts(tmem_d, tmem_a_hi + 8 * k, b_hi + k * bk, idesc, true);
+}
+
+// ---- issuer <-> epilogue-group handshake ------------------------------------------------------------------------
+// Kernels with MMA-issuer warp(s) and two epilogue groups g = 0, 1 (named barrier 1 + g): group g announces "the
+// operands of the next GEMM are in place" on ready[g] (group_ready), the issuer issues that GEMM and commits it to
+// done[g] (issue), the group waits on done[g] before it reads the accumulator or overwrites the operands
+// (group_wait).  bar_w completes when the weight blobs have landed.
+struct Pipe {
+    uint64_t bar_w, done[2], ready[2];
+    uint32_t tmem_slot, pad;
+};
+// barriers (ready[g] completes after `ready_arrivals` arrivals) and `tmem_cols` TMEM columns, visible to the CTA
+__device__ __forceinline__ void pipe_init(Pipe *p, uint32_t ready_arrivals, uint32_t tmem_cols) {
+    if (threadIdx.x == 0) {
+        mbar_init(&p->bar_w, 1);
+        for (int i = 0; i < 2; ++i) { mbar_init(&p->done[i], 1); mbar_init(&p->ready[i], ready_arrivals); }
+        mbar_fence_init();
+    }
+    if (threadIdx.x / 32 == 0) tmem_alloc(&p->tmem_slot, tmem_cols);
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+}
+// issuer warp: wait for group g's operands, issue `body` from one lane, make the MMAs' completion arrive on done[g]
+template <class F>
+__device__ __forceinline__ void issue(Pipe *p, int g, uint32_t parity, F &&body) {
+    mbar_wait(&p->ready[g], parity);
+    tc_fence_after();
+    if (elect_one()) {
+        body();
+        mma_commit(&p->done[g]);
+    }
+    __syncwarp();
+}
+// group g: make this thread's operand writes visible to the tensor core and hand them to the issuer.
+//   TMEM_OPERANDS: the operands were written with tcgen05.st (wait for them), else to shared memory (proxy fence)
+//   GRP_THREADS  : PER_WARP -- every warp arrives once and the group's warps never meet (ready[g] counts them);
+//                  otherwise the group's GRP_THREADS threads meet at named barrier 1 + g and one of them arrives
+constexpr int PER_WARP = 0;
+//   leader       : this thread arrives (lane 0 of its warp / one thread of the group)
+template <int GRP_THREADS, bool TMEM_OPERANDS = false>
+__device__ __forceinline__ void group_ready(Pipe *p, int g, bool leader) {
+    if constexpr (TMEM_OPERANDS) tmem_st_wait();
+    else fence_async_smem();
+    tc_fence_before();
+    if constexpr (GRP_THREADS == PER_WARP) {
+        __syncwarp();
+        if (leader) mbar_arrive(&p->ready[g]);
+    } else {
+        named_sync<GRP_THREADS>(1 + g);
+        if (leader) mbar_arrive(&p->ready[g]);
+    }
+}
+// group g: wait for the GEMMs of its last hand-over
+__device__ __forceinline__ void group_wait(Pipe *p, int g, uint32_t &parity) {
+    mbar_wait(&p->done[g], parity);
+    parity ^= 1u;
+    tc_fence_after();
 }
 
 // operand views of a tile image with `rows` rows
